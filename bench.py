@@ -1,6 +1,7 @@
 """Benchmark of the cnn_linear hot path (BASELINE.json metric: train sequences/sec, 20x224 breaths).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--backbone resnet18|densenet18]
+                    [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] -- cnn_linear / ResNet-18 training step on synthetic
 256 x 20 x 1 x 224 batches per GPU, bf16 storage + tcgen05 convolutions, fp32 statistics / gradients / weights.
@@ -27,6 +28,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark leaves the tree as build() left it: without this its imports that build() does not make
+# (deepards_b200.data_parallel, deepards_b200.synthetic, the CPU oracle) would write __pycache__ files there
+sys.dont_write_bytecode = True
 
 SEQ_PER_GPU = 256
 SUB_BATCH = 20
@@ -175,6 +179,7 @@ def workload_config(args, cpu_sample=None):
                       if getattr(args, "scaling", "weak") == "strong" else ""),
          "backbone": args.backbone, "sequences_per_gpu": per_gpu, "sub_batch": SUB_BATCH, "precision": "bf16 storage / "
          "tcgen05 convolutions, fp32 statistics, gradients and weights", "parallelism": "dp%d" % args.gpus,
+         "wgrad": os.environ.get("DEEPARDS_B200_WGRAD", "accumulate"),
          "cuda_graph": (not args.no_graph) and ("whole step" if args.gpus == 1 else getattr(args, "dp_graph_desc", "per segment, NCCL between")),
          "l2": "working set per step (>1 GB of activations) exceeds the 126 MB L2; 4 resident input batches are rotated"}
     if cpu_sample:
@@ -300,6 +305,8 @@ def run_b200(args):
         l0, g0 = lib.dards_launch_count(), trainer.graph_launches
         ms = timed(resident_step, steps)
         launches = (lib.dards_launch_count() - l0) + (trainer.graph_launches - g0)
+        if args.dump_outputs and backbone == args.backbone and rank == 0:
+            dump_outputs(args.dump_outputs, trainer, trainer.plan_for(xs[0]))
         prefetch(0)
         for i in range(2):
             e2e_step(i)
@@ -589,6 +596,24 @@ def kernel_roofline(trainer, x, t, args, backbone, steps=3):
     return out
 
 
+def dump_outputs(outdir, trainer, plan):
+    """--dump-outputs: what the last timed step computed, as float32 DIR/<name>.npy, so that two builds can be compared
+    output for output on the same seeded inputs: the loss it returned, the logits of its forward pass and, concatenated
+    in named_parameters() order, its gradients (before the clamp) and the parameters after its update (31 MB for
+    ResNet-18).  Unless DEEPARDS_B200_WGRAD is set, main() runs such a benchmark with the fixed-order weight-gradient
+    reduction, so the files are the same bit for bit from run to run."""
+    import numpy as np
+    import torch
+    params = [p for _, p in trainer.net.named_parameters()]
+    arrays = {"loss": trainer.loss_buf, "logits": plan.logits,
+              "grads": torch.cat([plan.grad_view(p).reshape(-1) for p in params]),
+              "params": torch.cat([p.detach().reshape(-1) for p in params])}
+    assert sum(a.numel() for a in arrays.values()) * 4 <= 64 << 20
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), a.detach().float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=int(os.environ.get("WORLD_SIZE", "1")))
@@ -604,7 +629,26 @@ def main():
     ap.add_argument("--no-extra", action="store_true",
                     help="only the headline legs: no sustained leg, no densenet18 / module_path / dp_parity sub-objects")
     ap.add_argument("--sustained-s", type=float, default=2.5, help="length of the sustained leg in seconds")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, logits, gradients and updated parameters of the last timed step as DIR/<name>.npy; "
+                         "unless DEEPARDS_B200_WGRAD is set, the run then sums weight gradients in a fixed order "
+                         "(DEEPARDS_B200_WGRAD=deterministic), so that repeated runs write identical files.  With the "
+                         "default arrival-order sums (DEEPARDS_B200_WGRAD=accumulate) two runs drift apart over the "
+                         "warm-up and timed steps")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
+    if args.dump_outputs:
+        # Outputs that can be compared need a step that computes the same thing every run.  The default weight-gradient
+        # kernels add their fp32 tiles in the L2 in arrival order; one step is reproducible to rounding, but the warm-up
+        # and timed steps of bf16 training can amplify those differences far beyond it (pairs of --warmup 5 --steps 20
+        # runs with DEEPARDS_B200_WGRAD=accumulate on a B200 at 1000 W: some agreed to 2e-8, one ended with logits 7 %
+        # of their largest value apart).  The
+        # fixed-order split-K reduction is bit-reproducible and slower (INTEGRATION.md, DEEPARDS_B200_WGRAD); the
+        # timings of the run are of the reduction config.wgrad names.
+        os.environ.setdefault("DEEPARDS_B200_WGRAD", "deterministic")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -41,6 +41,7 @@ from deepards.models.torch_cnn_linear_network import (  # noqa: E402
 OUT = os.path.join(ROOT, "tests", "golden")
 SAMPLE_STRIDE = 61
 FULL_LIMIT = 50_000  # tensors up to this many elements are stored whole
+MAX_FILE_BYTES = 1_000_000  # fixtures stay small: beyond this the largest whole gradients are sampled as well
 
 
 def real_sequences(n=2):
@@ -82,8 +83,24 @@ def record_grads(rec, model):
         if g.size <= FULL_LIMIT:
             rec["grad/" + name] = g.reshape(p.shape).copy()
         else:
-            rec["gradsample/" + name] = g[::SAMPLE_STRIDE].copy()
-            rec["gradstat/" + name] = np.array([g.sum(dtype=np.float64), np.sqrt((g.astype(np.float64) ** 2).sum())])
+            record_sample(rec, name, g)
+
+
+def record_sample(rec, name, g):
+    rec["gradsample/" + name] = g[::SAMPLE_STRIDE].copy()
+    rec["gradstat/" + name] = np.array([g.sum(dtype=np.float64), np.sqrt((g.astype(np.float64) ** 2).sum())])
+
+
+def save_within_limit(path, rec):
+    """np.savez_compressed, sampling the largest whole gradients (as record_grads samples those beyond FULL_LIMIT)
+    until the file fits in MAX_FILE_BYTES."""
+    while True:
+        np.savez_compressed(path, **rec)
+        whole = [k for k in rec if k.startswith("grad/")]
+        if os.path.getsize(path) <= MAX_FILE_BYTES or not whole:
+            return
+        key = max(whole, key=lambda k: rec[k].size)
+        record_sample(rec, key[len("grad/"):], rec.pop(key).reshape(-1))
 
 
 def run_case(name, model, sd, x, target, per_breath=False, extra=None):
@@ -107,7 +124,7 @@ def run_case(name, model, sd, x, target, per_breath=False, extra=None):
         rec.update(extra)
     os.makedirs(OUT, exist_ok=True)
     path = os.path.join(OUT, name + ".npz")
-    np.savez_compressed(path, **rec)
+    save_within_limit(path, rec)
     print("%-34s logits[0]=%s loss=%.6f  %.1f KB" % (name, out[0].detach().numpy().ravel()[:2], loss.item(),
                                                    os.path.getsize(path) / 1024))
 

@@ -124,6 +124,36 @@ def test_registries_and_install():
     assert fake.CNNLinearNetwork is D.CNNLinearNetwork
 
 
+def test_trainer_calls_build_b200_networks_after_install():
+    """What deepards/train_ards_detector.py does with a module patched by install(), replayed with the arguments it passes
+    (SURVEY.md, INTEGRATION.md): get_base_network calls resnet18(initial_planes, first_pool_type, double_conv_first)
+    (:389-394) or densenet18(with_fft, only_fft, fft_real_only) (:404-409); get_network builds
+    CNNLinearNetwork(base, n_sub_batches, n_metadata_inputs) (:938-939) or CNNSingleBreathLinearNetwork(base) (:963-964);
+    get_model registers a clamp hook on every parameter (:474-476); get_optimizer hands all parameters to SGD-Nesterov
+    (:416-422)."""
+    import types
+    import deepards_b200 as D
+    fake = types.ModuleType("train_ards_detector")
+    fake.base_networks = {}
+    D.install(fake)
+    assert fake.CNNSingleBreathLinearNetwork is D.CNNSingleBreathLinearNetwork
+    resnet = lambda: fake.base_networks["resnet18"](initial_planes=64, first_pool_type="max", double_conv_first=False)
+    densenet = lambda: fake.base_networks["densenet18"](with_fft=False, only_fft=False, fft_real_only=False)
+    for base, get_network, head_cls in ((resnet, lambda bb: fake.CNNLinearNetwork(bb, 20, 0), D.CNNLinearNetwork),
+                                        (densenet, lambda bb: fake.CNNLinearNetwork(bb, 20, 0), D.CNNLinearNetwork),
+                                        (resnet, fake.CNNSingleBreathLinearNetwork, D.CNNSingleBreathLinearNetwork)):
+        bb = base()
+        model = get_network(bb)
+        assert type(model) is head_cls and model.breath_block is bb
+        assert type(bb).__module__.startswith("deepards_b200.")
+        for p in model.parameters():
+            p.register_hook(lambda grad: torch.clamp(grad, -0.01, 0.01))   # raises for a tensor without requires_grad
+        opt = torch.optim.SGD(model.parameters(), lr=1e-3, momentum=0.9, weight_decay=1e-4, nesterov=True)
+        assert sum(p.numel() for g in opt.param_groups for p in g["params"]) == sum(p.numel() for p in model.parameters())
+        with pytest.raises(RuntimeError, match="no CPU fallback"):
+            model(torch.zeros(2, 20, 1, 224), None)
+
+
 def test_shard_bounds_live_ranges_and_buckets():
     from deepards_b200 import data_parallel as dp
     import deepards_b200 as D
