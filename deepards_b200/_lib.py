@@ -50,8 +50,11 @@ _SIGNATURES = {
     "dards_reduce_rows_batched": [P, I, I, P],
     "dards_bn_running_update_batched": [P, I, I, F, P],
     "dards_bn_running_update": [P, P, P, P, P, I, I, I, F, F, P],
+    "dards_bn_eval_coeffs_batched": [P, I, I, F, P],
+    "dards_conv1d_affine_fwd": [P, P, P, P, P, P, I, I, I, I, I, I, I, I, I, I, I, I, I, I, P],
     "dards_stem_workspace_bytes": [I, I, I, I],
     "dards_stem_fwd": [P, P, P, P, P, P, P, I, I, I, I, F, I, P, LL, I, P],
+    "dards_stem_eval_fwd": [P, P, P, P, P, I, I, I, I, I, P],
     "dards_stem_bwd": [P, P, P, P, P, P, P, P, P, P, I, I, I, I, I, P, LL, I, P],
     "dards_avgpool2_fwd": [P, P, I, I, I, I, I, I, P],
     "dards_avgpool2_bwd": [P, P, I, I, I, I, I, I, P],

@@ -43,6 +43,9 @@ class PlanFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dout):
         plan = ctx.plan
+        if plan.bn == "eval":
+            raise NotImplementedError("deepards_b200: backward through running-statistics BatchNorm (ResNet in eval() "
+                                      "mode) is not implemented; call train() on the network to train it")
         if ctx.serial != plan.fwd_serial:
             raise RuntimeError("deepards_b200: this network was called again before backward(); a plan keeps the "
                                "activations of its latest forward only")
@@ -66,14 +69,11 @@ def run_plan(net, backbone, linear, x, group, mode, dropout_key=()):
     """Common entry of every module forward: pick/build the plan, run it through autograd."""
     n = x.numel() // engine.SEQ_LEN
     training = backbone.training
-    if not training and backbone.network_name.startswith("resnet"):
-        # eval() on the reference ResNet would normalise with the running statistics; the reference never does
-        # that on this path (model.eval() is commented out, train_ards_detector.py:448), and a silent switch to
-        # batch statistics here would be a different function.
-        raise NotImplementedError("deepards_b200 ResNet implements training-mode BatchNorm (batch statistics) only; "
-                                  "keep the module in train() mode as train_ards_detector.py does")
+    # A ResNet in eval() normalises with its running statistics: every breath is independent of the rest of the batch, and
+    # `group` only shapes the heads.  DenseNet keeps no running statistics; its eval() only turns dropout off.
+    bn = "eval" if not training and backbone.network_name.startswith("resnet") else "train"
     plan = engine.get_plan(net, backbone, linear, n, group, module_precision(net), mode,
-                           dropout=dropout_key if training else (), update_running=training)
+                           dropout=dropout_key if training else (), update_running=training, bn=bn)
     # Only the parameters the backward writes are inputs of the autograd node.  ResNet's conv1_alt / conv2 / bn2 never
     # take part in forward() (resnet.py:141-163): in the reference they are not in the graph, their hooks never fire and
     # their .grad stays None -- a None handed to a `p.register_hook(lambda g: g.clamp(...))` hook would raise.

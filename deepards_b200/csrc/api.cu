@@ -36,6 +36,12 @@ int tc_conv_wgrad(const void* in, const void* dout, float* dw, int accumulate, v
                   int n_breaths, int l_in, int l_out, int c_in, int c_out, int in_stride, int dout_stride, int ktaps,
                   int stride, int pad, cudaStream_t st);
 long long tc_wgrad_workspace_bytes(int n_breaths, int l_out, int c_in, int c_out, int ktaps);
+int tc_conv_affine_fwd(const void* in, const void* w_koi, void* out, const void* res, const float* scale, const float* shift,
+                       int n_breaths, int l_in, int l_out, int c_in, int c_out, int in_stride, int out_stride, int res_stride,
+                       int ktaps, int stride, int pad, int relu, int src_last_use, cudaStream_t st);
+int launch_bn_eval_coeffs_batched(const dards_eval_coeff_desc*, int, int, float, cudaStream_t);
+int launch_stem_eval_fwd(const float*, const float*, const float*, const float*, void*, int, int, int, int, int,
+                         cudaStream_t);
 int tc_conv_wgrad_accum(const void* in, const void* dout, float* dw_t, int n_breaths, int l_in, int l_out, int c_in, int c_out,
                         int in_stride, int dout_stride, int ktaps, int stride, int pad, cudaStream_t st);
 int simt_unpack_wgrad_batched(const dards_unpack_desc*, int, int, cudaStream_t);
@@ -138,12 +144,53 @@ int dards_conv1d_fwd(const void* in, const void* w_packed, void* out, const void
                        addend_stride, ktaps, stride, pad, src_last_use, S(stream));
   }
   DARDS_CHECK_ARG(impl == 0, "conv1d_fwd: unknown impl %d", impl);
-  ConvGemmArgs a;
+  ConvGemmArgs a{};
   a.in = in; a.w = w_packed; a.out = out; a.addend = addend;
   a.m_total = (long long)n_breaths * l_out;
   a.l_src = l_in; a.l_dst = l_out; a.c_red = c_in; a.c_cols = c_out;
   a.src_stride = in_stride; a.dst_stride = out_stride; a.addend_stride = addend_stride;
   a.ktaps = ktaps; a.q_mul = stride; a.t_mul = 1; a.off = -pad; a.div = 1;
+  return simt_conv_gemm(a, dtype, S(stream));
+}
+
+int dards_conv1d_affine_fwd(const void* in, const void* w_packed, void* out, const void* res, const float* scale,
+                            const float* shift, int n_breaths, int l_in, int l_out, int c_in, int c_out, int in_stride,
+                            int out_stride, int res_stride, int ktaps, int stride, int pad, int relu, int dtype, int impl,
+                            void* stream) {
+  const int src_last_use = (relu & DARDS_HINT_LAST_USE) ? 1 : 0;
+  relu &= 0xff;
+  DARDS_CHECK_ARG(in && w_packed && out && scale && shift, "conv1d_affine_fwd: null pointer");
+  DARDS_CHECK_ARG(n_breaths >= 0 && l_in > 0 && c_in > 0 && c_out > 0 && ktaps > 0 && stride > 0 && pad >= 0,
+                  "conv1d_affine_fwd: bad shape");
+  DARDS_CHECK_ARG(l_out == conv_out_len(l_in, ktaps, stride, pad), "conv1d_affine_fwd: l_out %d != (l_in+2p-k)/s+1 = %d",
+                  l_out, conv_out_len(l_in, ktaps, stride, pad));
+  DARDS_CHECK_ARG(in_stride >= c_in && out_stride >= c_out && (!res || res_stride >= c_out),
+                  "conv1d_affine_fwd: row stride smaller than channel count");
+  DARDS_CHECK_ARG(relu == 0 || relu == 1, "conv1d_affine_fwd: relu must be 0 or 1");
+  if (res) {
+    const size_t esz = dtype == DARDS_BF16 ? 2 : 4;
+    const char* r0 = static_cast<const char*>(res);
+    const char* o0 = static_cast<const char*>(out);
+    const size_t rows = (size_t)n_breaths * l_out;
+    const char* r1 = r0 + (rows ? ((rows - 1) * res_stride + c_out) * esz : 0);
+    const char* o1 = o0 + (rows ? ((rows - 1) * out_stride + c_out) * esz : 0);
+    DARDS_CHECK_ARG(r1 <= o0 || o1 <= r0, "conv1d_affine_fwd: the residual must not overlap the output");
+  }
+  if (impl == 1) {
+    DARDS_CHECK_ARG(dtype == DARDS_BF16, "conv1d_affine_fwd: the tcgen05 path is bf16 only");
+    return tc_conv_affine_fwd(in, w_packed, out, res, scale, shift, n_breaths, l_in, l_out, c_in, c_out, in_stride,
+                              out_stride, res_stride, ktaps, stride, pad, relu, src_last_use, S(stream));
+  }
+  DARDS_CHECK_ARG(impl == 0, "conv1d_affine_fwd: unknown impl %d", impl);
+  DARDS_CHECK_ARG((reinterpret_cast<uintptr_t>(scale) & 15) == 0 && (reinterpret_cast<uintptr_t>(shift) & 15) == 0,
+                  "conv1d_affine_fwd: scale / shift must be 16-byte aligned");
+  ConvGemmArgs a{};
+  a.in = in; a.w = w_packed; a.out = out; a.addend = res;
+  a.m_total = (long long)n_breaths * l_out;
+  a.l_src = l_in; a.l_dst = l_out; a.c_red = c_in; a.c_cols = c_out;
+  a.src_stride = in_stride; a.dst_stride = out_stride; a.addend_stride = res_stride;
+  a.ktaps = ktaps; a.q_mul = stride; a.t_mul = 1; a.off = -pad; a.div = 1;
+  a.scale = scale; a.shift = shift; a.relu = relu;
   return simt_conv_gemm(a, dtype, S(stream));
 }
 
@@ -164,7 +211,7 @@ int dards_conv1d_dgrad(const void* dout, const void* w_packed, void* din, const 
                          addend_stride, ktaps, stride, pad, src_last_use, S(stream));
   }
   DARDS_CHECK_ARG(impl == 0, "conv1d_dgrad: unknown impl %d", impl);
-  ConvGemmArgs a;
+  ConvGemmArgs a{};
   a.in = dout; a.w = w_packed; a.out = din; a.addend = addend;
   a.m_total = (long long)n_breaths * l_in;
   a.l_src = l_out; a.l_dst = l_in; a.c_red = c_out; a.c_cols = c_in;
@@ -307,6 +354,12 @@ int dards_bn_running_update_batched(const dards_running_desc* descs_dev, int n_d
   return launch_bn_running_update_batched(descs_dev, n_descs, total_blocks, eps, S(stream));
 }
 
+int dards_bn_eval_coeffs_batched(const dards_eval_coeff_desc* descs_dev, int n_descs, int total_blocks, float eps,
+                                 void* stream) {
+  DARDS_CHECK_ARG(descs_dev && n_descs >= 0 && total_blocks >= 0, "bn_eval_coeffs_batched: bad argument");
+  return launch_bn_eval_coeffs_batched(descs_dev, n_descs, total_blocks, eps, S(stream));
+}
+
 int dards_bn_running_update(const float* save_mean, const float* save_rstd, float* running_mean, float* running_var,
                             long long* num_batches_tracked, int n_groups, int rows_per_group, int c, float momentum,
                             float eps, void* stream) {
@@ -327,6 +380,15 @@ int dards_stem_fwd(const float* x, const float* w, const float* gamma, const flo
   DARDS_CHECK_ARG(out_stride >= c0, "stem_fwd: row stride smaller than channel count");
   return launch_stem_fwd(x, w, gamma, beta, out, save_mean, save_rstd, n_groups, group, c0, out_stride, eps, pool, workspace,
                          workspace_bytes, dtype, S(stream));
+}
+
+int dards_stem_eval_fwd(const float* x, const float* w, const float* scale, const float* shift, void* out, int n_breaths,
+                        int c0, int out_stride, int pool, int dtype, void* stream) {
+  DARDS_CHECK_ARG(x && w && scale && shift && out, "stem_eval_fwd: null pointer");
+  DARDS_CHECK_ARG(n_breaths >= 0, "stem_eval_fwd: negative number of breaths");
+  DARDS_CHECK_ARG(pool == 0 || pool == 1, "stem_eval_fwd: pool must be 0 (max) or 1 (avg)");
+  DARDS_CHECK_ARG(out_stride >= c0, "stem_eval_fwd: row stride smaller than channel count");
+  return launch_stem_eval_fwd(x, w, scale, shift, out, n_breaths, c0, out_stride, pool, dtype, S(stream));
 }
 
 int dards_stem_bwd(const void* dout, const float* x, const float* w, const float* gamma, const float* beta,

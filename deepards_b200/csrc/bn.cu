@@ -707,6 +707,20 @@ __global__ void __launch_bounds__(256) bn_running_update_batched_kernel(const da
   running_update_block(d, ((int)blockIdx.x - d.first_block) * 64, eps, scratch);
 }
 
+// eval-mode BatchNorm as y*scale + shift for every layer of a network: thread = channel, 64 channels per block.
+// 1/sqrt (IEEE) rather than rsqrtf: a small running_var is amplified by gamma, and ATen's eval path divides by sqrt.
+__global__ void __launch_bounds__(64) bn_eval_coeffs_batched_kernel(const dards_eval_coeff_desc* __restrict__ descs, int n,
+                                                                    float eps) {
+  __shared__ dards_eval_coeff_desc d;
+  find_block_desc(descs, n, &d);
+  const int ch = ((int)blockIdx.x - d.first_block) * 64 + (int)threadIdx.x;
+  if (ch < d.c) {
+    const float sc = d.gamma[ch] / sqrtf(d.running_var[ch] + eps);
+    d.scale[ch] = sc;
+    d.shift[ch] = d.beta[ch] - d.running_mean[ch] * sc;
+  }
+}
+
 __global__ void __launch_bounds__(256) bn_running_update_kernel(dards_running_desc d, float eps) {
   __shared__ float4 scratch[256];
   running_update_block(d, (int)blockIdx.x * 64, eps, scratch);
@@ -977,6 +991,14 @@ int launch_bn_running_update_batched(const dards_running_desc* descs_dev, int n,
   if (n == 0 || total_blocks == 0) return DARDS_OK;
   bn_running_update_batched_kernel<<<total_blocks, 256, 0, st>>>(descs_dev, n, eps);
   DARDS_CHECK_LAUNCH("bn_running_update_batched");
+  return DARDS_OK;
+}
+
+int launch_bn_eval_coeffs_batched(const dards_eval_coeff_desc* descs_dev, int n, int total_blocks, float eps,
+                                  cudaStream_t st) {
+  if (n == 0 || total_blocks == 0) return DARDS_OK;
+  bn_eval_coeffs_batched_kernel<<<total_blocks, 64, 0, st>>>(descs_dev, n, eps);
+  DARDS_CHECK_LAUNCH("bn_eval_coeffs_batched");
   return DARDS_OK;
 }
 

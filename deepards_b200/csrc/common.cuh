@@ -102,6 +102,10 @@ struct ConvGemmArgs {
   long long m_total;   // n_breaths * l_dst
   int l_src, l_dst, c_red, c_cols, src_stride, dst_stride, addend_stride;
   int ktaps, q_mul, t_mul, off, div;  // source position = (q*q_mul + t*t_mul + off) / div
+  // eval-mode BatchNorm epilogue (conv_gemm_kernel<T, true> only): out = [relu](acc * scale + shift [+ addend])
+  const float* scale;
+  const float* shift;
+  int relu;
 };
 
 #define DARDS_DISPATCH_DTYPE(dtype, ...)                                  \

@@ -94,7 +94,8 @@ __global__ void __launch_bounds__(256) unpack_wgrad_batched_kernel(const dards_u
 
 constexpr int CG_BM = 128, CG_BN = 64, CG_BK = 16, CG_THREADS = 256;
 
-template <typename T>
+// AFFINE: eval-mode BatchNorm epilogue, out = [relu](acc * scale[c] + shift[c] [+ addend]) in fp32, one rounding
+template <typename T, bool AFFINE>
 __global__ void __launch_bounds__(CG_THREADS, 2) conv_gemm_kernel(ConvGemmArgs a) {
   __shared__ __align__(16) float As[2][CG_BK][CG_BM + 4];
   __shared__ __align__(16) float Bs[2][CG_BK][CG_BN];
@@ -190,14 +191,25 @@ __global__ void __launch_bounds__(CG_THREADS, 2) conv_gemm_kernel(ConvGemmArgs a
   const T* __restrict__ addend = static_cast<const T*>(a.addend);
   const int c = col0 + tx * 4;
   if (c < a.c_cols) {
+    float4 sc, sh;
+    if (AFFINE) {
+      sc = *reinterpret_cast<const float4*>(a.scale + c);
+      sh = *reinterpret_cast<const float4*>(a.shift + c);
+    }
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
       long long r = row0 + ty * 8 + i;
       if (r < a.m_total) {
         float4 v = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
+        if (AFFINE) {
+          v.x = fmaf(v.x, sc.x, sh.x); v.y = fmaf(v.y, sc.y, sh.y); v.z = fmaf(v.z, sc.z, sh.z); v.w = fmaf(v.w, sc.w, sh.w);
+        }
         if (addend) {
           float4 e = Elem<T>::ld4(addend + (size_t)r * a.addend_stride + c);
           v.x += e.x; v.y += e.y; v.z += e.z; v.w += e.w;
+        }
+        if (AFFINE && a.relu) {
+          v.x = fmaxf(v.x, 0.f); v.y = fmaxf(v.y, 0.f); v.z = fmaxf(v.z, 0.f); v.w = fmaxf(v.w, 0.f);
         }
         Elem<T>::st4(out + (size_t)r * a.dst_stride + c, v);
       }
@@ -368,7 +380,10 @@ int simt_conv_gemm(const ConvGemmArgs& a, int dtype, cudaStream_t st) {
                   "conv: row strides must be multiples of 4 elements");
   if (a.m_total == 0) return DARDS_OK;
   dim3 grid(ceil_div(a.m_total, CG_BM), ceil_div(a.c_cols, CG_BN));
-  DARDS_DISPATCH_DTYPE(dtype, { conv_gemm_kernel<T><<<grid, CG_THREADS, 0, st>>>(a); })
+  DARDS_DISPATCH_DTYPE(dtype, {
+    if (a.scale) conv_gemm_kernel<T, true><<<grid, CG_THREADS, 0, st>>>(a);
+    else conv_gemm_kernel<T, false><<<grid, CG_THREADS, 0, st>>>(a);
+  })
   DARDS_CHECK_LAUNCH("conv_gemm");
   return DARDS_OK;
 }

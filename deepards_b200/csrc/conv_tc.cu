@@ -81,11 +81,48 @@ struct TcConvParams {
   int halves;                 // 1: one store per tile; 2: two stores of nb/2 breaths through a half-size staging tile
 };
 
-template <int HALVES>
+// Eval-mode BatchNorm in the forward epilogue (AFFINE = true instantiations): every epilogue thread owns one output
+// channel, so scale / shift are two registers per tile.  The residual is read with plain loads straight from global
+// memory while the accumulator chunk is in flight: in channels-last layout the 32 lanes of a warp read 64 contiguous
+// bytes per position, and it keeps the staging tile and the TMA store path exactly as in the training kernels.
+struct TcAffine {
+  const float* scale;
+  const float* shift;
+  const __nv_bfloat16* res;  // nullable; (n_breaths, l, res_stride), never the output
+  int res_stride, relu, n_breaths, l;
+};
+
+__device__ __forceinline__ void tc_affine_coeffs(const TcAffine& af, int co, int c_cols, float& sc, float& sh) {
+  sc = co < c_cols ? af.scale[co] : 0.f;
+  sh = co < c_cols ? af.shift[co] : 0.f;
+}
+
+// residual of 16 consecutive tile columns from column c0 on: column = b*lp + m (breath n0+b, position m, valid for m < l)
+__device__ __forceinline__ void tc_res_ld16(const TcAffine& af, bool co_ok, int co, int n0, int lp, int c0, float (&r)[16]) {
+  int b = c0 / lp, m = c0 - b * lp;
+#pragma unroll
+  for (int j = 0; j < 16; ++j) {
+    const int n = n0 + b;
+    r[j] = 0.f;
+    if (af.res != nullptr && co_ok && n < af.n_breaths && m < af.l)
+      r[j] = __bfloat162float(af.res[((size_t)n * af.l + m) * af.res_stride + co]);
+    if (++m == lp) {
+      m = 0;
+      ++b;
+    }
+  }
+}
+
+__device__ __forceinline__ float tc_affine(float acc, float sc, float sh, float r, int relu) {
+  const float y = fmaf(acc, sc, sh) + r;
+  return relu ? fmaxf(y, 0.f) : y;
+}
+
+template <int HALVES, bool AFFINE>
 __global__ void __launch_bounds__(TC_THREADS, 1)
     tc_conv_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_x,
                    const __grid_constant__ CUtensorMap tm_o, __nv_bfloat16* __restrict__ out, const TcConvParams p,
-                   uint32_t desc_lbo16, uint32_t desc_sbo16, uint32_t desc_version) {
+                   uint32_t desc_lbo16, uint32_t desc_sbo16, uint32_t desc_version, const TcAffine af) {
   extern __shared__ uint8_t smem_raw[];
   // SWIZZLE_128B tiles need 1024-byte alignment
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -221,6 +258,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
       const uint32_t acc_phase = (uint32_t)(it >> 1) & 1u;
       const int co_tile = tile % p.n_co_tiles, pos_tile = tile / p.n_co_tiles;
       const int co0 = co_tile * TC_BLOCK_M, n0 = pos_tile * p.nb;
+      float a_sc = 0.f, a_sh = 0.f;
+      if (AFFINE) tc_affine_coeffs(af, co0 + cl, p.c_cols, a_sc, a_sh);
       mbar_wait(tfull_bar(buf), acc_phase);
       tc_fence_after();
       const uint32_t t_row = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)buf * TC_MAX_N;
@@ -237,12 +276,16 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
           for (int ch = (col_lo >> 4) + half; (ch << 4) < col_hi; ch += 2) {
             uint32_t v[16];
             tmem_ld16(t_row + (uint32_t)(ch << 4), v);
+            float r[16];
+            if (AFFINE) tc_res_ld16(af, co0 + cl < p.c_cols, co0 + cl, n0, p.l_tile, ch << 4, r);
             tmem_ld_wait();
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
               const int col = (ch << 4) + j;
+              float val = __uint_as_float(v[j]);
+              if (AFFINE) val = tc_affine(val, a_sc, a_sh, r[j], af.relu);
               if (HALVES == 1 || (col >= col_lo && col < col_hi))  // a 16-column chunk may straddle the two halves
-                stg[(col - col_lo) * TC_BLOCK_M + cl] = __float2bfloat16_rn(__uint_as_float(v[j]));
+                stg[(col - col_lo) * TC_BLOCK_M + cl] = __float2bfloat16_rn(val);
             }
           }
           if (h == n_halves - 1) {
@@ -275,6 +318,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
               if (n < p.n_breaths && c0 + j < n_tile) {
                 const size_t idx = ((size_t)n * p.out_l + (size_t)m * p.out_mul + p.out_off) * p.out_stride + co;
                 float val = __uint_as_float(v[j]);
+                if (AFFINE)  // forward only: output row = n * l + m
+                  val = tc_affine(val, a_sc, a_sh,
+                                  af.res ? __bfloat162float(af.res[((size_t)n * af.l + m) * af.res_stride + co]) : 0.f,
+                                  af.relu);
                 if (p.accumulate) val += __bfloat162float(out[idx]);
                 out[idx] = __float2bfloat16_rn(val);
               }
@@ -318,10 +365,11 @@ constexpr int TP_STAGE_BYTES = TC_A_BYTES + TC_B_BYTES / 2;  // 32 KB
 constexpr int TP_MAX_STAGES = 6;
 static int tp_smem_bytes(int stages) { return stages * TP_STAGE_BYTES + TC_STAGING_BYTES / 2 + 1024 + 256; }
 
+template <bool AFFINE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
     tc_conv_pair_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_x,
                         const __grid_constant__ CUtensorMap tm_o, const TcConvParams p, uint32_t desc_lbo16,
-                        uint32_t desc_sbo16, uint32_t desc_version) {
+                        uint32_t desc_sbo16, uint32_t desc_version, const TcAffine af) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const int n_stages = p.stages;
@@ -451,6 +499,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
       const uint32_t acc_phase = (uint32_t)(it >> 1) & 1u;
       const int co_tile = 2 * (job % n_co_pairs) + (int)rank, pos_tile = job / n_co_pairs;
       const int co0 = co_tile * TC_BLOCK_M, n0 = pos_tile * p.nb;
+      float a_sc = 0.f, a_sh = 0.f;
+      if (AFFINE) tc_affine_coeffs(af, co0 + cl, p.c_cols, a_sc, a_sh);
       mbar_wait(tfull_bar(buf), acc_phase);
       tc_fence_after();
       const uint32_t t_row = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)buf * TC_MAX_N;
@@ -462,11 +512,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
         for (int ch = (col_lo >> 4) + half; (ch << 4) < col_hi; ch += 2) {
           uint32_t v[16];
           tmem_ld16(t_row + (uint32_t)(ch << 4), v);
+          float r[16];
+          if (AFFINE) tc_res_ld16(af, co0 + cl < p.c_cols, co0 + cl, n0, p.l_tile, ch << 4, r);
           tmem_ld_wait();
 #pragma unroll
           for (int j = 0; j < 16; ++j) {
             const int col = (ch << 4) + j;
-            if (col >= col_lo && col < col_hi) stg[(col - col_lo) * TC_BLOCK_M + cl] = __float2bfloat16_rn(__uint_as_float(v[j]));
+            float val = __uint_as_float(v[j]);
+            if (AFFINE) val = tc_affine(val, a_sc, a_sh, r[j], af.relu);
+            if (col >= col_lo && col < col_hi) stg[(col - col_lo) * TC_BLOCK_M + cl] = __float2bfloat16_rn(val);
           }
         }
         if (h == 1) {
@@ -530,11 +584,13 @@ struct TcConv3Params {
   int n_pos_tiles, n_co_tiles;
   int accumulate;
   int src_evict_first;  // the activation tensor is read once by this launch and not again soon: L2 evict_first loads
+  int c_cols;           // valid output channels (read by the affine epilogue)
 };
 
+template <bool AFFINE>
 __global__ void __launch_bounds__(C3_THREADS, 1)
     tc_conv3_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_x,
-                    const __grid_constant__ CUtensorMap tm_o, const TcConv3Params p) {
+                    const __grid_constant__ CUtensorMap tm_o, const TcConv3Params p, const TcAffine af) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t b_base = smem_base;
@@ -678,6 +734,8 @@ __global__ void __launch_bounds__(C3_THREADS, 1)
     for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++it) {
       const int buf = it & 1;
       const int co0 = (tile % p.n_co_tiles) * TC_BLOCK_M, n0 = (tile / p.n_co_tiles) * p.nb;
+      float a_sc = 0.f, a_sh = 0.f;
+      if (AFFINE) tc_affine_coeffs(af, co0 + cl, p.c_cols, a_sc, a_sh);
       mbar_wait(tfull_bar(buf), (uint32_t)(it >> 1) & 1u);
       tc_fence_after();
       const uint32_t t_row = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)buf * TC_MAX_N;
@@ -686,9 +744,15 @@ __global__ void __launch_bounds__(C3_THREADS, 1)
       for (int ch = sub; ch < n_chunks; ch += 2) {
         uint32_t v[16];
         tmem_ld16(t_row + (uint32_t)(ch << 4), v);
+        float r[16];
+        if (AFFINE) tc_res_ld16(af, co0 + cl < p.c_cols, co0 + cl, n0, lp, ch << 4, r);
         tmem_ld_wait();
 #pragma unroll
-        for (int j = 0; j < 16; ++j) stg[((ch << 4) + j) * TC_BLOCK_M + cl] = __float2bfloat16_rn(__uint_as_float(v[j]));
+        for (int j = 0; j < 16; ++j) {
+          float val = __uint_as_float(v[j]);
+          if (AFFINE) val = tc_affine(val, a_sc, a_sh, r[j], af.relu);
+          stg[((ch << 4) + j) * TC_BLOCK_M + cl] = __float2bfloat16_rn(val);
+        }
       }
       tc_fence_before();
       __syncwarp();
@@ -827,7 +891,21 @@ struct TcProblem {
   TcConvParams p;
 };
 
-static int tc_launch(const TcProblem& q, cudaStream_t st) {
+// dynamic shared memory opt-in, once per kernel and size
+template <typename K>
+static int tc_smem_optin(K kernel, int smem_bytes, int* granted, const char* what) {
+  if (smem_bytes <= *granted) return DARDS_OK;
+  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+  if (e != cudaSuccess) {
+    set_error("%s: cannot opt in to %d bytes of shared memory: %s", what, smem_bytes, cudaGetErrorString(e));
+    return DARDS_ERR_CUDA;
+  }
+  *granted = smem_bytes;
+  return DARDS_OK;
+}
+
+// af == nullptr: the training kernels; otherwise the eval-mode BatchNorm epilogue (AFFINE instantiations)
+static int tc_launch(const TcProblem& q, cudaStream_t st, const TcAffine* af = nullptr) {
   DARDS_CHECK_ARG(q.c_red % 8 == 0 && q.src_stride % 8 == 0 && q.dst_stride % 8 == 0,
                   "tcgen05 conv: channels/strides must be multiples of 8");
   DARDS_CHECK_ARG((reinterpret_cast<uintptr_t>(q.src) & 15) == 0 && (reinterpret_cast<uintptr_t>(q.w) & 15) == 0 &&
@@ -893,47 +971,45 @@ static int tc_launch(const TcProblem& q, cudaStream_t st) {
   p.n_pos_tiles = ceil_div(q.n_breaths, p.nb);
   p.n_co_tiles = ceil_div(q.c_cols, TC_BLOCK_M);
   const int smem_bytes = tc_smem_bytes(p.stages, p.halves);
-  static int attr_smem[2] = {0, 0};
-  if (smem_bytes > attr_smem[p.halves - 1]) {
-    cudaError_t e = p.halves == 1 ? cudaFuncSetAttribute(tc_conv_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes)
-                                  : cudaFuncSetAttribute(tc_conv_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-    if (e != cudaSuccess) {
-      set_error("tcgen05 conv: cannot opt in to %d bytes of shared memory: %s", smem_bytes, cudaGetErrorString(e));
-      return DARDS_ERR_CUDA;
-    }
-    attr_smem[p.halves - 1] = smem_bytes;
-  }
   const int tiles = p.n_pos_tiles * p.n_co_tiles;
   const int grid = tiles < sm_count() ? tiles : sm_count();
   const uint32_t lbo = g_dbg_lbo >= 0 ? (uint32_t)g_dbg_lbo : 1u;
   const uint32_t sbo = g_dbg_sbo >= 0 ? (uint32_t)g_dbg_sbo : (1024u >> 4);
   const uint32_t ver = g_dbg_version >= 0 ? (uint32_t)g_dbg_version : 1u;
+  const TcAffine a = af ? *af : TcAffine{};
+  __nv_bfloat16* dst = static_cast<__nv_bfloat16*>(q.dst);
   if (pair) {
     p.stages = g_dbg_pair_stages > 0 && g_dbg_pair_stages <= TP_MAX_STAGES ? g_dbg_pair_stages : TP_MAX_STAGES;
     const int pair_smem = tp_smem_bytes(p.stages);
-    static int pair_attr = 0;
-    if (pair_smem > pair_attr) {
-      cudaError_t e = cudaFuncSetAttribute(tc_conv_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, pair_smem);
-      if (e != cudaSuccess) {
-        set_error("tcgen05 conv (CTA pairs): cannot opt in to %d bytes of shared memory: %s", pair_smem, cudaGetErrorString(e));
-        return DARDS_ERR_CUDA;
-      }
-      pair_attr = pair_smem;
-    }
+    static int pair_attr[2] = {0, 0};
+    int rc = af ? tc_smem_optin(tc_conv_pair_kernel<true>, pair_smem, &pair_attr[1], "tcgen05 conv (CTA pairs)")
+                : tc_smem_optin(tc_conv_pair_kernel<false>, pair_smem, &pair_attr[0], "tcgen05 conv (CTA pairs)");
+    if (rc) return rc;
     // one cluster of two per TPC; clusters that do not become resident at once simply start when an earlier one ends (the
     // pairs of different clusters never wait for each other)
     int clusters = sm_count() / 2;
     if (clusters > tiles / 2) clusters = tiles / 2;
-    tc_conv_pair_kernel<<<2 * clusters, TC_THREADS, pair_smem, st>>>(tm_w, tm_x, tm_o, p, lbo, sbo, ver);
+    if (af) tc_conv_pair_kernel<true><<<2 * clusters, TC_THREADS, pair_smem, st>>>(tm_w, tm_x, tm_o, p, lbo, sbo, ver, a);
+    else tc_conv_pair_kernel<false><<<2 * clusters, TC_THREADS, pair_smem, st>>>(tm_w, tm_x, tm_o, p, lbo, sbo, ver, a);
     DARDS_CHECK_LAUNCH("tc_conv_pair");
     return DARDS_OK;
   }
-  if (p.halves == 1)
-    tc_conv_kernel<1><<<grid, TC_THREADS, smem_bytes, st>>>(tm_w, tm_x, tm_o, static_cast<__nv_bfloat16*>(q.dst), p, lbo, sbo,
-                                                            ver);
-  else
-    tc_conv_kernel<2><<<grid, TC_THREADS, smem_bytes, st>>>(tm_w, tm_x, tm_o, static_cast<__nv_bfloat16*>(q.dst), p, lbo, sbo,
-                                                            ver);
+  static int attr_smem[2][2] = {{0, 0}, {0, 0}};
+  int* granted = &attr_smem[af ? 1 : 0][p.halves - 1];
+  int rc;
+  if (p.halves == 1) {
+    rc = af ? tc_smem_optin(tc_conv_kernel<1, true>, smem_bytes, granted, "tcgen05 conv")
+            : tc_smem_optin(tc_conv_kernel<1, false>, smem_bytes, granted, "tcgen05 conv");
+    if (rc) return rc;
+    if (af) tc_conv_kernel<1, true><<<grid, TC_THREADS, smem_bytes, st>>>(tm_w, tm_x, tm_o, dst, p, lbo, sbo, ver, a);
+    else tc_conv_kernel<1, false><<<grid, TC_THREADS, smem_bytes, st>>>(tm_w, tm_x, tm_o, dst, p, lbo, sbo, ver, a);
+  } else {
+    rc = af ? tc_smem_optin(tc_conv_kernel<2, true>, smem_bytes, granted, "tcgen05 conv")
+            : tc_smem_optin(tc_conv_kernel<2, false>, smem_bytes, granted, "tcgen05 conv");
+    if (rc) return rc;
+    if (af) tc_conv_kernel<2, true><<<grid, TC_THREADS, smem_bytes, st>>>(tm_w, tm_x, tm_o, dst, p, lbo, sbo, ver, a);
+    else tc_conv_kernel<2, false><<<grid, TC_THREADS, smem_bytes, st>>>(tm_w, tm_x, tm_o, dst, p, lbo, sbo, ver, a);
+  }
   DARDS_CHECK_LAUNCH("tc_conv");
   return DARDS_OK;
 }
@@ -950,7 +1026,7 @@ static bool tc3_applicable(int l, int c_red, int ktaps, int stride, int pad) {
 
 static int tc3_launch(const void* src, const void* w, void* dst, int n_breaths, int l, int c_red, int c_cols,
                       int src_stride, int dst_stride, bool reverse_taps, bool accumulate, int src_last_use,
-                      cudaStream_t st) {
+                      cudaStream_t st, const TcAffine* af = nullptr) {
   DARDS_CHECK_ARG(c_red % 8 == 0 && src_stride % 8 == 0 && dst_stride % 8 == 0,
                   "tcgen05 conv: channels/strides must be multiples of 8");
   DARDS_CHECK_ARG((reinterpret_cast<uintptr_t>(src) & 15) == 0 && (reinterpret_cast<uintptr_t>(w) & 15) == 0 &&
@@ -966,6 +1042,7 @@ static int tc3_launch(const void* src, const void* w, void* dst, int n_breaths, 
   p.k_chunks = ceil_div(c_red, TC_BLOCK_K);
   p.n_pos_tiles = ceil_div(n_breaths, nb);
   p.n_co_tiles = ceil_div(c_cols, TC_BLOCK_M);
+  p.c_cols = c_cols;
   p.accumulate = accumulate ? 1 : 0;
   // every activation byte is fetched once only when there is a single output-channel tile
   p.src_evict_first = (src_last_use && p.n_co_tiles == 1 && g_dbg_l2_hint != 0) ? 1 : 0;
@@ -992,38 +1069,36 @@ static int tc3_launch(const void* src, const void* w, void* dst, int n_breaths, 
     int rc = make_bf16_map(&tm_o, dst, 4, dims, str, box, false);
     if (rc) return rc;
   }
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(tc_conv3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, C3_SMEM_BYTES);
-    if (e != cudaSuccess) {
-      set_error("tcgen05 conv v3: cannot opt in to %d bytes of shared memory: %s", C3_SMEM_BYTES, cudaGetErrorString(e));
-      return DARDS_ERR_CUDA;
-    }
-    attr_set = true;
-  }
+  static int attr_set[2] = {0, 0};
+  const int rc = af ? tc_smem_optin(tc_conv3_kernel<true>, C3_SMEM_BYTES, &attr_set[1], "tcgen05 conv v3")
+                    : tc_smem_optin(tc_conv3_kernel<false>, C3_SMEM_BYTES, &attr_set[0], "tcgen05 conv v3");
+  if (rc) return rc;
   const int tiles = p.n_pos_tiles * p.n_co_tiles;
   const int grid = tiles < sm_count() ? tiles : sm_count();
-  tc_conv3_kernel<<<grid, C3_THREADS, C3_SMEM_BYTES, st>>>(tm_w, tm_x, tm_o, p);
+  const TcAffine a = af ? *af : TcAffine{};
+  if (af) tc_conv3_kernel<true><<<grid, C3_THREADS, C3_SMEM_BYTES, st>>>(tm_w, tm_x, tm_o, p, a);
+  else tc_conv3_kernel<false><<<grid, C3_THREADS, C3_SMEM_BYTES, st>>>(tm_w, tm_x, tm_o, p, a);
   DARDS_CHECK_LAUNCH("tc_conv3");
   return DARDS_OK;
 }
 
-int tc_conv_fwd(const void* in, const void* w_koi, void* out, const void* addend, int n_breaths, int l_in, int l_out,
-                int c_in, int c_out, int in_stride, int out_stride, int addend_stride, int ktaps, int stride, int pad,
-                int src_last_use, cudaStream_t st) {
+// forward; af != nullptr: eval-mode BatchNorm (+ residual, + ReLU) in the epilogue, through the same kernel selection
+static int tc_conv_fwd_sel(const void* in, const void* w_koi, void* out, const void* addend, int n_breaths, int l_in,
+                           int l_out, int c_in, int c_out, int in_stride, int out_stride, int addend_stride, int ktaps,
+                           int stride, int pad, int src_last_use, cudaStream_t st, const TcAffine* af) {
   DARDS_CHECK_ARG(stride == 1 || stride == 2, "tcgen05 conv: stride must be 1 or 2");
   DARDS_CHECK_ARG(ktaps <= TC_MAX_TAPS, "tcgen05 conv: at most %d taps", TC_MAX_TAPS);
   if (addend != nullptr && (addend != out || addend_stride != out_stride)) {
     set_error("tcgen05 conv: the addend must be the output itself (in-place accumulation)");
     return DARDS_ERR_UNSUPPORTED;
   }
-  if (shared_applicable(l_in, l_out, c_in, ktaps, stride, pad)) {
+  if (af == nullptr && shared_applicable(l_in, l_out, c_in, ktaps, stride, pad)) {
     const int rc = tc_conv3_shared(in, w_koi, out, n_breaths, l_in, c_in, c_out, in_stride, out_stride, false, addend != nullptr, st);
     if (rc != DARDS_ERR_UNSUPPORTED) return rc;
   }
   if (tc3_applicable(l_in, c_in, ktaps, stride, pad) && l_in == l_out)
     return tc3_launch(in, w_koi, out, n_breaths, l_in, c_in, c_out, in_stride, out_stride, false, addend != nullptr,
-                      src_last_use, st);
+                      src_last_use, st, af);
   TcProblem q{};
   q.src = in; q.w = w_koi; q.dst = out;
   q.n_breaths = n_breaths; q.l_src = l_in; q.src_planes = stride; q.l_dst = l_out; q.dst_planes = 1;
@@ -1043,7 +1118,22 @@ int tc_conv_fwd(const void* in, const void* w_koi, void* out, const void* addend
   p.nb = pick_nb_balanced(l_out, n_breaths, ceil_div(c_out, TC_BLOCK_M), p.n_taps * ceil_div(c_in, TC_BLOCK_K) >= 12);
   p.out_par = 0;
   p.accumulate = addend != nullptr;
-  return tc_launch(q, st);
+  return tc_launch(q, st, af);
+}
+
+int tc_conv_fwd(const void* in, const void* w_koi, void* out, const void* addend, int n_breaths, int l_in, int l_out,
+                int c_in, int c_out, int in_stride, int out_stride, int addend_stride, int ktaps, int stride, int pad,
+                int src_last_use, cudaStream_t st) {
+  return tc_conv_fwd_sel(in, w_koi, out, addend, n_breaths, l_in, l_out, c_in, c_out, in_stride, out_stride, addend_stride,
+                         ktaps, stride, pad, src_last_use, st, nullptr);
+}
+
+int tc_conv_affine_fwd(const void* in, const void* w_koi, void* out, const void* res, const float* scale, const float* shift,
+                       int n_breaths, int l_in, int l_out, int c_in, int c_out, int in_stride, int out_stride, int res_stride,
+                       int ktaps, int stride, int pad, int relu, int src_last_use, cudaStream_t st) {
+  const TcAffine af = {scale, shift, static_cast<const __nv_bfloat16*>(res), res_stride, relu, n_breaths, l_out};
+  return tc_conv_fwd_sel(in, w_koi, out, nullptr, n_breaths, l_in, l_out, c_in, c_out, in_stride, out_stride, 0, ktaps,
+                         stride, pad, src_last_use, st, &af);
 }
 
 int tc_conv_dgrad(const void* dout, const void* w_kio, void* din, const void* addend, int n_breaths, int l_in, int l_out,

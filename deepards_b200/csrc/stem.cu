@@ -34,7 +34,7 @@ constexpr int STEM_BS = STEM_L + 2 * STEM_PAD;       // 240: smem breath stride 
 constexpr int STEM_RUN = 28;                         // conv outputs per run; 4 runs per breath
 constexpr int STEM_FUSED_GROUP = 226;                // largest group of the one-kernel path: 226 * 240 * 4 B = 212 KB of dynamic smem
 constexpr int STEM_CHUNK = 64;                       // breaths per CTA on the chunked path
-enum { STEM_FUSED = 0, STEM_STATS = 1, STEM_APPLY = 2 };
+enum { STEM_FUSED = 0, STEM_STATS = 1, STEM_APPLY = 2, STEM_EVAL = 3 };
 
 // 16-byte asynchronous global -> shared copy (L2-only caching: the data is read once)
 __device__ __forceinline__ void stem_cp_async16(const void* smem_dst, const void* gsrc) {
@@ -102,7 +102,8 @@ __device__ __forceinline__ void stem_tap_sums(const float* xs, int group, float*
   __syncthreads();
 }
 
-// MODE: STEM_FUSED (one CTA = one whole group), STEM_STATS / STEM_APPLY (one CTA = one chunk of a group; see the header)
+// MODE: STEM_FUSED (one CTA = one whole group), STEM_STATS / STEM_APPLY (one CTA = one chunk of a group; see the header),
+// STEM_EVAL (one CTA = one chunk of breaths; eval-mode BatchNorm: `gamma` / `beta` carry the per-channel scale / shift)
 template <typename T, int MODE>
 __global__ void __launch_bounds__(STEM_THREADS)
     stem_fwd_kernel(const float* __restrict__ x, const float* __restrict__ w, const float* __restrict__ gamma,
@@ -125,59 +126,66 @@ __global__ void __launch_bounds__(STEM_THREADS)
   for (int t = 0; t < STEM_K; ++t) wr[t] = w[ch * STEM_K + t];
 
   const int n_runs = nb * (STEM_LC / STEM_RUN);
-  float mean, var;
-  if (MODE != STEM_APPLY) {
-    const float inv_n = 1.f / (float)(nb * STEM_LC);
-    stem_tap_sums(xs, nb, red, xt);
-    mean = 0.f;
-#pragma unroll
-    for (int t = 0; t < STEM_K; ++t) mean = fmaf(wr[t], xt[t], mean);
-    mean *= inv_n;
-    // ---- sweep 1: centred sum of squares ----------------------------------------------------------------
-    float q = 0.f;
-    for (int run = rl; run < n_runs; run += STEM_LANES) {
-      const float* xb = xs + (run >> 2) * STEM_BS + STEM_PAD + 2 * (run & 3) * STEM_RUN - 3;
-      float x0 = xb[0], x1 = xb[1], x2 = xb[2], x3 = xb[3], x4 = xb[4], x5 = xb[5], x6 = xb[6];
-#pragma unroll
-      for (int j = 0; j < STEM_RUN; ++j) {
-        const float d = stem_dot7(wr, x0, x1, x2, x3, x4, x5, x6) - mean;
-        q = fmaf(d, d, q);
-        const float2 nx = *reinterpret_cast<const float2*>(xb + 7 + 2 * j);  // absolute index is even
-        x0 = x2; x1 = x3; x2 = x4; x3 = x5; x4 = x6; x5 = nx.x; x6 = nx.y;
-      }
-    }
-    const float m2 = stem_lane_sum(q, red, c, rl);
-    if (MODE == STEM_STATS) {
-      if (rl == 0) {
-        float* r = part + (size_t)blockIdx.x * 3 * c0 + ch;
-        r[0] = (float)(nb * STEM_LC);
-        r[c0] = mean;
-        r[2 * c0] = m2;
-      }
-      return;
-    }
-    var = m2 * inv_n + eps;
+  float sc, sh;
+  if (MODE == STEM_EVAL) {
+    sc = gamma[ch];
+    sh = beta[ch];
   } else {
-    // Chan merge of the group's chunk records, in chunk order (every CTA of the group computes the same numbers)
-    float n = 0.f, m2 = 0.f;
-    mean = 0.f;
-    for (int kk = 0; kk < n_chunks; ++kk) {
-      const float* r = part + (size_t)(g * n_chunks + kk) * 3 * c0 + ch;
-      const float ne = r[0], me = r[c0], qe = r[2 * c0];
-      const float nn = n + ne, d = me - mean;
-      mean += d * (ne / nn);
-      m2 += qe + d * d * (n * ne / nn);
-      n = nn;
+    float mean, var;
+    if (MODE != STEM_APPLY) {
+      const float inv_n = 1.f / (float)(nb * STEM_LC);
+      stem_tap_sums(xs, nb, red, xt);
+      mean = 0.f;
+#pragma unroll
+      for (int t = 0; t < STEM_K; ++t) mean = fmaf(wr[t], xt[t], mean);
+      mean *= inv_n;
+      // ---- sweep 1: centred sum of squares ----------------------------------------------------------------
+      float q = 0.f;
+      for (int run = rl; run < n_runs; run += STEM_LANES) {
+        const float* xb = xs + (run >> 2) * STEM_BS + STEM_PAD + 2 * (run & 3) * STEM_RUN - 3;
+        float x0 = xb[0], x1 = xb[1], x2 = xb[2], x3 = xb[3], x4 = xb[4], x5 = xb[5], x6 = xb[6];
+#pragma unroll
+        for (int j = 0; j < STEM_RUN; ++j) {
+          const float d = stem_dot7(wr, x0, x1, x2, x3, x4, x5, x6) - mean;
+          q = fmaf(d, d, q);
+          const float2 nx = *reinterpret_cast<const float2*>(xb + 7 + 2 * j);  // absolute index is even
+          x0 = x2; x1 = x3; x2 = x4; x3 = x5; x4 = x6; x5 = nx.x; x6 = nx.y;
+        }
+      }
+      const float m2 = stem_lane_sum(q, red, c, rl);
+      if (MODE == STEM_STATS) {
+        if (rl == 0) {
+          float* r = part + (size_t)blockIdx.x * 3 * c0 + ch;
+          r[0] = (float)(nb * STEM_LC);
+          r[c0] = mean;
+          r[2 * c0] = m2;
+        }
+        return;
+      }
+      var = m2 * inv_n + eps;
+    } else {
+      // Chan merge of the group's chunk records, in chunk order (every CTA of the group computes the same numbers)
+      float n = 0.f, m2 = 0.f;
+      mean = 0.f;
+      for (int kk = 0; kk < n_chunks; ++kk) {
+        const float* r = part + (size_t)(g * n_chunks + kk) * 3 * c0 + ch;
+        const float ne = r[0], me = r[c0], qe = r[2 * c0];
+        const float nn = n + ne, d = me - mean;
+        mean += d * (ne / nn);
+        m2 += qe + d * d * (n * ne / nn);
+        n = nn;
+      }
+      var = m2 / n + eps;
     }
-    var = m2 / n + eps;
+    float rstd = rsqrtf(var);
+    rstd = rstd * (1.5f - 0.5f * var * rstd * rstd);
+    if (rl == 0 && k == 0) {
+      save_mean[(size_t)g * c0 + ch] = mean;
+      save_rstd[(size_t)g * c0 + ch] = rstd;
+    }
+    sc = rstd * gamma[ch];
+    sh = beta[ch] - mean * sc;
   }
-  float rstd = rsqrtf(var);
-  rstd = rstd * (1.5f - 0.5f * var * rstd * rstd);
-  if (rl == 0 && k == 0) {
-    save_mean[(size_t)g * c0 + ch] = mean;
-    save_rstd[(size_t)g * c0 + ch] = rstd;
-  }
-  const float sc = rstd * gamma[ch], sh = beta[ch] - mean * sc;
 
   // ---- sweep 2: conv + BN + ReLU + pool; run = 14 pool outputs = conv positions 2*lp0-1 .. 2*lp0+27 ----------
   for (int run = rl; run < n_runs; run += STEM_LANES) {
@@ -521,6 +529,26 @@ int launch_stem_fwd(const float* x, const float* w, const float* gamma, const fl
                                                                     eps, pool);
   })
   DARDS_CHECK_LAUNCH("stem_fwd (chunk apply)");
+  return DARDS_OK;
+}
+
+int launch_stem_eval_fwd(const float* x, const float* w, const float* scale, const float* shift, void* out, int n_breaths,
+                         int c0, int out_stride, int pool, int dtype, cudaStream_t st) {
+  DARDS_CHECK_ARG(stem_c0_ok(c0), "stem: initial planes must be a multiple of %d (got %d)", STEM_CS, c0);
+  if (n_breaths == 0) return DARDS_OK;
+  DARDS_CHECK_ARG(c0 / STEM_CS <= 65535, "stem: grid too large");
+  const int nc = ceil_div(n_breaths, STEM_CHUNK);
+  const size_t smem = (size_t)STEM_CHUNK * STEM_BS * sizeof(float);
+  dim3 grid((unsigned)nc, c0 / STEM_CS);
+  static size_t granted[2] = {44 * 1024, 44 * 1024};
+  DARDS_DISPATCH_DTYPE(dtype, {
+    int rc = stem_smem_optin(stem_fwd_kernel<T, STEM_EVAL>, smem, &granted[dtype == DARDS_BF16 ? 1 : 0]);
+    if (rc) return rc;
+    stem_fwd_kernel<T, STEM_EVAL><<<grid, STEM_THREADS, smem, st>>>(x, w, scale, shift, static_cast<T*>(out), nullptr, nullptr,
+                                                                   nullptr, n_breaths, STEM_CHUNK, nc, c0, out_stride, 0.f,
+                                                                   pool);
+  })
+  DARDS_CHECK_LAUNCH("stem_eval_fwd");
   return DARDS_OK;
 }
 

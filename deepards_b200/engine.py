@@ -107,13 +107,18 @@ class _ConvRec(object):
 
 class Plan(object):
     """See module docstring.  mode: 'backbone' (-> feat (N,F)), 'cnn_linear' (-> logits (B,2)),
-    'per_breath' (-> logits (B,group,2)), 'features' (DenseNet only, -> norm5 output (N,F,7))."""
+    'per_breath' (-> logits (B,group,2)), 'features' (DenseNet only, -> norm5 output (N,F,7)).
+    bn: 'train' (batch statistics; forward and backward) or 'eval' (ResNet only: BatchNorm with the running statistics,
+    applied in the convolution epilogues; a forward only, see _build_resnet_eval)."""
 
-    def __init__(self, net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running):
+    def __init__(self, net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running, bn="train"):
         if precision not in _DTYPES:
             raise ValueError("precision must be 'fp32' or 'bf16', got %r" % (precision,))
         if n_breaths % group != 0:
             raise ValueError("number of breaths (%d) is not a multiple of the BatchNorm group (%d)" % (n_breaths, group))
+        if bn not in ("train", "eval"):
+            raise ValueError("bn must be 'train' or 'eval', got %r" % (bn,))
+        self.bn = bn
         self.net, self.backbone, self.linear = net, backbone, linear
         self.N, self.group, self.G = n_breaths, group, n_breaths // group
         self.precision, self.mode = precision, mode
@@ -149,8 +154,10 @@ class Plan(object):
             self.goff[id(p)] = off
             off += (p.numel() + 3) // 4 * 4  # keep every slot 16-byte aligned
         self.grad_numel = off
-        self.grad_flat = self.new((max(off, 4),), torch.float32, zero=True)
+        # an eval plan has no backward: no gradient buffer
+        self.grad_flat = self.new((max(off, 4),), torch.float32, zero=True) if bn == "train" else None
         self.grad_written = set()
+        self.eval_reads = set()  # eval plans: the parameters the forward reads (the autograd inputs)
         self.param_sig = self._param_signature()
 
         # ---- I/O buffers ------------------------------------------------------------------------------------
@@ -165,14 +172,19 @@ class Plan(object):
         self._dwt_arena = None
         self._dwt_used = 0
         self._pending_unpack = []
-        if not self.simt_only and self.wgrad_mode == "accumulate":
+        if not self.simt_only and self.wgrad_mode == "accumulate" and bn == "train":
             import torch.nn as nn
             total = sum((m.weight.numel() + 3) // 4 * 4 for m in backbone.modules() if isinstance(m, nn.Conv1d))
             self._dwt_arena = self.new((max(total, 4),), torch.float32, zero=True)
         self._running = []   # (mean, rstd, bn, rows, c): running-statistics updates, one batched launch per forward
         self._pending_red = []  # (partial table, rows, c, destination pointer): flushed as one batched launch
         kind = backbone.network_name
-        if kind.startswith("resnet"):
+        if bn == "eval":
+            if not kind.startswith("resnet"):
+                raise NotImplementedError("eval-mode BatchNorm plans exist for ResNet backbones only (DenseNet's "
+                                          "BatchNorm layers keep no running statistics)")
+            self._build_resnet_eval()
+        elif kind.startswith("resnet"):
             self._build_resnet()
         elif kind.startswith("densenet"):
             self._build_densenet()
@@ -200,7 +212,10 @@ class Plan(object):
         return self._scratch[k]
 
     def _param_signature(self):
-        return tuple(p.data_ptr() for _, p in self.params)
+        sig = tuple(p.data_ptr() for _, p in self.params)
+        if self.bn == "eval":  # the recorded coefficient launch reads the running buffers through their pointers
+            sig += tuple(b.data_ptr() for _, b in self.backbone.named_buffers() if b is not None)
+        return sig
 
     def valid(self):
         return self.param_sig == self._param_signature()
@@ -635,6 +650,107 @@ class Plan(object):
         self._stem_bwd(m.conv1, m.bn1, pool, stem_st, d_out.data_ptr(), c0)
 
     # ------------------------------------------------------------------------------------------------------
+    # ResNet in eval(): BatchNorm with the running statistics, a fixed per-channel affine map per layer
+    # ------------------------------------------------------------------------------------------------------
+    def _eval_coeffs(self, bns):
+        """scale / shift (fp32, 16-byte aligned slots) of every BatchNorm layer, computed by ONE launch at the start of every
+        forward: load_state_dict() and `.data` edits change the running buffers in place, so values taken when the plan is
+        built would go stale.  Returns {id(bn): (scale pointer, shift pointer)}."""
+        import numpy as np
+        for bn in bns:
+            if getattr(bn, "running_mean", None) is None or getattr(bn, "running_var", None) is None:
+                raise NotImplementedError("eval() with a BatchNorm layer that keeps no running statistics "
+                                          "(track_running_stats=False) is not implemented on the B200 backend")
+        slots = [(bn.num_features + 3) // 4 * 4 for bn in bns]
+        coef = self.new((2, max(sum(slots), 4)), torch.float32)
+        dt = np.dtype([("gamma", "<u8"), ("beta", "<u8"), ("rm", "<u8"), ("rv", "<u8"), ("scale", "<u8"), ("shift", "<u8"),
+                       ("c", "<i4"), ("first_block", "<i4")])
+        tab = np.zeros(len(bns), dtype=dt)
+        out, off, first = {}, 0, 0
+        for i, bn in enumerate(bns):
+            sc, sh = coef[0].data_ptr() + 4 * off, coef[1].data_ptr() + 4 * off
+            tab[i] = (bn.weight.data_ptr(), bn.bias.data_ptr(), bn.running_mean.data_ptr(), bn.running_var.data_ptr(), sc, sh,
+                      bn.num_features, first)
+            out[id(bn)] = (sc, sh)
+            self.eval_reads.update((id(bn.weight), id(bn.bias)))
+            off += slots[i]
+            first += (bn.num_features + 63) // 64
+        t = torch.from_numpy(tab.view(np.uint8).copy()).to(self.device)
+        self.bufs.append(t)
+        self.fwd.add("dards_bn_eval_coeffs_batched", t.data_ptr(), len(bns), first, BN_EPS)
+        return out
+
+    def conv_affine_fwd(self, c, coef, src, src_stride, l_in, dst, relu, res=None, src_last_use=False):
+        """dst = [relu](bn_eval(conv(src)) [+ res]): one launch, BatchNorm / residual / ReLU in the convolution epilogue.
+        `dst` and `res` are (N, l_out, cout) pointers."""
+        l_out = (l_in + 2 * c.pad - c.k) // c.stride + 1
+        tc = self._tc_ok(c, "fwd")
+        w = c.koi if tc else c.kio
+        self.eval_reads.add(id(c.mod.weight))
+        self.fwd.add("dards_conv1d_affine_fwd", src, w.data_ptr(), dst, res, coef[0], coef[1], self.N, l_in, l_out, c.cin,
+                     c.cout, src_stride, c.cout, c.cout if res is not None else 0, c.k, c.stride, c.pad,
+                     (1 if relu else 0) | (_lib.HINT_LAST_USE if src_last_use else 0), self.dt, 1 if tc else 0)
+        return l_out
+
+    def _build_resnet_eval(self):
+        """Forward only: pack, coefficients, eval stem, then per block conv1 -> affine + ReLU and conv2 -> affine + residual +
+        ReLU (the downsample branch -> affine into a scratch buffer first), avgpool, head.  No statistics, no running-statistics
+        update, no gradient buffers.  Activations rotate through four buffers, each the size of the largest (N, L, C)
+        activation: block input (= identity residual), conv1 output, downsample output, block output."""
+        m = self.backbone
+        if m.double_conv_first:
+            raise NotImplementedError("resnet double_conv_first=True is not implemented on the B200 backend")
+        if self.mode == "features":
+            raise NotImplementedError("'features' mode exists for DenseNet only (gradcam.py:45 needs .features)")
+        N = self.N
+        pool = 0 if m.first_pool_type == "max" else 1
+        c0 = m.conv1.out_channels
+        if m.conv1.in_channels != 1 or m.conv1.kernel_size[0] != 7 or m.conv1.stride[0] != 2 or m.conv1.padding[0] != 3:
+            raise NotImplementedError("stem must be Conv1d(1, C0, 7, stride 2, padding 3)")
+        blocks = [blk for layer in (m.layer1, m.layer2, m.layer3, m.layer4) for blk in layer]
+        bns = [m.bn1]
+        largest, L = 56 * c0, 56
+        for blk in blocks:
+            bns += [blk.bn1, blk.bn2] + ([blk.downsample[1]] if blk.downsample is not None else [])
+            L = (L + 2 - 3) // blk.conv1.stride[0] + 1
+            largest = max(largest, L * blk.conv1.out_channels)
+        coef = self._eval_coeffs(bns)
+        pool_bufs = [self.new((N * largest,)) for _ in range(4)]
+        self.act_bytes = sum(t.numel() * t.element_size() for t in pool_bufs)
+
+        def free(*busy):
+            return next(t for t in pool_bufs if all(t is not b for b in busy))
+
+        a = pool_bufs[0]
+        self.eval_reads.add(id(m.conv1.weight))
+        self.fwd.add("dards_stem_eval_fwd", self.x_buf.data_ptr(), m.conv1.weight.data_ptr(), coef[id(m.bn1)][0],
+                     coef[id(m.bn1)][1], a.data_ptr(), N, c0, c0, pool, self.dt)
+        L, cin = 56, c0
+        for blk in blocks:
+            c1, c2 = self.conv(blk.conv1), self.conv(blk.conv2)
+            cout = c1.cout
+            a1 = free(a)
+            lo = self.conv_affine_fwd(c1, coef[id(blk.bn1)], a.data_ptr(), cin, L, a1.data_ptr(), True)
+            if blk.downsample is not None:
+                cd = self.conv(blk.downsample[0])
+                res = free(a, a1)
+                self.conv_affine_fwd(cd, coef[id(blk.downsample[1])], a.data_ptr(), cin, L, res.data_ptr(), False,
+                                     src_last_use=True)
+            else:
+                if cin != cout or c1.stride != 1:
+                    raise RuntimeError("BasicBlock without downsample must keep the shape")
+                res = a
+            out = free(a, a1, res)
+            self.conv_affine_fwd(c2, coef[id(blk.bn2)], a1.data_ptr(), cout, lo, out.data_ptr(), True, res=res.data_ptr(),
+                                 src_last_use=True)
+            a, L, cin = out, lo, cout
+        if L != 7:
+            raise RuntimeError("unexpected final length %d" % L)
+        self._head_fwd(a.data_ptr(), cin, L, cin)
+        if self.linear is not None and self.mode in ("cnn_linear", "per_breath"):
+            self.eval_reads.update((id(self.linear.weight), id(self.linear.bias)))
+
+    # ------------------------------------------------------------------------------------------------------
     # DenseNet
     # ------------------------------------------------------------------------------------------------------
     def _build_densenet(self):
@@ -880,8 +996,11 @@ class Plan(object):
         self.bwd_serial = self.fwd_serial
 
     def autograd_params(self):
-        """The parameters that receive a gradient from this plan's backward, in named_parameters() order."""
-        return [p for _, p in self.params if id(p) in self.grad_written]
+        """The parameters that receive a gradient from this plan's backward, in named_parameters() order.  An eval plan has
+        no backward: there they are the parameters its forward reads, so that an output computed with grad enabled stays
+        attached to a node whose backward says so."""
+        ids = self.grad_written if self.bn == "train" else self.eval_reads
+        return [p for _, p in self.params if id(p) in ids]
 
     def grads(self):
         """{param: gradient view} for every parameter the backward writes (fresh copy of the flat buffer)."""
@@ -894,14 +1013,16 @@ class Plan(object):
         return out
 
 
-def get_plan(net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running):
+def get_plan(net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running, bn="train"):
     """Plan cache on the owning module (invalidated when a parameter's storage moves)."""
     cache = net.__dict__.setdefault("_dards_plans", {})
     # multi-rank plans flush their pending partial-sum reductions at every all-reduce mark: a plan built before
     # init_process_group() must not be reused afterwards
     key = (n_breaths, group, precision, mode, tuple(dropout), bool(update_running), _multi_rank())
+    if bn != "train":
+        key += (bn,)
     plan = cache.get(key)
     if plan is None or not plan.valid():
-        plan = Plan(net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running)
+        plan = Plan(net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running, bn)
         cache[key] = plan
     return plan

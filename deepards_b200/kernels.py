@@ -46,6 +46,48 @@ def conv1d_fwd(x, w, stride, pad, impl=0, out=None, addend=None):
     return out
 
 
+def conv1d_affine_fwd(x, w, scale, shift, stride, pad, impl=0, res=None, relu=True, out=None):
+    """out = [relu](conv(x) * scale + shift [+ res]): eval-mode BatchNorm in the convolution epilogue."""
+    n, l, cin = x.shape
+    cout, _, k = w.shape
+    lo = (l + 2 * pad - k) // stride + 1
+    kio, koi = pack_conv_weight(w, x.dtype)
+    if out is None:
+        out = torch.empty((n, lo, cout), dtype=x.dtype, device=x.device)
+    _lib.call("dards_conv1d_affine_fwd", x.data_ptr(), (koi if impl == 1 else kio).data_ptr(), out.data_ptr(),
+              res.data_ptr() if res is not None else None, scale.data_ptr(), shift.data_ptr(), n, l, lo, cin, cout,
+              _rowstride(x), _rowstride(out), _rowstride(res) if res is not None else 0, k, stride, pad, 1 if relu else 0,
+              _dt(x), impl, _st(x))
+    return out
+
+
+def bn_eval_coeffs(layers, eps=1e-5):
+    """layers: [(gamma, beta, running_mean, running_var)] fp32 -> [(scale, shift)], one batched launch."""
+    import numpy as np
+    dt = np.dtype([("gamma", "<u8"), ("beta", "<u8"), ("rm", "<u8"), ("rv", "<u8"), ("scale", "<u8"), ("shift", "<u8"),
+                   ("c", "<i4"), ("first_block", "<i4")])
+    tab = np.zeros(len(layers), dtype=dt)
+    outs, first = [], 0
+    for i, (g, b, rm, rv) in enumerate(layers):
+        sc, sh = torch.empty_like(g), torch.empty_like(g)
+        outs.append((sc, sh))
+        tab[i] = (g.data_ptr(), b.data_ptr(), rm.data_ptr(), rv.data_ptr(), sc.data_ptr(), sh.data_ptr(), g.numel(), first)
+        first += (g.numel() + 63) // 64
+    t = torch.from_numpy(tab.view(np.uint8).copy()).to(layers[0][0].device)
+    _lib.call("dards_bn_eval_coeffs_batched", t.data_ptr(), len(layers), first, eps, _st(t))
+    torch.cuda.current_stream(t.device).synchronize()  # the table is freed on return
+    return outs
+
+
+def stem_eval_fwd(x, w, scale, shift, pool, dtype):
+    """x (N, 224) fp32 -> (N, 56, C0): conv -> y*scale + shift -> ReLU -> pool (eval-mode BatchNorm)."""
+    n, c0 = x.shape[0], w.shape[0]
+    out = torch.empty((n, 56, c0), dtype=dtype, device=x.device)
+    _lib.call("dards_stem_eval_fwd", x.data_ptr(), w.data_ptr(), scale.data_ptr(), shift.data_ptr(), out.data_ptr(), n, c0,
+              c0, pool, _DT[dtype], _st(x))
+    return out
+
+
 def conv1d_dgrad(dout, w, l_in, stride, pad, impl=0, out=None, addend=None):
     n, lo, cout = dout.shape
     _, cin, k = w.shape

@@ -95,7 +95,8 @@ class ResNet(_Picklable, nn.Module):
         return nn.Sequential(*blocks)
 
     def forward(self, x):
-        """x: (N, 1, 224) -> (N, n_out_filters); BatchNorm over all N breaths (resnet.py:141-163)."""
+        """x: (N, 1, 224) -> (N, n_out_filters); in train() BatchNorm over all N breaths (resnet.py:141-163), in eval() with
+        the running statistics (every breath on its own)."""
         if x.dim() != 3 or x.shape[1] != 1 or x.shape[2] != 224:
             raise RuntimeError("deepards_b200 ResNet expects (N, 1, 224), got %s" % (tuple(x.shape),))
         return _ag.run_plan(self, self, None, x, x.shape[0], "backbone")

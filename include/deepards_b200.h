@@ -207,6 +207,33 @@ typedef struct dards_running_desc {
 int dards_bn_running_update_batched(const dards_running_desc* descs_dev, int n_descs, int total_blocks, float eps,
                                     void* stream);
 
+/* ---- eval-mode BatchNorm (running statistics) ------------------------------------------ */
+/* nn.BatchNorm1d in eval() is a fixed per-channel affine map y*scale[c] + shift[c].  For every layer of a network in ONE
+ * launch:  scale = gamma / sqrt(running_var + eps),  shift = beta - running_mean * scale  (fp32).  Descriptor j owns
+ * ceil(c/64) blocks starting at first_block_j (first_block_0 = 0); total_blocks is their sum.  Meant to run at the start
+ * of every eval forward: the running buffers may have been edited in place since the last one. */
+typedef struct dards_eval_coeff_desc {
+  const float* gamma;
+  const float* beta;
+  const float* running_mean;
+  const float* running_var;
+  float* scale;
+  float* shift;
+  int c, first_block;
+} dards_eval_coeff_desc;
+int dards_bn_eval_coeffs_batched(const dards_eval_coeff_desc* descs_dev, int n_descs, int total_blocks, float eps,
+                                 void* stream);
+
+/* Convolution with eval-mode BatchNorm, residual add and ReLU in its epilogue (resnet.py:27-38 under eval()):
+ *   out[n,q,co] = [relu]( conv(in)[n,q,co] * scale[co] + shift[co] [+ res[n,q,co]] )
+ * computed in fp32 on the accumulator and rounded to the storage type once.  `res` may be NULL and must not overlap
+ * `out`; `relu` is 0 or 1 and may carry DARDS_HINT_LAST_USE for `in`.  Shapes, strides and `w_packed` as for
+ * dards_conv1d_fwd: impl 0 = CUDA cores (fp32 or bf16), impl 1 = tcgen05 (bf16). */
+int dards_conv1d_affine_fwd(const void* in, const void* w_packed, void* out, const void* res, const float* scale,
+                            const float* shift, int n_breaths, int l_in, int l_out, int c_in, int c_out, int in_stride,
+                            int out_stride, int res_stride, int ktaps, int stride, int pad, int relu, int dtype, int impl,
+                            void* stream);
+
 /* ---- stem: Conv1d(1->C0,k7,s2,p3) + BN + ReLU + Max/AvgPool1d(3,2,1) ---------------- */
 /* resnet.py:143-153 / densenet.py:119-123 fused: x (N,224) fp32 -> out (N,56,C0).  Nothing but the
  * group statistics is saved; the backward recomputes the convolution from x. pool: 0 max, 1 avg.
@@ -218,6 +245,10 @@ long long dards_stem_workspace_bytes(int n_groups, int group, int c0, int backwa
 int dards_stem_fwd(const float* x, const float* w, const float* gamma, const float* beta, void* out,
                    float* save_mean, float* save_rstd, int n_groups, int group, int c0, int out_stride,
                    float eps, int pool, void* workspace, long long workspace_bytes, int dtype, void* stream);
+/* Eval-mode stem: conv -> y*scale[c] + shift[c] (dards_bn_eval_coeffs_batched) -> ReLU -> pool, x (N,224) fp32 ->
+ * out (N,56,C0).  Every breath is independent of the others: any n_breaths >= 1, no workspace. */
+int dards_stem_eval_fwd(const float* x, const float* w, const float* scale, const float* shift, void* out, int n_breaths,
+                        int c0, int out_stride, int pool, int dtype, void* stream);
 /* dout (N,56,C0) -> per-group partials dw_part [n_groups][C0][7], dgamma_part/dbeta_part [n_groups][C0]. */
 int dards_stem_bwd(const void* dout, const float* x, const float* w, const float* gamma, const float* beta,
                    const float* save_mean, const float* save_rstd, float* dw_part, float* dgamma_part,
