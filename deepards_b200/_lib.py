@@ -56,6 +56,10 @@ _SIGNATURES = {
     "dards_stem_fwd": [P, P, P, P, P, P, P, I, I, I, I, F, I, P, LL, I, P],
     "dards_stem_eval_fwd": [P, P, P, P, P, I, I, I, I, I, P],
     "dards_stem_bwd": [P, P, P, P, P, P, P, P, P, P, I, I, I, I, I, P, LL, I, P],
+    "dards_bn_affine_apply": [P, P, P, P, P, P, P, P, I, I, I, I, I, I, I, I, P],
+    "dards_bn_frozen_bwd": [P, P, P, P, P, P, P, P, I, P, P, P, I, I, I, I, I, I, I, I, I, I, P],
+    "dards_stem_frozen_chunks": [I],
+    "dards_stem_frozen_bwd": [P, P, P, P, P, P, P, P, P, P, I, I, I, I, I, P],
     "dards_avgpool2_fwd": [P, P, I, I, I, I, I, I, P],
     "dards_avgpool2_bwd": [P, P, I, I, I, I, I, I, P],
     "dards_avgpool_full_fwd": [P, P, I, I, I, I, I, P],

@@ -70,8 +70,10 @@ def run_plan(net, backbone, linear, x, group, mode, dropout_key=()):
     n = x.numel() // engine.SEQ_LEN
     training = backbone.training
     # A ResNet in eval() normalises with its running statistics: every breath is independent of the rest of the batch, and
-    # `group` only shapes the heads.  DenseNet keeps no running statistics; its eval() only turns dropout off.
-    bn = "eval" if not training and backbone.network_name.startswith("resnet") else "train"
+    # `group` only shapes the heads.  A ResNet in train() with its BatchNorm layers in eval() does the same and trains
+    # (frozen BatchNorm); mixed BatchNorm states raise.  DenseNet keeps no running statistics; its eval() only turns dropout
+    # off.  engine.bn_mode states the rule.
+    bn = engine.bn_mode(backbone)
     plan = engine.get_plan(net, backbone, linear, n, group, module_precision(net), mode,
                            dropout=dropout_key if training else (), update_running=training, bn=bn)
     # Only the parameters the backward writes are inputs of the autograd node.  ResNet's conv1_alt / conv2 / bn2 never

@@ -42,6 +42,13 @@ int tc_conv_affine_fwd(const void* in, const void* w_koi, void* out, const void*
 int launch_bn_eval_coeffs_batched(const dards_eval_coeff_desc*, int, int, float, cudaStream_t);
 int launch_stem_eval_fwd(const float*, const float*, const float*, const float*, void*, int, int, int, int, int,
                          cudaStream_t);
+int launch_bn_affine_apply(const void*, void*, const void*, const float*, const float*, const void*, const float*,
+                           const float*, int, int, int, int, int, int, int, int, cudaStream_t);
+int launch_bn_frozen_bwd(const void*, const void*, const void*, const float*, const float*, const float*, const float*,
+                         void*, int, void*, float*, float*, int, int, int, int, int, int, int, int, int, int, cudaStream_t);
+int stem_frozen_chunks(int n_breaths);
+int launch_stem_frozen_bwd(const void*, const float*, const float*, const float*, const float*, const float*, const float*,
+                           float*, float*, float*, int, int, int, int, int, cudaStream_t);
 int tc_conv_wgrad_accum(const void* in, const void* dout, float* dw_t, int n_breaths, int l_in, int l_out, int c_in, int c_out,
                         int in_stride, int dout_stride, int ktaps, int stride, int pad, cudaStream_t st);
 int simt_unpack_wgrad_batched(const dards_unpack_desc*, int, int, cudaStream_t);
@@ -389,6 +396,42 @@ int dards_stem_eval_fwd(const float* x, const float* w, const float* scale, cons
   DARDS_CHECK_ARG(pool == 0 || pool == 1, "stem_eval_fwd: pool must be 0 (max) or 1 (avg)");
   DARDS_CHECK_ARG(out_stride >= c0, "stem_eval_fwd: row stride smaller than channel count");
   return launch_stem_eval_fwd(x, w, scale, shift, out, n_breaths, c0, out_stride, pool, dtype, S(stream));
+}
+
+int dards_bn_affine_apply(const void* y, void* out, const void* res, const float* scale, const float* shift,
+                          const void* y2, const float* scale2, const float* shift2, int rows, int c, int y_stride,
+                          int out_stride, int res_stride, int y2_stride, int relu, int dtype, void* stream) {
+  DARDS_CHECK_ARG(relu == 0 || relu == 1, "bn_affine_apply: relu must be 0 or 1");
+  DARDS_CHECK_ARG(dtype == DARDS_F32 || dtype == DARDS_BF16, "bn_affine_apply: unknown dtype %d", dtype);
+  return launch_bn_affine_apply(y, out, res, scale, shift, y2, scale2, shift2, rows, c, y_stride, out_stride, res_stride,
+                                y2_stride, relu, dtype, S(stream));
+}
+
+int dards_bn_frozen_bwd(const void* dout, const void* y, const void* mask_src, const float* scale, const float* shift,
+                        const float* running_mean, const float* rstd, void* dx, int accumulate_dx, void* dres,
+                        float* dgamma_part, float* dbeta_part, int n_tiles, int rows_per_tile, int c, int dout_stride,
+                        int y_stride, int mask_stride, int dx_stride, int dres_stride, int relu_mode, int dtype,
+                        void* stream) {
+  DARDS_CHECK_ARG(dout && y && scale && shift && running_mean && rstd && dx, "bn_frozen_bwd: null pointer");
+  DARDS_CHECK_ARG(relu_mode >= 0 && relu_mode <= 2, "bn_frozen_bwd: relu_mode must be 0, 1 or 2");
+  DARDS_CHECK_ARG(n_tiles >= 0 && rows_per_tile > 0 && c > 0, "bn_frozen_bwd: bad shape");
+  return launch_bn_frozen_bwd(dout, y, mask_src, scale, shift, running_mean, rstd, dx, accumulate_dx, dres, dgamma_part,
+                              dbeta_part, n_tiles, rows_per_tile, c, dout_stride, y_stride, mask_stride, dx_stride,
+                              dres_stride, relu_mode, dtype, S(stream));
+}
+
+int dards_stem_frozen_chunks(int n_breaths) { return stem_frozen_chunks(n_breaths); }
+
+int dards_stem_frozen_bwd(const void* dout, const float* x, const float* w, const float* scale, const float* shift,
+                          const float* running_mean, const float* rstd, float* dw_part, float* dgamma_part,
+                          float* dbeta_part, int n_breaths, int c0, int dout_stride, int pool, int dtype, void* stream) {
+  DARDS_CHECK_ARG(dout && x && w && scale && shift && running_mean && rstd && dw_part && dgamma_part && dbeta_part,
+                  "stem_frozen_bwd: null pointer");
+  DARDS_CHECK_ARG(n_breaths >= 0, "stem_frozen_bwd: negative number of breaths");
+  DARDS_CHECK_ARG(pool == 0 || pool == 1, "stem_frozen_bwd: pool must be 0 (max) or 1 (avg)");
+  DARDS_CHECK_ARG(dout_stride >= c0, "stem_frozen_bwd: row stride smaller than channel count");
+  return launch_stem_frozen_bwd(dout, x, w, scale, shift, running_mean, rstd, dw_part, dgamma_part, dbeta_part, n_breaths,
+                                c0, dout_stride, pool, dtype, S(stream));
 }
 
 int dards_stem_bwd(const void* dout, const float* x, const float* w, const float* gamma, const float* beta,

@@ -253,7 +253,11 @@ __global__ void __launch_bounds__(THREADS)
 }
 
 // NT = number of cached tensors: 2 (gradient, x) or 3 (+ the ReLU mask source of relu_mode 2)
-template <typename T, int VPR, int THREADS, int RELU_MODE>
+// FROZEN: BatchNorm with constant statistics (nn.BatchNorm1d in eval() under a network in train(): running statistics).
+// `gamma` / `beta` carry the forward's per-channel scale / shift (dards_bn_eval_coeffs_batched), `save_mean` / `save_rstd`
+// the per-channel running_mean and 1/sqrt(running_var + eps); a "group" is just a tile of rows.  dx = scale * g: there
+// is no mean-of-gradient term, and the per-tile sums are partials of dbeta / dgamma only.
+template <typename T, int VPR, int THREADS, int RELU_MODE, bool FROZEN = false>
 __global__ void __launch_bounds__(THREADS)
     gbn_bwd_cached_kernel(const T* dout, const T* x, const T* mask_src, const float* __restrict__ gamma,
                           const float* __restrict__ beta, const float* __restrict__ save_mean,
@@ -322,10 +326,17 @@ __global__ void __launch_bounds__(THREADS)
     if (active) {
 #pragma unroll
       for (int j = 0; j < V; ++j) {
-        mean[j] = save_mean[(size_t)g * c + c0 + j];
-        rstd[j] = save_rstd[(size_t)g * c + c0 + j];
-        sc[j] = rstd[j] * gamma[c0 + j];          // same arithmetic as the forward: y = fmaf(x, sc, sh)
-        sh[j] = beta[c0 + j] - mean[j] * sc[j];
+        if (FROZEN) {
+          mean[j] = save_mean[c0 + j];
+          rstd[j] = save_rstd[c0 + j];
+          sc[j] = gamma[c0 + j];
+          sh[j] = beta[c0 + j];
+        } else {
+          mean[j] = save_mean[(size_t)g * c + c0 + j];
+          rstd[j] = save_rstd[(size_t)g * c + c0 + j];
+          sc[j] = rstd[j] * gamma[c0 + j];          // same arithmetic as the forward: y = fmaf(x, sc, sh)
+          sh[j] = beta[c0 + j] - mean[j] * sc[j];
+        }
       }
       // ---- sweep 1 (shared): mask the gradient in place, accumulate sum g and sum g*(x - mean) ----
       T* drp = dres ? dres + row0 * dres_stride + c0 : nullptr;
@@ -374,13 +385,13 @@ __global__ void __launch_bounds__(THREADS)
           if (dgamma_part) dgamma_part[(size_t)g * c + c0 + j] = acc[V + j];
         }
       }
-      // dx = sc*(g - m1 - xhat*m2) = sc*g + kb*x + kc
+      // dx = sc*(g - m1 - xhat*m2) = sc*g + kb*x + kc  (FROZEN: dx = sc*g)
       float kb[V], kc[V];
 #pragma unroll
       for (int j = 0; j < V; ++j) {
         const float m1 = acc[j] * inv_n, m2 = acc[V + j] * inv_n;
-        kb[j] = -sc[j] * m2 * rstd[j];
-        kc[j] = -sc[j] * m1 - kb[j] * mean[j];
+        kb[j] = FROZEN ? 0.f : -sc[j] * m2 * rstd[j];
+        kc[j] = FROZEN ? 0.f : -sc[j] * m1 - kb[j] * mean[j];
       }
       // ---- sweep 2 (shared -> global): dx; refill the cache with the next tile ----
       T* dxp = dx + row0 * dx_stride + c0;
@@ -402,7 +413,7 @@ __global__ void __launch_bounds__(THREADS)
         Vec<T>::unpack(rg, gv);
         Vec<T>::unpack(rx, xv);
 #pragma unroll
-        for (int j = 0; j < V; ++j) o[j] = fmaf(sc[j], gv[j], fmaf(kb[j], xv[j], kc[j]));
+        for (int j = 0; j < V; ++j) o[j] = FROZEN ? sc[j] * gv[j] : fmaf(sc[j], gv[j], fmaf(kb[j], xv[j], kc[j]));
         if (accumulate_dx) {
           float e[V];
           Vec<T>::unpack(ro, e);
@@ -526,7 +537,7 @@ __global__ void __launch_bounds__(BN_THREADS)
   }
 }
 
-template <typename T>
+template <typename T, bool FROZEN = false>  // FROZEN: as in gbn_bwd_cached_kernel
 __global__ void __launch_bounds__(BN_THREADS)
     gbn_bwd_kernel(const T* dout, const T* x, const T* mask_src, const float* __restrict__ gamma,
                    const float* __restrict__ beta, const float* __restrict__ save_mean, const float* __restrict__ save_rstd,
@@ -549,11 +560,12 @@ __global__ void __launch_bounds__(BN_THREADS)
   float mean[V], rstd[V], sc[V], sh[V];
 #pragma unroll
   for (int j = 0; j < V; ++j) {
-    mean[j] = active ? save_mean[(size_t)g * c + c0 + j] : 0.f;
-    rstd[j] = active ? save_rstd[(size_t)g * c + c0 + j] : 0.f;
+    const size_t so = FROZEN ? 0 : (size_t)g * c;
+    mean[j] = active ? save_mean[so + c0 + j] : 0.f;
+    rstd[j] = active ? save_rstd[so + c0 + j] : 0.f;
     const float gm = active ? gamma[c0 + j] : 0.f, bt = active ? beta[c0 + j] : 0.f;
-    sc[j] = rstd[j] * gm;
-    sh[j] = bt - mean[j] * sc[j];
+    sc[j] = FROZEN ? gm : rstd[j] * gm;
+    sh[j] = FROZEN ? bt : bt - mean[j] * sc[j];
   }
   auto load_row = [&](int r, float (&gv)[V], float (&xv)[V]) {
     Vec<T>::unpack(ld16(gp + (size_t)r * dout_stride), gv);
@@ -598,8 +610,8 @@ __global__ void __launch_bounds__(BN_THREADS)
 #pragma unroll
   for (int j = 0; j < V; ++j) {
     const float m1 = s1[j] * inv_n, m2 = s2[j] * inv_n;
-    kb[j] = -sc[j] * m2 * rstd[j];
-    kc[j] = -sc[j] * m1 - kb[j] * mean[j];
+    kb[j] = FROZEN ? 0.f : -sc[j] * m2 * rstd[j];
+    kc[j] = FROZEN ? 0.f : -sc[j] * m1 - kb[j] * mean[j];
   }
   T* dxp = dx + row_base * dx_stride + c0;
   T* drp = dres ? dres + row_base * dres_stride + c0 : nullptr;
@@ -607,7 +619,7 @@ __global__ void __launch_bounds__(BN_THREADS)
     float gv[V], xv[V], o[V];
     load_row(r, gv, xv);
 #pragma unroll
-    for (int j = 0; j < V; ++j) o[j] = fmaf(sc[j], gv[j], fmaf(kb[j], xv[j], kc[j]));
+    for (int j = 0; j < V; ++j) o[j] = FROZEN ? sc[j] * gv[j] : fmaf(sc[j], gv[j], fmaf(kb[j], xv[j], kc[j]));
     if (drp) st16(drp + (size_t)r * dres_stride, Vec<T>::pack(gv));
     if (accumulate_dx) {
       float e[V];
@@ -854,31 +866,31 @@ static int run_fwd_cached(const void* x, void* out, const void* res, const float
 #undef BN_FWD_V
 }
 
-template <typename T, int VPR, int THREADS, int RELU_MODE>
+template <typename T, int VPR, int THREADS, int RELU_MODE, bool FROZEN>
 static int run_bwd_cached_v(const void* dout, const void* x, const void* mask_src, const float* gamma, const float* beta,
                             const float* save_mean, const float* save_rstd, void* dx, int accumulate_dx, void* dres,
                             float* dgamma_part, float* dbeta_part, int n_groups, int rows, int c, int dout_stride,
                             int x_stride, int mask_stride, int dx_stride, int dres_stride, cudaStream_t st) {
   static size_t granted = 24 * 1024;
   const size_t smem = (size_t)ceil_div(rows, THREADS / VPR) * THREADS * 16 * (RELU_MODE == 2 ? 3 : 2);
-  int rc = bn_smem_optin(gbn_bwd_cached_kernel<T, VPR, THREADS, RELU_MODE>, smem, &granted);
+  int rc = bn_smem_optin(gbn_bwd_cached_kernel<T, VPR, THREADS, RELU_MODE, FROZEN>, smem, &granted);
   if (rc) return rc;
   const int n_tiles = ceil_div(c, VPR * Vec<T>::N) * n_groups;
   const int grid = bn_persistent_grid(smem, (THREADS / 32 + 1) * VPR * 2 * Vec<T>::N * 4, THREADS, n_tiles);
-  gbn_bwd_cached_kernel<T, VPR, THREADS, RELU_MODE><<<grid, THREADS, smem, st>>>(
+  gbn_bwd_cached_kernel<T, VPR, THREADS, RELU_MODE, FROZEN><<<grid, THREADS, smem, st>>>(
       static_cast<const T*>(dout), static_cast<const T*>(x), static_cast<const T*>(mask_src), gamma, beta, save_mean,
       save_rstd, static_cast<T*>(dx), accumulate_dx, static_cast<T*>(dres), dgamma_part, dbeta_part, n_groups, rows, c,
       dout_stride, x_stride, mask_stride, dx_stride, dres_stride, g_dbg_l2_hint != 0 ? 1 : 0);
   return DARDS_OK;
 }
 
-template <typename T, int VPR, int THREADS>
+template <typename T, int VPR, int THREADS, bool FROZEN>
 static int run_bwd_cached(const void* dout, const void* x, const void* mask_src, const float* gamma, const float* beta,
                           const float* save_mean, const float* save_rstd, void* dx, int accumulate_dx, void* dres,
                           float* dgamma_part, float* dbeta_part, int n_groups, int rows, int c, int dout_stride,
                           int x_stride, int mask_stride, int dx_stride, int dres_stride, int relu_mode, cudaStream_t st) {
 #define BN_BWD_V(M)                                                                                                     \
-  return run_bwd_cached_v<T, VPR, THREADS, M>(dout, x, mask_src, gamma, beta, save_mean, save_rstd, dx, accumulate_dx, \
+  return run_bwd_cached_v<T, VPR, THREADS, M, FROZEN>(dout, x, mask_src, gamma, beta, save_mean, save_rstd, dx, accumulate_dx, \
                                               dres, dgamma_part, dbeta_part, n_groups, rows, c, dout_stride, x_stride, \
                                               mask_stride, dx_stride, dres_stride, st)
   if (relu_mode == 0) BN_BWD_V(0);
@@ -926,38 +938,59 @@ int launch_gbn_fwd(const void* x, void* out, const void* res, const float* gamma
   return DARDS_OK;
 }
 
-int launch_gbn_bwd(const void* dout, const void* x, const void* mask_src, const float* gamma, const float* beta,
-                   const float* save_mean, const float* save_rstd, void* dx, int accumulate_dx, void* dres,
-                   float* dgamma_part, float* dbeta_part, int n_groups, int rows, int c, int dout_stride, int x_stride,
-                   int mask_stride, int dx_stride, int dres_stride, int relu_mode, int dtype, cudaStream_t st) {
+// shared by the batch-statistics backward (launch_gbn_bwd) and the constant-statistics one (launch_bn_frozen_bwd)
+template <bool FROZEN>
+static int run_gbn_bwd(const char* name, const void* dout, const void* x, const void* mask_src, const float* gamma,
+                       const float* beta, const float* save_mean, const float* save_rstd, void* dx, int accumulate_dx,
+                       void* dres, float* dgamma_part, float* dbeta_part, int n_groups, int rows, int c, int dout_stride,
+                       int x_stride, int mask_stride, int dx_stride, int dres_stride, int relu_mode, int dtype,
+                       cudaStream_t st) {
   const int v = vec_of(dtype);
   DARDS_CHECK_ARG(c % v == 0 && dout_stride % v == 0 && x_stride % v == 0 && dx_stride % v == 0,
-                  "gbn_bwd: channels and strides must be multiples of %d", v);
-  DARDS_CHECK_ARG(relu_mode != 2 || (mask_src && mask_stride % v == 0), "gbn_bwd: relu_mode 2 needs mask_src");
-  DARDS_CHECK_ARG(!dres || dres_stride % v == 0, "gbn_bwd: dres stride");
+                  "%s: channels and strides must be multiples of %d", name, v);
+  DARDS_CHECK_ARG(relu_mode != 2 || (mask_src && mask_stride % v == 0), "%s: relu_mode 2 needs mask_src", name);
+  DARDS_CHECK_ARG(!dres || dres_stride % v == 0, "%s: dres stride", name);
   if (n_groups == 0) return DARDS_OK;
-  DARDS_CHECK_ARG(n_groups <= 65535, "gbn_bwd: too many groups (%d)", n_groups);
+  DARDS_CHECK_ARG(n_groups <= 65535, "%s: too many groups (%d)", name, n_groups);
   const int cfg = bn_pick_cfg(rows, c, v, relu_mode == 2 ? 3 : 2);
   if (cfg >= 0) {
     int rc = DARDS_OK;
     DARDS_DISPATCH_DTYPE(dtype, {
-      BN_DISPATCH_CFG(cfg, (rc = run_bwd_cached<T, VPR, THREADS>(dout, x, mask_src, gamma, beta, save_mean, save_rstd, dx,
-                                                                 accumulate_dx, dres, dgamma_part, dbeta_part, n_groups, rows,
-                                                                 c, dout_stride, x_stride, mask_stride, dx_stride,
-                                                                 dres_stride, relu_mode, st)));
+      BN_DISPATCH_CFG(cfg, (rc = run_bwd_cached<T, VPR, THREADS, FROZEN>(dout, x, mask_src, gamma, beta, save_mean, save_rstd,
+                                                                         dx, accumulate_dx, dres, dgamma_part, dbeta_part,
+                                                                         n_groups, rows, c, dout_stride, x_stride,
+                                                                         mask_stride, dx_stride, dres_stride, relu_mode, st)));
     })
     if (rc) return rc;
   } else {
     dim3 grid(ceil_div(c, BN_QUADS * v), n_groups);
     DARDS_DISPATCH_DTYPE(dtype, {
-      gbn_bwd_kernel<T><<<grid, BN_THREADS, 0, st>>>(
+      gbn_bwd_kernel<T, FROZEN><<<grid, BN_THREADS, 0, st>>>(
           static_cast<const T*>(dout), static_cast<const T*>(x), static_cast<const T*>(mask_src), gamma, beta, save_mean,
           save_rstd, static_cast<T*>(dx), accumulate_dx, static_cast<T*>(dres), dgamma_part, dbeta_part, rows, c,
           dout_stride, x_stride, mask_stride, dx_stride, dres_stride, relu_mode);
     })
   }
-  DARDS_CHECK_LAUNCH("gbn_bwd");
+  DARDS_CHECK_LAUNCH(name);
   return DARDS_OK;
+}
+
+int launch_gbn_bwd(const void* dout, const void* x, const void* mask_src, const float* gamma, const float* beta,
+                   const float* save_mean, const float* save_rstd, void* dx, int accumulate_dx, void* dres,
+                   float* dgamma_part, float* dbeta_part, int n_groups, int rows, int c, int dout_stride, int x_stride,
+                   int mask_stride, int dx_stride, int dres_stride, int relu_mode, int dtype, cudaStream_t st) {
+  return run_gbn_bwd<false>("gbn_bwd", dout, x, mask_src, gamma, beta, save_mean, save_rstd, dx, accumulate_dx, dres,
+                            dgamma_part, dbeta_part, n_groups, rows, c, dout_stride, x_stride, mask_stride, dx_stride,
+                            dres_stride, relu_mode, dtype, st);
+}
+
+int launch_bn_frozen_bwd(const void* dout, const void* y, const void* mask_src, const float* scale, const float* shift,
+                         const float* running_mean, const float* rstd, void* dx, int accumulate_dx, void* dres,
+                         float* dgamma_part, float* dbeta_part, int n_tiles, int rows, int c, int dout_stride, int y_stride,
+                         int mask_stride, int dx_stride, int dres_stride, int relu_mode, int dtype, cudaStream_t st) {
+  return run_gbn_bwd<true>("bn_frozen_bwd", dout, y, mask_src, scale, shift, running_mean, rstd, dx, accumulate_dx, dres,
+                           dgamma_part, dbeta_part, n_tiles, rows, c, dout_stride, y_stride, mask_stride, dx_stride,
+                           dres_stride, relu_mode, dtype, st);
 }
 
 int launch_reduce_rows(const float* part, float* out, int rows, int c, int accumulate, cudaStream_t st) {

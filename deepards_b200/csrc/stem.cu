@@ -222,7 +222,13 @@ __device__ __forceinline__ int stem_r_index(int a, int b) {  // a <= b
 // slots 47 % busy).  Groups too large for the extra 35 KB per 20 breaths use the direct path.
 // PARTIAL: one CTA = one chunk of a group; the moments and the per-channel sums go to the workspace instead of through
 // section C (stem_bwd_combine_kernel finishes the group).
-template <typename T, bool STAGE, bool PARTIAL>
+// FROZEN (the STEM_FROZEN backward of a network in train() whose BatchNorm is in eval()): constant statistics; one CTA = one
+// chunk of breaths (n_chunks chunks of a single "group" of all breaths).  `gamma` / `beta` carry the per-channel scale / shift
+// that dards_stem_eval_fwd applied, `save_mean` / `save_rstd` the running_mean and 1/sqrt(running_var + eps).  The pre-pool
+// values are recomputed with exactly STEM_EVAL's arithmetic, fmaxf(fmaf(stem_dot7(..), scale, shift), 0), so the max-pool
+// arg-max is the forward's.  No input moments are needed: dy = scale * g, so dW_t = scale * G_t; the chunk's S1 (dbeta),
+// S2 (dgamma) and scale * G_t (dW) are written as partials, row blockIdx.x, for the batched row reduction.
+template <typename T, bool STAGE, bool PARTIAL, bool FROZEN = false>
 __global__ void __launch_bounds__(STEM_THREADS)
     stem_bwd_kernel(const T* __restrict__ dout, const float* __restrict__ x, const float* __restrict__ w,
                     const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ save_mean,
@@ -255,7 +261,7 @@ __global__ void __launch_bounds__(STEM_THREADS)
   const int n_conv = group * STEM_LC;
 
   // ---- A. channel-independent input moments: X_t = sum xin_t, R[a][b] = sum xin_a * xin_b --------------
-  {
+  if (!FROZEN) {
     float acc[STEM_K + STEM_NR];
 #pragma unroll
     for (int i = 0; i < STEM_K + STEM_NR; ++i) acc[i] = 0.f;
@@ -301,7 +307,7 @@ __global__ void __launch_bounds__(STEM_THREADS)
   for (int t = 0; t < STEM_K; ++t) wr[t] = w[ch * STEM_K + t];
   const float mean = save_mean[(size_t)g * c0 + ch], rstd = save_rstd[(size_t)g * c0 + ch];
   const float gm = gamma[ch];
-  const float sc = rstd * gm, sh = beta[ch] - mean * sc;
+  const float sc = FROZEN ? gm : rstd * gm, sh = FROZEN ? beta[ch] : beta[ch] - mean * sc;
   float s1 = 0.f, s2 = 0.f, gt[STEM_K];
 #pragma unroll
   for (int t = 0; t < STEM_K; ++t) gt[t] = 0.f;
@@ -390,6 +396,14 @@ __global__ void __launch_bounds__(STEM_THREADS)
       o[c0] = s2;
 #pragma unroll
       for (int t = 0; t < STEM_K; ++t) o[(size_t)(2 + t) * c0] = gt[t];
+      return;
+    }
+    if (FROZEN) {
+      const size_t o = (size_t)blockIdx.x * c0 + ch;
+      dbeta_part[o] = s1;
+      dgamma_part[o] = s2;
+#pragma unroll
+      for (int t = 0; t < STEM_K; ++t) dw_part[o * STEM_K + t] = sc * gt[t];
       return;
     }
     // ---- C. BN backward folded into the weight gradient ------------------------------------------------
@@ -560,12 +574,12 @@ struct StemBwdArgs {
   int group, chunk, n_chunks, c0, dout_stride, pool;
 };
 
-template <typename T, bool STAGE, bool PARTIAL>
+template <typename T, bool STAGE, bool PARTIAL, bool FROZEN = false>
 static int stem_bwd_run(const StemBwdArgs<T>& a, dim3 grid, size_t smem, cudaStream_t st) {
   static size_t granted = 36 * 1024;  // 9.4 KB of static smem on top
-  int rc = stem_smem_optin(stem_bwd_kernel<T, STAGE, PARTIAL>, smem, &granted);
+  int rc = stem_smem_optin(stem_bwd_kernel<T, STAGE, PARTIAL, FROZEN>, smem, &granted);
   if (rc) return rc;
-  stem_bwd_kernel<T, STAGE, PARTIAL><<<grid, STEM_THREADS, smem, st>>>(a.dout, a.x, a.w, a.gamma, a.beta, a.save_mean,
+  stem_bwd_kernel<T, STAGE, PARTIAL, FROZEN><<<grid, STEM_THREADS, smem, st>>>(a.dout, a.x, a.w, a.gamma, a.beta, a.save_mean,
                                                                       a.save_rstd, a.dw_part, a.dgamma_part, a.dbeta_part,
                                                                       a.mom_part, a.ch_part, a.group, a.chunk, a.n_chunks,
                                                                       a.c0, a.dout_stride, a.pool);
@@ -614,6 +628,32 @@ int launch_stem_bwd(const void* dout, const float* x, const float* w, const floa
                                                    dbeta_part, group, nc, c0);
     DARDS_CHECK_LAUNCH("stem_bwd (chunk combine)");
   }
+  return DARDS_OK;
+}
+
+int stem_frozen_chunks(int n_breaths) { return n_breaths > 0 ? ceil_div(n_breaths, STEM_CHUNK) : 0; }
+
+int launch_stem_frozen_bwd(const void* dout, const float* x, const float* w, const float* scale, const float* shift,
+                           const float* running_mean, const float* rstd, float* dw_part, float* dgamma_part,
+                           float* dbeta_part, int n_breaths, int c0, int dout_stride, int pool, int dtype, cudaStream_t st) {
+  DARDS_CHECK_ARG(stem_c0_ok(c0), "stem: initial planes must be a multiple of %d (got %d)", STEM_CS, c0);
+  if (n_breaths == 0) return DARDS_OK;
+  DARDS_CHECK_ARG(c0 / STEM_CS <= 65535, "stem: grid too large");
+  const int nc = stem_frozen_chunks(n_breaths);
+  const size_t smem_x = (size_t)STEM_CHUNK * STEM_BS * sizeof(float);
+  dim3 grid((unsigned)nc, c0 / STEM_CS);
+  int rc = DARDS_OK;
+  DARDS_DISPATCH_DTYPE(dtype, {
+    const size_t smem_d = (size_t)STEM_CHUNK * STEM_LP * STEM_CS * sizeof(T);
+    const bool stage = (dout_stride * sizeof(T)) % 16 == 0 && (reinterpret_cast<uintptr_t>(dout) & 15) == 0 &&
+                       smem_x + smem_d <= 200 * 1024;
+    const size_t smem = smem_x + (stage ? smem_d : 0);
+    const StemBwdArgs<T> a = {static_cast<const T*>(dout), x, w, scale, shift, running_mean, rstd, dw_part, dgamma_part,
+                              dbeta_part, nullptr, nullptr, n_breaths, STEM_CHUNK, nc, c0, dout_stride, pool};
+    rc = stage ? stem_bwd_run<T, true, false, true>(a, grid, smem, st) : stem_bwd_run<T, false, false, true>(a, grid, smem, st);
+  })
+  if (rc) return rc;
+  DARDS_CHECK_LAUNCH("stem_frozen_bwd");
   return DARDS_OK;
 }
 

@@ -177,14 +177,17 @@ class DataParallelTrainer(object):
         mode = "per_breath" if isinstance(net, CNNSingleBreathLinearNetwork) else "cnn_linear"
         n = x.numel() // engine.SEQ_LEN
         training = bb.training
-        if not training and bb.network_name.startswith("resnet"):
-            # the same guard as the autograd path (autograd.run_plan): eval() on the reference ResNet normalises with the
-            # running statistics, which this backend does not implement -- never silently a different function
-            raise NotImplementedError("deepards_b200 ResNet implements training-mode BatchNorm (batch statistics) only; "
-                                      "keep the module in train() mode as train_ards_detector.py does")
+        # the same rule as the autograd path (autograd.run_plan, engine.bn_mode): batch statistics, or frozen running
+        # statistics when every BatchNorm layer of a ResNet in train() is in eval(); mixed states raise
+        bn = engine.bn_mode(bb)
+        if bn == "eval":
+            # a ResNet in eval() is inference only (its backward raises on the autograd path as well)
+            raise NotImplementedError("deepards_b200: DataParallelTrainer trains a ResNet in train() mode only (BatchNorm "
+                                      "layers all in train(), or all in eval() to fine-tune with frozen statistics); "
+                                      "this one is in eval()")
         from .autograd import module_precision
         plan = engine.get_plan(net, bb, net.linear_final, n, x.shape[1], module_precision(net), mode,
-                               dropout=_drop_key(bb) if training else (), update_running=training)
+                               dropout=_drop_key(bb) if training else (), update_running=training, bn=bn)
         if getattr(plan, "_dp_ranges", None) is None:
             live = set(i for i in plan.grad_written
                        if any(id(p) == i and p.requires_grad for _, p, _ in self.layout))

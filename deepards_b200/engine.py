@@ -75,6 +75,45 @@ class nvtx_range(object):
             torch.cuda.nvtx.range_pop()
 
 
+def resnet_bn_layers(backbone):
+    """(name, module) of the BatchNorm layers a ResNet's forward uses (resnet.py:141-163): the stem's bn1 and every block's
+    bn1 / bn2 / downsample BatchNorm.  The stem's bn2 (built by the constructor, never called) is not one of them."""
+    out = [("bn1", backbone.bn1)]
+    for li, layer in enumerate((backbone.layer1, backbone.layer2, backbone.layer3, backbone.layer4), 1):
+        for bi, blk in enumerate(layer):
+            pre = "layer%d.%d." % (li, bi)
+            out += [(pre + "bn1", blk.bn1), (pre + "bn2", blk.bn2)]
+            if blk.downsample is not None:
+                out.append((pre + "downsample.1", blk.downsample[1]))
+    return out
+
+
+def bn_mode(backbone):
+    """Which BatchNorm a plan for `backbone` implements, from the module's own training flags, as nn.BatchNorm1d would:
+      'train'  -- batch statistics, running statistics updated (every DenseNet; a ResNet in train() with its BatchNorm
+                  layers in train());
+      'frozen' -- a ResNet in train() with every BatchNorm layer in eval(): normalised with the running statistics, which
+                  stay untouched, and still back-propagated into gamma, beta and the convolutions (fine-tuning with frozen
+                  BatchNorm);
+      'eval'   -- a ResNet in eval(): inference with the running statistics, whatever its BatchNorm layers say.
+    A ResNet in train() with some BatchNorm layers in train() and others in eval() raises NotImplementedError.
+    DenseNet's BatchNorm layers keep no running statistics, so torch normalises with batch statistics in either state."""
+    if not backbone.network_name.startswith("resnet"):
+        return "train"
+    if not backbone.training:
+        return "eval"
+    layers = resnet_bn_layers(backbone)
+    frozen = [n for n, m in layers if not m.training]
+    if not frozen:
+        return "train"
+    if len(frozen) == len(layers):
+        return "frozen"
+    training = [n for n, m in layers if m.training]
+    raise NotImplementedError("deepards_b200: a ResNet in train() needs its BatchNorm layers all in train() (batch "
+                              "statistics) or all in eval() (frozen running statistics); in train(): %s; in eval(): %s"
+                              % (", ".join(training), ", ".join(frozen)))
+
+
 class Recorder(object):
     """A replayable list of C-ABI calls."""
 
@@ -108,16 +147,17 @@ class _ConvRec(object):
 class Plan(object):
     """See module docstring.  mode: 'backbone' (-> feat (N,F)), 'cnn_linear' (-> logits (B,2)),
     'per_breath' (-> logits (B,group,2)), 'features' (DenseNet only, -> norm5 output (N,F,7)).
-    bn: 'train' (batch statistics; forward and backward) or 'eval' (ResNet only: BatchNorm with the running statistics,
-    applied in the convolution epilogues; a forward only, see _build_resnet_eval)."""
+    bn: 'train' (batch statistics; forward and backward), 'eval' (ResNet only: BatchNorm with the running statistics,
+    applied in the convolution epilogues; a forward only, see _build_resnet_eval) or 'frozen' (ResNet only: BatchNorm with
+    the running statistics, forward and backward, no running-statistics update; see bn_mode and _build_resnet)."""
 
     def __init__(self, net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running, bn="train"):
         if precision not in _DTYPES:
             raise ValueError("precision must be 'fp32' or 'bf16', got %r" % (precision,))
         if n_breaths % group != 0:
             raise ValueError("number of breaths (%d) is not a multiple of the BatchNorm group (%d)" % (n_breaths, group))
-        if bn not in ("train", "eval"):
-            raise ValueError("bn must be 'train' or 'eval', got %r" % (bn,))
+        if bn not in ("train", "eval", "frozen"):
+            raise ValueError("bn must be 'train', 'eval' or 'frozen', got %r" % (bn,))
         self.bn = bn
         self.net, self.backbone, self.linear = net, backbone, linear
         self.N, self.group, self.G = n_breaths, group, n_breaths // group
@@ -155,7 +195,7 @@ class Plan(object):
             off += (p.numel() + 3) // 4 * 4  # keep every slot 16-byte aligned
         self.grad_numel = off
         # an eval plan has no backward: no gradient buffer
-        self.grad_flat = self.new((max(off, 4),), torch.float32, zero=True) if bn == "train" else None
+        self.grad_flat = self.new((max(off, 4),), torch.float32, zero=True) if bn != "eval" else None
         self.grad_written = set()
         self.eval_reads = set()  # eval plans: the parameters the forward reads (the autograd inputs)
         self.param_sig = self._param_signature()
@@ -172,17 +212,17 @@ class Plan(object):
         self._dwt_arena = None
         self._dwt_used = 0
         self._pending_unpack = []
-        if not self.simt_only and self.wgrad_mode == "accumulate" and bn == "train":
+        if not self.simt_only and self.wgrad_mode == "accumulate" and bn != "eval":
             import torch.nn as nn
             total = sum((m.weight.numel() + 3) // 4 * 4 for m in backbone.modules() if isinstance(m, nn.Conv1d))
             self._dwt_arena = self.new((max(total, 4),), torch.float32, zero=True)
         self._running = []   # (mean, rstd, bn, rows, c): running-statistics updates, one batched launch per forward
         self._pending_red = []  # (partial table, rows, c, destination pointer): flushed as one batched launch
         kind = backbone.network_name
+        if bn != "train" and not kind.startswith("resnet"):
+            raise NotImplementedError("running-statistics BatchNorm plans exist for ResNet backbones only (DenseNet's "
+                                      "BatchNorm layers keep no running statistics)")
         if bn == "eval":
-            if not kind.startswith("resnet"):
-                raise NotImplementedError("eval-mode BatchNorm plans exist for ResNet backbones only (DenseNet's "
-                                          "BatchNorm layers keep no running statistics)")
             self._build_resnet_eval()
         elif kind.startswith("resnet"):
             self._build_resnet()
@@ -213,7 +253,7 @@ class Plan(object):
 
     def _param_signature(self):
         sig = tuple(p.data_ptr() for _, p in self.params)
-        if self.bn == "eval":  # the recorded coefficient launch reads the running buffers through their pointers
+        if self.bn != "train":  # the recorded coefficient launch reads the running buffers through their pointers
             sig += tuple(b.data_ptr() for _, b in self.backbone.named_buffers() if b is not None)
         return sig
 
@@ -317,7 +357,10 @@ class Plan(object):
 
     def gbn_fwd(self, bn, x, x_stride, out, out_stride, rows, c, relu, res=None, res_stride=0, x_last_use=True):
         """x_last_use: x is a convolution output that nothing else reads before the backward pass (False for DenseNet's
-        concatenation buffer, which the following layers read again)."""
+        concatenation buffer, which the following layers read again).
+        Frozen plans: the affine map of the running statistics over all G * rows rows; returns the layer's coefficients."""
+        if self.bn == "frozen":
+            return self.bn_affine_apply(bn, x, x_stride, out, out_stride, self.G * rows, c, relu, res, res_stride)
         mean, rstd = self.stats(c)
         self.fwd.add("dards_gbn_fwd", x, out, res, bn.weight.data_ptr(), bn.bias.data_ptr(), mean.data_ptr(),
                      rstd.data_ptr(), self.G, rows, c, x_stride, out_stride, res_stride, BN_EPS,
@@ -335,8 +378,8 @@ class Plan(object):
         2: BatchNorm (+ residual, + ReLU) entirely in the convolution epilogue.
         merged_branch: the layer is one of the two branches of a downsample block, whose two BatchNorms + add + ReLU
         become ONE elementwise pass in mode 1 (fuse_bn "3" enables mode 1 for those only)."""
-        if self.simt_only or self.fuse_bn == "0" or not self._tc_ok(c, "fwd"):
-            return 0
+        if self.simt_only or self.fuse_bn == "0" or self.bn == "frozen" or not self._tc_ok(c, "fwd"):
+            return 0  # (the fused kernel takes batch statistics)
         mode = _lib.fn("dards_conv1d_bn_mode")(*self._cb_shape(c, l_in), self.dt)
         if mode == 1 and not (self.fuse_bn == "1" or (merged_branch and self.fuse_bn == "3")):
             return 0
@@ -403,6 +446,41 @@ class Plan(object):
         self._note_running(bn, st[0], st[1], rows, cout)
         return st, std
 
+    # ---- frozen BatchNorm (running statistics under train()) -------------------------------------------------
+    def bn_affine_apply(self, bn, y, y_stride, out, out_stride, rows, c, relu, res=None, res_stride=0, second=None):
+        """out = [relu](bn(y) [+ res] [+ bn_d(y_d)]) with the running statistics; second = (bn_d, y_d pointer, stride)."""
+        co = self._coef[id(bn)]
+        y2, s2, h2, y2s = None, None, None, 0
+        if second is not None:
+            bnd, y2, y2s = second
+            s2, h2 = self._coef[id(bnd)][:2]
+        self.fwd.add("dards_bn_affine_apply", y, out, res, co[0], co[1], y2, s2, h2, rows, c, y_stride, out_stride,
+                     res_stride if res is not None else 0, y2s, 1 if relu else 0, self.dt)
+        return co
+
+    @staticmethod
+    def _frozen_tile_rows(total, c):
+        """Rows per tile of a frozen BatchNorm backward: the largest divisor of `total` up to the tile of the training
+        kernels (rows * C = 71680, at most 1120 rows), so that the whole tile fits the cached kernel."""
+        target = min(1120, max(8, 71680 // c), total)
+        for d in range(target, 0, -1):
+            if total % d == 0:
+                return d
+        return 1
+
+    def _frozen_bwd(self, bn, co, dout, dout_stride, y, y_stride, dx, dx_stride, rows, c, relu_mode, mask, mask_stride,
+                    accumulate, dres, dres_stride):
+        total = self.G * rows
+        tile = self._frozen_tile_rows(total, c)
+        n_tiles = total // tile
+        dg = self.new((n_tiles, c), torch.float32)
+        db = self.new((n_tiles, c), torch.float32)
+        self.bwd.add("dards_bn_frozen_bwd", dout, y, mask, co[0], co[1], co[3], co[2], dx, 1 if accumulate else 0, dres,
+                     dg.data_ptr(), db.data_ptr(), n_tiles, tile, c, dout_stride, y_stride, mask_stride, dx_stride,
+                     dres_stride, relu_mode, self.dt)
+        self._pending_red.append((dg, n_tiles, c, self.gptr(bn.weight)))
+        self._pending_red.append((db, n_tiles, c, self.gptr(bn.bias)))
+
     def _note_running(self, bn, mean, rstd, rows, c):
         if self.update_running and getattr(bn, "running_mean", None) is not None:
             self._running.append((mean, rstd, bn, rows, c))
@@ -467,6 +545,9 @@ class Plan(object):
 
     def gbn_bwd(self, bn, st, dout, dout_stride, x, x_stride, dx, dx_stride, rows, c, relu_mode, mask=None,
                 mask_stride=0, accumulate=False, dres=None, dres_stride=0):
+        if self.bn == "frozen":
+            return self._frozen_bwd(bn, st, dout, dout_stride, x, x_stride, dx, dx_stride, rows, c, relu_mode, mask,
+                                    mask_stride, accumulate, dres, dres_stride)
         mean, rstd = st
         dg = self.new((self.G, c), torch.float32)   # per layer: they live until the next flush
         db = self.new((self.G, c), torch.float32)
@@ -483,6 +564,11 @@ class Plan(object):
         c0 = conv.out_channels
         if conv.in_channels != 1 or conv.kernel_size[0] != 7 or conv.stride[0] != 2 or conv.padding[0] != 3:
             raise NotImplementedError("stem must be Conv1d(1, C0, 7, stride 2, padding 3)")
+        if self.bn == "frozen":
+            co = self._coef[id(bn)]
+            self.fwd.add("dards_stem_eval_fwd", self.x_buf.data_ptr(), conv.weight.data_ptr(), co[0], co[1], out, self.N,
+                         c0, out_stride, pool, self.dt)
+            return co
         mean, rstd = self.stats(c0)
         # a BatchNorm group that does not fit the fused stem's shared memory (a flat batch of more than 226 breaths is ONE
         # group) runs in chunks and needs a workspace for the chunk records (stem.cu)
@@ -502,6 +588,18 @@ class Plan(object):
 
     def _stem_bwd(self, conv, bn, pool, st, dout, dout_stride):
         c0 = conv.out_channels
+        if self.bn == "frozen":
+            nc = _lib.fn("dards_stem_frozen_chunks")(self.N)
+            dwp = self.new((nc, c0 * 7), torch.float32)
+            dgp = self.new((nc, c0), torch.float32)
+            dbp = self.new((nc, c0), torch.float32)
+            self.bwd.add("dards_stem_frozen_bwd", dout, self.x_buf.data_ptr(), conv.weight.data_ptr(), st[0], st[1], st[3],
+                         st[2], dwp.data_ptr(), dgp.data_ptr(), dbp.data_ptr(), self.N, c0, dout_stride, pool, self.dt)
+            self._pending_red.append((dwp, nc, c0 * 7, self.gptr(conv.weight)))
+            self._pending_red.append((dgp, nc, c0, self.gptr(bn.weight)))
+            self._pending_red.append((dbp, nc, c0, self.gptr(bn.bias)))
+            self._flush_reductions()
+            return
         mean, rstd = st
         dwp = self.new((self.G, c0 * 7), torch.float32)
         dgp = self.new((self.G, c0), torch.float32)
@@ -557,6 +655,9 @@ class Plan(object):
         N = self.N
         pool = 0 if m.first_pool_type == "max" else 1
         c0 = m.conv1.out_channels
+        if self.bn == "frozen":
+            # scale / shift / rstd of every layer from the running buffers, computed at the start of every forward
+            self._coef = self._eval_coeffs([bn for _, bn in resnet_bn_layers(m)], with_rstd=True)
         a = self.new((N, 56, c0))
         stem_st = self._stem(m.conv1, m.bn1, pool, a.data_ptr(), c0)
         L = 56
@@ -583,6 +684,13 @@ class Plan(object):
                     if m2 and self.cb_mode(cd, L, True) == m2:
                         st2, std = self.conv_bn_fwd(c2, blk.bn2, a1.data_ptr(), cout, lo, y2, out, True, src_last_use=True,
                                                     ds=(cd, blk.downsample[1], a.data_ptr(), cin, L, yd), merged_branch=True)
+                    elif self.bn == "frozen":
+                        # out = relu(bn2(y2) + bn_d(y_d)): one pass over both branches
+                        self.conv_fwd(c2, a1.data_ptr(), cout, y2.data_ptr(), cout, lo, src_last_use=True)
+                        self.conv_fwd(cd, a.data_ptr(), cin, yd.data_ptr(), cout, L)
+                        st2 = self.bn_affine_apply(blk.bn2, y2.data_ptr(), cout, out.data_ptr(), cout, N * lo, cout, True,
+                                                   second=(blk.downsample[1], yd.data_ptr(), cout))
+                        std = self._coef[id(blk.downsample[1])]
                     else:
                         self.conv_fwd(c2, a1.data_ptr(), cout, y2.data_ptr(), cout, lo, src_last_use=True)
                         self.conv_fwd(cd, a.data_ptr(), cin, yd.data_ptr(), cout, L)
@@ -652,32 +760,46 @@ class Plan(object):
     # ------------------------------------------------------------------------------------------------------
     # ResNet in eval(): BatchNorm with the running statistics, a fixed per-channel affine map per layer
     # ------------------------------------------------------------------------------------------------------
-    def _eval_coeffs(self, bns):
+    def _eval_coeffs(self, bns, with_rstd=False):
         """scale / shift (fp32, 16-byte aligned slots) of every BatchNorm layer, computed by ONE launch at the start of every
         forward: load_state_dict() and `.data` edits change the running buffers in place, so values taken when the plan is
-        built would go stale.  Returns {id(bn): (scale pointer, shift pointer)}."""
+        built would go stale.  Returns {id(bn): (scale pointer, shift pointer)}.
+        with_rstd (frozen plans, whose backward needs the normalised input): the same launch also evaluates every layer with
+        gamma = 1, beta = 0, i.e. rstd = 1/sqrt(running_var + eps); returns {id(bn): (scale, shift, rstd, running_mean)}."""
         import numpy as np
         for bn in bns:
             if getattr(bn, "running_mean", None) is None or getattr(bn, "running_var", None) is None:
                 raise NotImplementedError("eval() with a BatchNorm layer that keeps no running statistics "
                                           "(track_running_stats=False) is not implemented on the B200 backend")
         slots = [(bn.num_features + 3) // 4 * 4 for bn in bns]
-        coef = self.new((2, max(sum(slots), 4)), torch.float32)
+        coef = self.new((4 if with_rstd else 2, max(sum(slots), 4)), torch.float32)
+        if with_rstd:
+            unit = self.new((2, max(bn.num_features for bn in bns)), torch.float32)
+            unit[0].fill_(1.0)
+            unit[1].zero_()
         dt = np.dtype([("gamma", "<u8"), ("beta", "<u8"), ("rm", "<u8"), ("rv", "<u8"), ("scale", "<u8"), ("shift", "<u8"),
                        ("c", "<i4"), ("first_block", "<i4")])
-        tab = np.zeros(len(bns), dtype=dt)
+        tab = np.zeros(len(bns) * (2 if with_rstd else 1), dtype=dt)
         out, off, first = {}, 0, 0
         for i, bn in enumerate(bns):
             sc, sh = coef[0].data_ptr() + 4 * off, coef[1].data_ptr() + 4 * off
             tab[i] = (bn.weight.data_ptr(), bn.bias.data_ptr(), bn.running_mean.data_ptr(), bn.running_var.data_ptr(), sc, sh,
                       bn.num_features, first)
             out[id(bn)] = (sc, sh)
+            if with_rstd:
+                rs, nsh = coef[2].data_ptr() + 4 * off, coef[3].data_ptr() + 4 * off
+                tab[len(bns) + i] = (unit[0].data_ptr(), unit[1].data_ptr(), bn.running_mean.data_ptr(),
+                                     bn.running_var.data_ptr(), rs, nsh, bn.num_features, 0)
+                out[id(bn)] = (sc, sh, rs, bn.running_mean.data_ptr())
             self.eval_reads.update((id(bn.weight), id(bn.bias)))
             off += slots[i]
             first += (bn.num_features + 63) // 64
+        for i in range(len(bns), len(tab)):  # the rstd descriptors follow the scale / shift ones
+            tab[i]["first_block"] = first
+            first += (int(tab[i]["c"]) + 63) // 64
         t = torch.from_numpy(tab.view(np.uint8).copy()).to(self.device)
         self.bufs.append(t)
-        self.fwd.add("dards_bn_eval_coeffs_batched", t.data_ptr(), len(bns), first, BN_EPS)
+        self.fwd.add("dards_bn_eval_coeffs_batched", t.data_ptr(), len(tab), first, BN_EPS)
         return out
 
     def conv_affine_fwd(self, c, coef, src, src_stride, l_in, dst, relu, res=None, src_last_use=False):
@@ -999,7 +1121,7 @@ class Plan(object):
         """The parameters that receive a gradient from this plan's backward, in named_parameters() order.  An eval plan has
         no backward: there they are the parameters its forward reads, so that an output computed with grad enabled stays
         attached to a node whose backward says so."""
-        ids = self.grad_written if self.bn == "train" else self.eval_reads
+        ids = self.eval_reads if self.bn == "eval" else self.grad_written
         return [p for _, p in self.params if id(p) in ids]
 
     def grads(self):

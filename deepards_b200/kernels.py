@@ -88,6 +88,64 @@ def stem_eval_fwd(x, w, scale, shift, pool, dtype):
     return out
 
 
+def _reduce_rows(part):
+    """(rows, c) fp32 partials -> (c,) sums in a fixed order."""
+    rows, c = part.shape
+    out = torch.empty((c,), dtype=torch.float32, device=part.device)
+    _lib.call("dards_reduce_rows", part.data_ptr(), out.data_ptr(), rows, c, 0, _st(part))
+    return out
+
+
+def bn_affine_apply(y, scale, shift, res=None, relu=True, second=None, out=None):
+    """out = [relu](y * scale + shift [+ res] [+ y2 * scale2 + shift2]) over (N, L, C) rows (BatchNorm with the running
+    statistics); second = (y2, scale2, shift2)."""
+    n, l, c = y.shape
+    if out is None:
+        out = torch.empty((n, l, c), dtype=y.dtype, device=y.device)
+    y2, s2, h2 = second if second is not None else (None, None, None)
+    _lib.call("dards_bn_affine_apply", y.data_ptr(), out.data_ptr(), res.data_ptr() if res is not None else None,
+              scale.data_ptr(), shift.data_ptr(), y2.data_ptr() if y2 is not None else None,
+              s2.data_ptr() if s2 is not None else None, h2.data_ptr() if h2 is not None else None, n * l, c, _rowstride(y),
+              _rowstride(out), _rowstride(res) if res is not None else 0, _rowstride(y2) if y2 is not None else 0,
+              1 if relu else 0, _dt(y), _st(y))
+    return out
+
+
+def bn_frozen_bwd(dout, y, scale, shift, running_mean, rstd, relu_mode, mask_src=None, want_dres=False, dx=None,
+                  accumulate=False, tile_rows=None):
+    """Backward of bn_affine_apply with constant statistics: -> (dx, dgamma, dbeta, dres or None).  `dx` may be given
+    (and accumulated into); tile_rows splits the N*L rows into tiles for the partial sums (default: one tile per breath)."""
+    n, l, c = y.shape
+    rows = n * l
+    tile = tile_rows or l
+    assert rows % tile == 0
+    tiles = rows // tile
+    if dx is None:
+        dx = torch.empty_like(y)
+    dres = torch.empty_like(dout) if want_dres else None
+    dg = torch.empty((tiles, c), dtype=torch.float32, device=y.device)
+    db = torch.empty((tiles, c), dtype=torch.float32, device=y.device)
+    _lib.call("dards_bn_frozen_bwd", dout.data_ptr(), y.data_ptr(), mask_src.data_ptr() if mask_src is not None else None,
+              scale.data_ptr(), shift.data_ptr(), running_mean.data_ptr(), rstd.data_ptr(), dx.data_ptr(),
+              1 if accumulate else 0, dres.data_ptr() if dres is not None else None, dg.data_ptr(), db.data_ptr(), tiles, tile,
+              c, _rowstride(dout), _rowstride(y), _rowstride(mask_src) if mask_src is not None else 0, _rowstride(dx),
+              _rowstride(dres) if dres is not None else 0, relu_mode, _dt(y), _st(y))
+    return dx, _reduce_rows(dg), _reduce_rows(db), dres
+
+
+def stem_frozen_bwd(dout, x, w, scale, shift, running_mean, rstd, pool):
+    """dout (N, 56, C0) of stem_eval_fwd -> (dW (C0, 1, 7), dgamma, dbeta) with constant statistics."""
+    n, c0 = x.shape[0], w.shape[0]
+    nc = _lib.fn("dards_stem_frozen_chunks")(n)
+    dwp = torch.empty((nc, c0 * 7), dtype=torch.float32, device=x.device)
+    dgp = torch.empty((nc, c0), dtype=torch.float32, device=x.device)
+    dbp = torch.empty((nc, c0), dtype=torch.float32, device=x.device)
+    _lib.call("dards_stem_frozen_bwd", dout.data_ptr(), x.data_ptr(), w.data_ptr(), scale.data_ptr(), shift.data_ptr(),
+              running_mean.data_ptr(), rstd.data_ptr(), dwp.data_ptr(), dgp.data_ptr(), dbp.data_ptr(), n, c0, _rowstride(dout),
+              pool, _dt(dout), _st(x))
+    return _reduce_rows(dwp).view(c0, 1, 7), _reduce_rows(dgp), _reduce_rows(dbp)
+
+
 def conv1d_dgrad(dout, w, l_in, stride, pad, impl=0, out=None, addend=None):
     n, lo, cout = dout.shape
     _, cin, k = w.shape

@@ -234,6 +234,29 @@ int dards_conv1d_affine_fwd(const void* in, const void* w_packed, void* out, con
                             int out_stride, int res_stride, int ktaps, int stride, int pad, int relu, int dtype, int impl,
                             void* stream);
 
+/* ---- BatchNorm with constant statistics under training (frozen BatchNorm) ------------- */
+/* A network in train() whose nn.BatchNorm1d layers are in eval() (the usual fine-tuning idiom, resnet.py:27-38 and
+ * 146-153 with running statistics): the forward is the eval-mode affine map, and the backward reaches gamma, beta and
+ * the convolutions through it.
+ * Elementwise forward: out = [relu]( y*scale[c] + shift[c] [+ res] [+ y2*scale2[c] + shift2[c]] ) over `rows` rows,
+ * in fp32, rounded once; scale / shift as from dards_bn_eval_coeffs_batched.  The second operand is the downsample
+ * branch of a ResNet block (resnet.py:34-38), so relu(bn2(y2) + bn_d(y_d)) is one pass.  fp32 or bf16; c and every
+ * stride a multiple of 4 (fp32) / 8 (bf16), tensors 16-byte aligned; `out` must not overlap y, res or y2. */
+int dards_bn_affine_apply(const void* y, void* out, const void* res, const float* scale, const float* shift,
+                          const void* y2, const float* scale2, const float* shift2, int rows, int c, int y_stride,
+                          int out_stride, int res_stride, int y2_stride, int relu, int dtype, void* stream);
+/* Its backward, rows split into n_tiles tiles of rows_per_tile rows (any split: tiles only shape the partial sums):
+ *   g = dout [* (mask)]    relu_mode 0: none, 1: y*scale + shift > 0 (recomputed), 2: mask_src > 0
+ *   dres (optional) = g;   dx (+)= g * scale     (scale = gamma * rstd: no mean-of-gradient terms)
+ *   dbeta_part[t][c] = sum over tile t of g,   dgamma_part[t][c] = sum over tile t of g * (y - running_mean) * rstd
+ * with rstd = 1/sqrt(running_var + eps), which dards_bn_eval_coeffs_batched computes as `scale` for gamma = 1, beta = 0.
+ * The partials are summed with dards_reduce_rows[_batched] (fixed order: deterministic).  dx may alias dout. */
+int dards_bn_frozen_bwd(const void* dout, const void* y, const void* mask_src, const float* scale, const float* shift,
+                        const float* running_mean, const float* rstd, void* dx, int accumulate_dx, void* dres,
+                        float* dgamma_part, float* dbeta_part, int n_tiles, int rows_per_tile, int c, int dout_stride,
+                        int y_stride, int mask_stride, int dx_stride, int dres_stride, int relu_mode, int dtype,
+                        void* stream);
+
 /* ---- stem: Conv1d(1->C0,k7,s2,p3) + BN + ReLU + Max/AvgPool1d(3,2,1) ---------------- */
 /* resnet.py:143-153 / densenet.py:119-123 fused: x (N,224) fp32 -> out (N,56,C0).  Nothing but the
  * group statistics is saved; the backward recomputes the convolution from x. pool: 0 max, 1 avg.
@@ -249,6 +272,14 @@ int dards_stem_fwd(const float* x, const float* w, const float* gamma, const flo
  * out (N,56,C0).  Every breath is independent of the others: any n_breaths >= 1, no workspace. */
 int dards_stem_eval_fwd(const float* x, const float* w, const float* scale, const float* shift, void* out, int n_breaths,
                         int c0, int out_stride, int pool, int dtype, void* stream);
+/* Backward of dards_stem_eval_fwd for a network in train() with the stem's BatchNorm in eval(): dout (N,56,C0) ->
+ * partials dw_part [n_chunks][C0][7], dgamma_part / dbeta_part [n_chunks][C0] over chunks of 64 breaths,
+ * n_chunks = dards_stem_frozen_chunks(n_breaths), summed with dards_reduce_rows[_batched].  scale / shift: the
+ * forward's; rstd = 1/sqrt(running_var + eps) (see dards_bn_frozen_bwd).  Any n_breaths, no workspace. */
+int dards_stem_frozen_chunks(int n_breaths);
+int dards_stem_frozen_bwd(const void* dout, const float* x, const float* w, const float* scale, const float* shift,
+                          const float* running_mean, const float* rstd, float* dw_part, float* dgamma_part,
+                          float* dbeta_part, int n_breaths, int c0, int dout_stride, int pool, int dtype, void* stream);
 /* dout (N,56,C0) -> per-group partials dw_part [n_groups][C0][7], dgamma_part/dbeta_part [n_groups][C0]. */
 int dards_stem_bwd(const void* dout, const float* x, const float* w, const float* gamma, const float* beta,
                    const float* save_mean, const float* save_rstd, float* dw_part, float* dgamma_part,
