@@ -7,6 +7,8 @@ import ctypes
 import os
 from ctypes import c_double, c_float, c_int, c_longlong, c_ulonglong, c_void_p
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libdeepards_b200.so")
 
@@ -23,6 +25,57 @@ class GradcamDesc(ctypes.Structure):
                                         "seq_raw", "seq_u8", "read_resized", "seq_resized", "conv_out", "grad_out")] + \
                [(n, c_int) for n in ("a_stride", "target", "n_groups", "group", "l", "f", "n_out", "resized_len", "dtype",
                                      "reserved")]
+
+
+# Descriptors of the batched entry points, read from a DEVICE array (desc_table).  Each kernel gives descriptor j the
+# blocks [first_block_j, first_block_j + blocks()).
+class _ChannelBlocks(ctypes.Structure):
+    def blocks(self):  # one per 64 channels
+        return (self.c + 63) // 64
+
+
+class _TileBlocks(ctypes.Structure):
+    def blocks(self):  # one per 32 x 32 tile of the (c_out, c_in) weight plane
+        return ((self.c_out + 31) // 32) * ((self.c_in + 31) // 32)
+
+
+class PackDesc(_TileBlocks):
+    """dards_pack_desc."""
+    _fields_ = [("w", P), ("w_kio", P), ("w_koi", P), ("c_out", I), ("c_in", I), ("ktaps", I), ("first_block", I)]
+
+
+class UnpackDesc(_TileBlocks):
+    """dards_unpack_desc."""
+    _fields_ = [("dw_t", P), ("dw", P), ("c_out", I), ("c_in", I), ("ktaps", I), ("first_block", I)]
+
+
+class ReduceDesc(_ChannelBlocks):
+    """dards_reduce_desc."""
+    _fields_ = [("part", P), ("out", P), ("rows", I), ("c", I), ("accumulate", I), ("first_block", I)]
+
+
+class RunningDesc(_ChannelBlocks):
+    """dards_running_desc."""
+    _fields_ = [("save_mean", P), ("save_rstd", P), ("running_mean", P), ("running_var", P), ("num_batches_tracked", P),
+                ("n_groups", I), ("rows_per_group", I), ("c", I), ("momentum", F), ("first_block", I), ("reserved", I)]
+
+
+class EvalCoeffDesc(_ChannelBlocks):
+    """dards_eval_coeff_desc."""
+    _fields_ = [("gamma", P), ("beta", P), ("running_mean", P), ("running_var", P), ("scale", P), ("shift", P),
+                ("c", I), ("first_block", I)]
+
+
+def desc_table(layout, rows, device):
+    """rows -> (uint8 tensor on `device` holding one `layout` descriptor per row, total_blocks).  A row gives the fields
+    before first_block in declaration order (pointers as ints, None for NULL); first_block is the running sum of the
+    blocks of the rows before it, and fields after it are 0."""
+    tab = (layout * len(rows))(*[layout(*r) for r in rows])
+    total = 0
+    for d in tab:
+        d.first_block = total
+        total += d.blocks()
+    return torch.frombuffer(bytearray(tab), dtype=torch.uint8).to(device), total
 
 
 # name -> argtypes (all functions return int unless listed in _RESTYPES)

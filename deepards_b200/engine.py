@@ -16,6 +16,7 @@ Reference semantics implemented here (file:line in /root/reference/deepards):
   models/torch_cnn_linear_network.py:57-67, 104-113   per-breath and per-sequence linear heads
 """
 import os
+from collections import namedtuple
 
 import torch
 
@@ -142,6 +143,11 @@ class Recorder(object):
 
 class _ConvRec(object):
     __slots__ = ("mod", "cin", "cout", "k", "stride", "pad", "kio", "koi", "goff", "dwt")
+
+
+# A BatchNorm layer applied with its running statistics (Plan._eval_coeffs): pointers to its fp32 scale and shift, and, for
+# frozen plans, whose backward needs them, to rstd = 1/sqrt(running_var + eps) and running_mean (None in eval plans).
+Coef = namedtuple("Coef", "scale shift rstd mean")
 
 
 class Plan(object):
@@ -453,8 +459,8 @@ class Plan(object):
         y2, s2, h2, y2s = None, None, None, 0
         if second is not None:
             bnd, y2, y2s = second
-            s2, h2 = self._coef[id(bnd)][:2]
-        self.fwd.add("dards_bn_affine_apply", y, out, res, co[0], co[1], y2, s2, h2, rows, c, y_stride, out_stride,
+            s2, h2 = self._coef[id(bnd)].scale, self._coef[id(bnd)].shift
+        self.fwd.add("dards_bn_affine_apply", y, out, res, co.scale, co.shift, y2, s2, h2, rows, c, y_stride, out_stride,
                      res_stride if res is not None else 0, y2s, 1 if relu else 0, self.dt)
         return co
 
@@ -475,8 +481,8 @@ class Plan(object):
         n_tiles = total // tile
         dg = self.new((n_tiles, c), torch.float32)
         db = self.new((n_tiles, c), torch.float32)
-        self.bwd.add("dards_bn_frozen_bwd", dout, y, mask, co[0], co[1], co[3], co[2], dx, 1 if accumulate else 0, dres,
-                     dg.data_ptr(), db.data_ptr(), n_tiles, tile, c, dout_stride, y_stride, mask_stride, dx_stride,
+        self.bwd.add("dards_bn_frozen_bwd", dout, y, mask, co.scale, co.shift, co.mean, co.rstd, dx, 1 if accumulate else 0,
+                     dres, dg.data_ptr(), db.data_ptr(), n_tiles, tile, c, dout_stride, y_stride, mask_stride, dx_stride,
                      dres_stride, relu_mode, self.dt)
         self._pending_red.append((dg, n_tiles, c, self.gptr(bn.weight)))
         self._pending_red.append((db, n_tiles, c, self.gptr(bn.bias)))
@@ -490,20 +496,12 @@ class Plan(object):
         step reads them)."""
         if not self._running:
             return
-        import numpy as np
-        dt = np.dtype([("mean", "<u8"), ("rstd", "<u8"), ("rm", "<u8"), ("rv", "<u8"), ("nbt", "<u8"), ("n_groups", "<i4"),
-                       ("rows", "<i4"), ("c", "<i4"), ("momentum", "<f4"), ("first_block", "<i4"), ("reserved", "<i4")])
-        tab = np.zeros(len(self._running), dtype=dt)
-        first = 0
-        for i, (mean, rstd, bn, rows, c) in enumerate(self._running):
-            nbt = bn.num_batches_tracked.data_ptr() if bn.num_batches_tracked is not None else 0
-            mom = BN_MOMENTUM if bn.momentum is None else bn.momentum
-            tab[i] = (mean.data_ptr(), rstd.data_ptr(), bn.running_mean.data_ptr(), bn.running_var.data_ptr(), nbt, self.G,
-                      rows, c, mom, first, 0)
-            first += (c + 63) // 64
-        t = torch.from_numpy(tab.view(np.uint8).copy()).to(self.device)
+        descs = [(mean.data_ptr(), rstd.data_ptr(), bn.running_mean.data_ptr(), bn.running_var.data_ptr(),
+                  bn.num_batches_tracked.data_ptr() if bn.num_batches_tracked is not None else None, self.G, rows, c,
+                  BN_MOMENTUM if bn.momentum is None else bn.momentum) for mean, rstd, bn, rows, c in self._running]
+        t, total = _lib.desc_table(_lib.RunningDesc, descs, self.device)
         self.bufs.append(t)
-        self.fwd.add("dards_bn_running_update_batched", t.data_ptr(), len(self._running), first, BN_EPS)
+        self.fwd.add("dards_bn_running_update_batched", t.data_ptr(), len(descs), total, BN_EPS)
         self._running = []
 
     def _flush_unpack(self):
@@ -511,17 +509,10 @@ class Plan(object):
         (Cout, Cin, K) gradient slots, in one launch."""
         if not self._pending_unpack:
             return
-        import numpy as np
-        dt = np.dtype([("dw_t", "<u8"), ("dw", "<u8"), ("c_out", "<i4"), ("c_in", "<i4"), ("ktaps", "<i4"),
-                       ("first_block", "<i4")])
-        tab = np.zeros(len(self._pending_unpack), dtype=dt)
-        first = 0
-        for i, (c, dst) in enumerate(self._pending_unpack):
-            tab[i] = (c.dwt.data_ptr(), dst, c.cout, c.cin, c.k, first)
-            first += ((c.cout + 31) // 32) * ((c.cin + 31) // 32)
-        t = torch.from_numpy(tab.view(np.uint8).copy()).to(self.device)
+        descs = [(c.dwt.data_ptr(), dst, c.cout, c.cin, c.k) for c, dst in self._pending_unpack]
+        t, total = _lib.desc_table(_lib.UnpackDesc, descs, self.device)
         self.bufs.append(t)
-        self.bwd.add("dards_unpack_wgrad_batched", t.data_ptr(), len(self._pending_unpack), first)
+        self.bwd.add("dards_unpack_wgrad_batched", t.data_ptr(), len(descs), total)
         self._pending_unpack = []
 
     def _flush_reductions(self):
@@ -530,17 +521,10 @@ class Plan(object):
         self._flush_unpack()
         if not self._pending_red:
             return
-        import numpy as np
-        dt = np.dtype([("part", "<u8"), ("out", "<u8"), ("rows", "<i4"), ("c", "<i4"), ("accumulate", "<i4"),
-                       ("first_block", "<i4")])
-        tab = np.zeros(len(self._pending_red), dtype=dt)
-        first = 0
-        for i, (part, rows, c, dst) in enumerate(self._pending_red):
-            tab[i] = (part.data_ptr(), dst, rows, c, 0, first)
-            first += (c + 63) // 64
-        t = torch.from_numpy(tab.view(np.uint8).copy()).to(self.device)
+        descs = [(part.data_ptr(), dst, rows, c, 0) for part, rows, c, dst in self._pending_red]
+        t, total = _lib.desc_table(_lib.ReduceDesc, descs, self.device)
         self.bufs.append(t)
-        self.bwd.add("dards_reduce_rows_batched", t.data_ptr(), len(self._pending_red), first)
+        self.bwd.add("dards_reduce_rows_batched", t.data_ptr(), len(descs), total)
         self._pending_red = []
 
     def gbn_bwd(self, bn, st, dout, dout_stride, x, x_stride, dx, dx_stride, rows, c, relu_mode, mask=None,
@@ -564,10 +548,11 @@ class Plan(object):
         c0 = conv.out_channels
         if conv.in_channels != 1 or conv.kernel_size[0] != 7 or conv.stride[0] != 2 or conv.padding[0] != 3:
             raise NotImplementedError("stem must be Conv1d(1, C0, 7, stride 2, padding 3)")
-        if self.bn == "frozen":
+        if self.bn != "train":  # frozen and eval plans: the running statistics' affine map, every breath on its own
             co = self._coef[id(bn)]
-            self.fwd.add("dards_stem_eval_fwd", self.x_buf.data_ptr(), conv.weight.data_ptr(), co[0], co[1], out, self.N,
-                         c0, out_stride, pool, self.dt)
+            self.eval_reads.add(id(conv.weight))
+            self.fwd.add("dards_stem_eval_fwd", self.x_buf.data_ptr(), conv.weight.data_ptr(), co.scale, co.shift, out,
+                         self.N, c0, out_stride, pool, self.dt)
             return co
         mean, rstd = self.stats(c0)
         # a BatchNorm group that does not fit the fused stem's shared memory (a flat batch of more than 226 breaths is ONE
@@ -593,8 +578,9 @@ class Plan(object):
             dwp = self.new((nc, c0 * 7), torch.float32)
             dgp = self.new((nc, c0), torch.float32)
             dbp = self.new((nc, c0), torch.float32)
-            self.bwd.add("dards_stem_frozen_bwd", dout, self.x_buf.data_ptr(), conv.weight.data_ptr(), st[0], st[1], st[3],
-                         st[2], dwp.data_ptr(), dgp.data_ptr(), dbp.data_ptr(), self.N, c0, dout_stride, pool, self.dt)
+            self.bwd.add("dards_stem_frozen_bwd", dout, self.x_buf.data_ptr(), conv.weight.data_ptr(), st.scale, st.shift,
+                         st.mean, st.rstd, dwp.data_ptr(), dgp.data_ptr(), dbp.data_ptr(), self.N, c0, dout_stride, pool,
+                         self.dt)
             self._pending_red.append((dwp, nc, c0 * 7, self.gptr(conv.weight)))
             self._pending_red.append((dgp, nc, c0, self.gptr(bn.weight)))
             self._pending_red.append((dbp, nc, c0, self.gptr(bn.bias)))
@@ -646,85 +632,90 @@ class Plan(object):
     # ------------------------------------------------------------------------------------------------------
     # ResNet (BasicBlock)
     # ------------------------------------------------------------------------------------------------------
-    def _build_resnet(self):
+    def _resnet_blocks(self):
+        """The checks every ResNet plan shares, run before anything is recorded (the stem's shape is checked by _stem).
+        Returns (stem pool type, c0, [(block, site prefix 'layer{li}.{bi}', l_in, l_out, cin, cout)])."""
         m = self.backbone
         if m.double_conv_first:
             raise NotImplementedError("resnet double_conv_first=True is not implemented on the B200 backend")
         if self.mode == "features":
             raise NotImplementedError("'features' mode exists for DenseNet only (gradcam.py:45 needs .features)")
-        N = self.N
-        pool = 0 if m.first_pool_type == "max" else 1
-        c0 = m.conv1.out_channels
-        if self.bn == "frozen":
-            # scale / shift / rstd of every layer from the running buffers, computed at the start of every forward
-            self._coef = self._eval_coeffs([bn for _, bn in resnet_bn_layers(m)], with_rstd=True)
-        a = self.new((N, 56, c0))
-        stem_st = self._stem(m.conv1, m.bn1, pool, a.data_ptr(), c0)
-        L = 56
-        recs = []
+        blocks, L = [], 56
         for li, layer in enumerate((m.layer1, m.layer2, m.layer3, m.layer4), 1):
             for bi, blk in enumerate(layer):
-                r = {"blk": blk, "a_in": a, "l_in": L}
-                c1, c2 = self.conv(blk.conv1), self.conv(blk.conv2)
-                cin, cout = c1.cin, c1.cout
-                lo = (L + 2 - 3) // c1.stride + 1
-                y1 = self.new((N, lo, cout))
-                a1 = self.new((N, lo, cout))
-                if self.cb_mode(c1, L):
-                    st1, _ = self.conv_bn_fwd(c1, blk.bn1, a.data_ptr(), cin, L, y1, a1, True)
-                else:
-                    self.conv_fwd(c1, a.data_ptr(), cin, y1.data_ptr(), cout, L)
-                    st1 = self.gbn_fwd(blk.bn1, y1.data_ptr(), cout, a1.data_ptr(), cout, self.group * lo, cout, True)
-                y2 = self.new((N, lo, cout))
-                out = self.new((N, lo, cout))
-                m2 = self.cb_mode(c2, lo, blk.downsample is not None)
-                if blk.downsample is not None:
-                    cd = self.conv(blk.downsample[0])
-                    yd = self.new((N, lo, cout))
-                    if m2 and self.cb_mode(cd, L, True) == m2:
-                        st2, std = self.conv_bn_fwd(c2, blk.bn2, a1.data_ptr(), cout, lo, y2, out, True, src_last_use=True,
-                                                    ds=(cd, blk.downsample[1], a.data_ptr(), cin, L, yd), merged_branch=True)
-                    elif self.bn == "frozen":
-                        # out = relu(bn2(y2) + bn_d(y_d)): one pass over both branches
-                        self.conv_fwd(c2, a1.data_ptr(), cout, y2.data_ptr(), cout, lo, src_last_use=True)
-                        self.conv_fwd(cd, a.data_ptr(), cin, yd.data_ptr(), cout, L)
-                        st2 = self.bn_affine_apply(blk.bn2, y2.data_ptr(), cout, out.data_ptr(), cout, N * lo, cout, True,
-                                                   second=(blk.downsample[1], yd.data_ptr(), cout))
-                        std = self._coef[id(blk.downsample[1])]
-                    else:
-                        self.conv_fwd(c2, a1.data_ptr(), cout, y2.data_ptr(), cout, lo, src_last_use=True)
-                        self.conv_fwd(cd, a.data_ptr(), cin, yd.data_ptr(), cout, L)
-                        res = self.scratch("ds_res", (N, lo, cout))
-                        std = self.gbn_fwd(blk.downsample[1], yd.data_ptr(), cout, res.data_ptr(), cout, self.group * lo,
-                                           cout, False)
-                        st2 = self.gbn_fwd(blk.bn2, y2.data_ptr(), cout, out.data_ptr(), cout, self.group * lo, cout, True,
-                                           res=res.data_ptr(), res_stride=cout)
-                    r.update(cd=cd, yd=yd, std=std)
-                else:
-                    if cin != cout or c1.stride != 1:
-                        raise RuntimeError("BasicBlock without downsample must keep the shape")
-                    if m2:
-                        st2, _ = self.conv_bn_fwd(c2, blk.bn2, a1.data_ptr(), cout, lo, y2, out, True, res=a,
-                                                  src_last_use=True)
-                    else:
-                        self.conv_fwd(c2, a1.data_ptr(), cout, y2.data_ptr(), cout, lo, src_last_use=True)
-                        st2 = self.gbn_fwd(blk.bn2, y2.data_ptr(), cout, out.data_ptr(), cout, self.group * lo, cout, True,
-                                           res=a.data_ptr(), res_stride=cout)
-                r.update(c1=c1, c2=c2, y1=y1, a1=a1, st1=st1, y2=y2, st2=st2, out=out, lo=lo, cin=cin, cout=cout)
-                self.sites["layer%d.%d.relu1" % (li, bi)] = a1
-                self.sites["layer%d.%d.relu2" % (li, bi)] = out
-                recs.append(r)
-                a, L = out, lo
-        f = recs[-1]["cout"]
+                cin, cout, stride = blk.conv1.in_channels, blk.conv1.out_channels, blk.conv1.stride[0]
+                if blk.downsample is None and (cin != cout or stride != 1):
+                    raise RuntimeError("BasicBlock without downsample must keep the shape")
+                lo = (L + 2 - 3) // stride + 1
+                blocks.append((blk, "layer%d.%d" % (li, bi), L, lo, cin, cout))
+                L = lo
         if L != 7:
             raise RuntimeError("unexpected final length %d" % L)
+        return (0 if m.first_pool_type == "max" else 1), m.conv1.out_channels, blocks
+
+    def _build_resnet(self):
+        m = self.backbone
+        pool, c0, blocks = self._resnet_blocks()
+        N = self.N
+        if self.bn == "frozen":
+            # scale / shift / rstd of every layer from the running buffers, computed at the start of every forward
+            self._coef = self._eval_coeffs(with_rstd=True)
+        a = self.new((N, 56, c0))
+        stem_st = self._stem(m.conv1, m.bn1, pool, a.data_ptr(), c0)
+        recs = []
+        for blk, site, L, lo, cin, cout in blocks:
+            r = {"a_in": a}
+            c1, c2 = self.conv(blk.conv1), self.conv(blk.conv2)
+            y1 = self.new((N, lo, cout))
+            a1 = self.new((N, lo, cout))
+            if self.cb_mode(c1, L):
+                st1, _ = self.conv_bn_fwd(c1, blk.bn1, a.data_ptr(), cin, L, y1, a1, True)
+            else:
+                self.conv_fwd(c1, a.data_ptr(), cin, y1.data_ptr(), cout, L)
+                st1 = self.gbn_fwd(blk.bn1, y1.data_ptr(), cout, a1.data_ptr(), cout, self.group * lo, cout, True)
+            y2 = self.new((N, lo, cout))
+            out = self.new((N, lo, cout))
+            m2 = self.cb_mode(c2, lo, blk.downsample is not None)
+            if blk.downsample is not None:
+                cd = self.conv(blk.downsample[0])
+                yd = self.new((N, lo, cout))
+                if m2 and self.cb_mode(cd, L, True) == m2:
+                    st2, std = self.conv_bn_fwd(c2, blk.bn2, a1.data_ptr(), cout, lo, y2, out, True, src_last_use=True,
+                                                ds=(cd, blk.downsample[1], a.data_ptr(), cin, L, yd), merged_branch=True)
+                elif self.bn == "frozen":
+                    # out = relu(bn2(y2) + bn_d(y_d)): one pass over both branches
+                    self.conv_fwd(c2, a1.data_ptr(), cout, y2.data_ptr(), cout, lo, src_last_use=True)
+                    self.conv_fwd(cd, a.data_ptr(), cin, yd.data_ptr(), cout, L)
+                    st2 = self.bn_affine_apply(blk.bn2, y2.data_ptr(), cout, out.data_ptr(), cout, N * lo, cout, True,
+                                               second=(blk.downsample[1], yd.data_ptr(), cout))
+                    std = self._coef[id(blk.downsample[1])]
+                else:
+                    self.conv_fwd(c2, a1.data_ptr(), cout, y2.data_ptr(), cout, lo, src_last_use=True)
+                    self.conv_fwd(cd, a.data_ptr(), cin, yd.data_ptr(), cout, L)
+                    res = self.scratch("ds_res", (N, lo, cout))
+                    std = self.gbn_fwd(blk.downsample[1], yd.data_ptr(), cout, res.data_ptr(), cout, self.group * lo,
+                                       cout, False)
+                    st2 = self.gbn_fwd(blk.bn2, y2.data_ptr(), cout, out.data_ptr(), cout, self.group * lo, cout, True,
+                                       res=res.data_ptr(), res_stride=cout)
+                r.update(cd=cd, yd=yd, std=std)
+            elif m2:
+                st2, _ = self.conv_bn_fwd(c2, blk.bn2, a1.data_ptr(), cout, lo, y2, out, True, res=a, src_last_use=True)
+            else:
+                self.conv_fwd(c2, a1.data_ptr(), cout, y2.data_ptr(), cout, lo, src_last_use=True)
+                st2 = self.gbn_fwd(blk.bn2, y2.data_ptr(), cout, out.data_ptr(), cout, self.group * lo, cout, True,
+                                   res=a.data_ptr(), res_stride=cout)
+            r.update(c1=c1, c2=c2, y1=y1, a1=a1, st1=st1, y2=y2, st2=st2, out=out)
+            self.sites[site + ".relu1"] = a1
+            self.sites[site + ".relu2"] = out
+            recs.append(r)
+            a = out
+        L, f = blocks[-1][3], blocks[-1][5]
         self._head_fwd(a.data_ptr(), f, L, f)
 
         # ---------------- backward ----------------
         d_out = self.scratch("gA", (N, L, f))
         self._head_bwd(d_out.data_ptr(), f, L, f)
-        for r in reversed(recs):
-            blk, lo, cin, cout, l_in = r["blk"], r["lo"], r["cin"], r["cout"], r["l_in"]
+        for (blk, _, l_in, lo, cin, cout), r in zip(reversed(blocks), reversed(recs)):
             rows = self.group * lo
             # out = relu(bn2(y2) + res):  g = d_out * (out > 0) written over d_out; dy2 = BN2 backward
             dy2 = self.scratch("gB", (N, lo, cout))
@@ -760,13 +751,13 @@ class Plan(object):
     # ------------------------------------------------------------------------------------------------------
     # ResNet in eval(): BatchNorm with the running statistics, a fixed per-channel affine map per layer
     # ------------------------------------------------------------------------------------------------------
-    def _eval_coeffs(self, bns, with_rstd=False):
-        """scale / shift (fp32, 16-byte aligned slots) of every BatchNorm layer, computed by ONE launch at the start of every
-        forward: load_state_dict() and `.data` edits change the running buffers in place, so values taken when the plan is
-        built would go stale.  Returns {id(bn): (scale pointer, shift pointer)}.
+    def _eval_coeffs(self, with_rstd=False):
+        """Coef of every BatchNorm layer of the ResNet's forward (resnet_bn_layers): scale / shift in fp32, 16-byte aligned
+        slots, computed by ONE launch at the start of every forward: load_state_dict() and `.data` edits change the running
+        buffers in place, so values taken when the plan is built would go stale.  Returns {id(bn): Coef}.
         with_rstd (frozen plans, whose backward needs the normalised input): the same launch also evaluates every layer with
-        gamma = 1, beta = 0, i.e. rstd = 1/sqrt(running_var + eps); returns {id(bn): (scale, shift, rstd, running_mean)}."""
-        import numpy as np
+        gamma = 1, beta = 0, i.e. rstd = 1/sqrt(running_var + eps), in descriptors after the scale / shift ones."""
+        bns = [bn for _, bn in resnet_bn_layers(self.backbone)]
         for bn in bns:
             if getattr(bn, "running_mean", None) is None or getattr(bn, "running_var", None) is None:
                 raise NotImplementedError("eval() with a BatchNorm layer that keeps no running statistics "
@@ -777,42 +768,34 @@ class Plan(object):
             unit = self.new((2, max(bn.num_features for bn in bns)), torch.float32)
             unit[0].fill_(1.0)
             unit[1].zero_()
-        dt = np.dtype([("gamma", "<u8"), ("beta", "<u8"), ("rm", "<u8"), ("rv", "<u8"), ("scale", "<u8"), ("shift", "<u8"),
-                       ("c", "<i4"), ("first_block", "<i4")])
-        tab = np.zeros(len(bns) * (2 if with_rstd else 1), dtype=dt)
-        out, off, first = {}, 0, 0
-        for i, bn in enumerate(bns):
+        descs, rstd_descs, out, off = [], [], {}, 0
+        for bn, slot in zip(bns, slots):
+            rm, rv, c = bn.running_mean.data_ptr(), bn.running_var.data_ptr(), bn.num_features
             sc, sh = coef[0].data_ptr() + 4 * off, coef[1].data_ptr() + 4 * off
-            tab[i] = (bn.weight.data_ptr(), bn.bias.data_ptr(), bn.running_mean.data_ptr(), bn.running_var.data_ptr(), sc, sh,
-                      bn.num_features, first)
-            out[id(bn)] = (sc, sh)
+            descs.append((bn.weight.data_ptr(), bn.bias.data_ptr(), rm, rv, sc, sh, c))
+            out[id(bn)] = Coef(sc, sh, None, None)
             if with_rstd:
-                rs, nsh = coef[2].data_ptr() + 4 * off, coef[3].data_ptr() + 4 * off
-                tab[len(bns) + i] = (unit[0].data_ptr(), unit[1].data_ptr(), bn.running_mean.data_ptr(),
-                                     bn.running_var.data_ptr(), rs, nsh, bn.num_features, 0)
-                out[id(bn)] = (sc, sh, rs, bn.running_mean.data_ptr())
+                rs = coef[2].data_ptr() + 4 * off
+                rstd_descs.append((unit[0].data_ptr(), unit[1].data_ptr(), rm, rv, rs, coef[3].data_ptr() + 4 * off, c))
+                out[id(bn)] = Coef(sc, sh, rs, rm)
             self.eval_reads.update((id(bn.weight), id(bn.bias)))
-            off += slots[i]
-            first += (bn.num_features + 63) // 64
-        for i in range(len(bns), len(tab)):  # the rstd descriptors follow the scale / shift ones
-            tab[i]["first_block"] = first
-            first += (int(tab[i]["c"]) + 63) // 64
-        t = torch.from_numpy(tab.view(np.uint8).copy()).to(self.device)
+            off += slot
+        t, total = _lib.desc_table(_lib.EvalCoeffDesc, descs + rstd_descs, self.device)
         self.bufs.append(t)
-        self.fwd.add("dards_bn_eval_coeffs_batched", t.data_ptr(), len(tab), first, BN_EPS)
+        self.fwd.add("dards_bn_eval_coeffs_batched", t.data_ptr(), len(descs) + len(rstd_descs), total, BN_EPS)
         return out
 
-    def conv_affine_fwd(self, c, coef, src, src_stride, l_in, dst, relu, res=None, src_last_use=False):
+    def conv_affine_fwd(self, c, bn, src, src_stride, l_in, dst, relu, res=None, src_last_use=False):
         """dst = [relu](bn_eval(conv(src)) [+ res]): one launch, BatchNorm / residual / ReLU in the convolution epilogue.
         `dst` and `res` are (N, l_out, cout) pointers."""
         l_out = (l_in + 2 * c.pad - c.k) // c.stride + 1
         tc = self._tc_ok(c, "fwd")
         w = c.koi if tc else c.kio
+        co = self._coef[id(bn)]
         self.eval_reads.add(id(c.mod.weight))
-        self.fwd.add("dards_conv1d_affine_fwd", src, w.data_ptr(), dst, res, coef[0], coef[1], self.N, l_in, l_out, c.cin,
+        self.fwd.add("dards_conv1d_affine_fwd", src, w.data_ptr(), dst, res, co.scale, co.shift, self.N, l_in, l_out, c.cin,
                      c.cout, src_stride, c.cout, c.cout if res is not None else 0, c.k, c.stride, c.pad,
                      (1 if relu else 0) | (_lib.HINT_LAST_USE if src_last_use else 0), self.dt, 1 if tc else 0)
-        return l_out
 
     def _build_resnet_eval(self):
         """Forward only: pack, coefficients, eval stem, then per block conv1 -> affine + ReLU and conv2 -> affine + residual +
@@ -820,23 +803,10 @@ class Plan(object):
         update, no gradient buffers.  Activations rotate through four buffers, each the size of the largest (N, L, C)
         activation: block input (= identity residual), conv1 output, downsample output, block output."""
         m = self.backbone
-        if m.double_conv_first:
-            raise NotImplementedError("resnet double_conv_first=True is not implemented on the B200 backend")
-        if self.mode == "features":
-            raise NotImplementedError("'features' mode exists for DenseNet only (gradcam.py:45 needs .features)")
+        pool, c0, blocks = self._resnet_blocks()
         N = self.N
-        pool = 0 if m.first_pool_type == "max" else 1
-        c0 = m.conv1.out_channels
-        if m.conv1.in_channels != 1 or m.conv1.kernel_size[0] != 7 or m.conv1.stride[0] != 2 or m.conv1.padding[0] != 3:
-            raise NotImplementedError("stem must be Conv1d(1, C0, 7, stride 2, padding 3)")
-        blocks = [blk for layer in (m.layer1, m.layer2, m.layer3, m.layer4) for blk in layer]
-        bns = [m.bn1]
-        largest, L = 56 * c0, 56
-        for blk in blocks:
-            bns += [blk.bn1, blk.bn2] + ([blk.downsample[1]] if blk.downsample is not None else [])
-            L = (L + 2 - 3) // blk.conv1.stride[0] + 1
-            largest = max(largest, L * blk.conv1.out_channels)
-        coef = self._eval_coeffs(bns)
+        self._coef = self._eval_coeffs()
+        largest = max([56 * c0] + [lo * cout for _, _, _, lo, _, cout in blocks])
         pool_bufs = [self.new((N * largest,)) for _ in range(4)]
         self.act_bytes = sum(t.numel() * t.element_size() for t in pool_bufs)
 
@@ -844,31 +814,23 @@ class Plan(object):
             return next(t for t in pool_bufs if all(t is not b for b in busy))
 
         a = pool_bufs[0]
-        self.eval_reads.add(id(m.conv1.weight))
-        self.fwd.add("dards_stem_eval_fwd", self.x_buf.data_ptr(), m.conv1.weight.data_ptr(), coef[id(m.bn1)][0],
-                     coef[id(m.bn1)][1], a.data_ptr(), N, c0, c0, pool, self.dt)
-        L, cin = 56, c0
-        for blk in blocks:
+        self._stem(m.conv1, m.bn1, pool, a.data_ptr(), c0)
+        for blk, _, L, lo, cin, cout in blocks:
             c1, c2 = self.conv(blk.conv1), self.conv(blk.conv2)
-            cout = c1.cout
             a1 = free(a)
-            lo = self.conv_affine_fwd(c1, coef[id(blk.bn1)], a.data_ptr(), cin, L, a1.data_ptr(), True)
+            self.conv_affine_fwd(c1, blk.bn1, a.data_ptr(), cin, L, a1.data_ptr(), True)
             if blk.downsample is not None:
                 cd = self.conv(blk.downsample[0])
                 res = free(a, a1)
-                self.conv_affine_fwd(cd, coef[id(blk.downsample[1])], a.data_ptr(), cin, L, res.data_ptr(), False,
-                                     src_last_use=True)
+                self.conv_affine_fwd(cd, blk.downsample[1], a.data_ptr(), cin, L, res.data_ptr(), False, src_last_use=True)
             else:
-                if cin != cout or c1.stride != 1:
-                    raise RuntimeError("BasicBlock without downsample must keep the shape")
                 res = a
             out = free(a, a1, res)
-            self.conv_affine_fwd(c2, coef[id(blk.bn2)], a1.data_ptr(), cout, lo, out.data_ptr(), True, res=res.data_ptr(),
+            self.conv_affine_fwd(c2, blk.bn2, a1.data_ptr(), cout, lo, out.data_ptr(), True, res=res.data_ptr(),
                                  src_last_use=True)
-            a, L, cin = out, lo, cout
-        if L != 7:
-            raise RuntimeError("unexpected final length %d" % L)
-        self._head_fwd(a.data_ptr(), cin, L, cin)
+            a = out
+        L, f = blocks[-1][3], blocks[-1][5]
+        self._head_fwd(a.data_ptr(), f, L, f)
         if self.linear is not None and self.mode in ("cnn_linear", "per_breath"):
             self.eval_reads.update((id(self.linear.weight), id(self.linear.bias)))
 
@@ -1015,17 +977,10 @@ class Plan(object):
     def _build_pack_table(self):
         """One `dards_pack_desc` per convolution, uploaded once: the whole network's weights are re-packed by a
         single launch whenever they change."""
-        import numpy as np
-        dt = np.dtype([("w", "<u8"), ("kio", "<u8"), ("koi", "<u8"), ("c_out", "<i4"), ("c_in", "<i4"), ("ktaps", "<i4"),
-                       ("first_block", "<i4")])
-        tab = np.zeros(len(self.convs), dtype=dt)
-        first = 0
-        for i, c in enumerate(self.convs):
-            tab[i] = (c.mod.weight.data_ptr(), c.kio.data_ptr(), c.koi.data_ptr(), c.cout, c.cin, c.k, first)
-            first += ((c.cout + 31) // 32) * ((c.cin + 31) // 32)
-        self.pack_table = torch.from_numpy(tab.view(np.uint8).copy()).to(self.device)
+        descs = [(c.mod.weight.data_ptr(), c.kio.data_ptr(), c.koi.data_ptr(), c.cout, c.cin, c.k) for c in self.convs]
+        self.pack_table, total = _lib.desc_table(_lib.PackDesc, descs, self.device)
         self.bufs.append(self.pack_table)
-        self.pack.add("dards_pack_conv_weights_batched", self.pack_table.data_ptr(), len(self.convs), first, self.dt)
+        self.pack.add("dards_pack_conv_weights_batched", self.pack_table.data_ptr(), len(descs), total, self.dt)
 
     def _pack_if_needed(self, st):
         ver = 0

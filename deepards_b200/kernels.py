@@ -63,18 +63,11 @@ def conv1d_affine_fwd(x, w, scale, shift, stride, pad, impl=0, res=None, relu=Tr
 
 def bn_eval_coeffs(layers, eps=1e-5):
     """layers: [(gamma, beta, running_mean, running_var)] fp32 -> [(scale, shift)], one batched launch."""
-    import numpy as np
-    dt = np.dtype([("gamma", "<u8"), ("beta", "<u8"), ("rm", "<u8"), ("rv", "<u8"), ("scale", "<u8"), ("shift", "<u8"),
-                   ("c", "<i4"), ("first_block", "<i4")])
-    tab = np.zeros(len(layers), dtype=dt)
-    outs, first = [], 0
-    for i, (g, b, rm, rv) in enumerate(layers):
-        sc, sh = torch.empty_like(g), torch.empty_like(g)
-        outs.append((sc, sh))
-        tab[i] = (g.data_ptr(), b.data_ptr(), rm.data_ptr(), rv.data_ptr(), sc.data_ptr(), sh.data_ptr(), g.numel(), first)
-        first += (g.numel() + 63) // 64
-    t = torch.from_numpy(tab.view(np.uint8).copy()).to(layers[0][0].device)
-    _lib.call("dards_bn_eval_coeffs_batched", t.data_ptr(), len(layers), first, eps, _st(t))
+    outs = [(torch.empty_like(g), torch.empty_like(g)) for g, _, _, _ in layers]
+    descs = [(g.data_ptr(), b.data_ptr(), rm.data_ptr(), rv.data_ptr(), sc.data_ptr(), sh.data_ptr(), g.numel())
+             for (g, b, rm, rv), (sc, sh) in zip(layers, outs)]
+    t, total = _lib.desc_table(_lib.EvalCoeffDesc, descs, layers[0][0].device)
+    _lib.call("dards_bn_eval_coeffs_batched", t.data_ptr(), len(layers), total, eps, _st(t))
     torch.cuda.current_stream(t.device).synchronize()  # the table is freed on return
     return outs
 
@@ -176,7 +169,6 @@ def conv1d_wgrad(x, dout, k, stride, pad, impl=0):
 
 def conv1d_wgrad_accum(x, dout, k, stride, pad):
     """tcgen05 weight gradient through the accumulate path: zeroed tap-major buffer, L2 reduce-adds, one unpack launch."""
-    import numpy as np
     n, l, cin = x.shape
     _, lo, cout = dout.shape
     dwt = torch.zeros((k, cout, cin), dtype=torch.float32, device=x.device)
@@ -184,11 +176,8 @@ def conv1d_wgrad_accum(x, dout, k, stride, pad):
     _lib.call("dards_memset_zero", dwt.data_ptr(), dwt.numel() * 4, _st(x))
     _lib.call("dards_conv1d_wgrad_accum", x.data_ptr(), dout.data_ptr(), dwt.data_ptr(), n, l, lo, cin, cout, _rowstride(x),
               _rowstride(dout), k, stride, pad, _dt(x), _st(x))
-    dt = np.dtype([("dw_t", "<u8"), ("dw", "<u8"), ("c_out", "<i4"), ("c_in", "<i4"), ("ktaps", "<i4"), ("first_block", "<i4")])
-    tab = np.zeros(1, dtype=dt)
-    tab[0] = (dwt.data_ptr(), dw.data_ptr(), cout, cin, k, 0)
-    t = torch.from_numpy(tab.view(np.uint8).copy()).to(x.device)
-    _lib.call("dards_unpack_wgrad_batched", t.data_ptr(), 1, ((cout + 31) // 32) * ((cin + 31) // 32), _st(x))
+    t, total = _lib.desc_table(_lib.UnpackDesc, [(dwt.data_ptr(), dw.data_ptr(), cout, cin, k)], x.device)
+    _lib.call("dards_unpack_wgrad_batched", t.data_ptr(), 1, total, _st(x))
     torch.cuda.synchronize()
     return dw
 

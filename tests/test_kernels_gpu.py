@@ -385,21 +385,6 @@ def test_bn_running_update_matches_sequential_torch():
     assert int(nbt) == 3
 
 
-def _desc_table(dt_fields, rows):
-    import numpy as np
-    tab = np.zeros(len(rows), dtype=np.dtype(dt_fields))
-    for i, r in enumerate(rows):
-        tab[i] = r
-    return torch.from_numpy(tab.view(np.uint8).copy()).to(DEV)
-
-
-RUNNING_DESC = [("mean", "<u8"), ("rstd", "<u8"), ("rm", "<u8"), ("rv", "<u8"), ("nbt", "<u8"), ("n_groups", "<i4"),
-                ("rows", "<i4"), ("c", "<i4"), ("momentum", "<f4"), ("first_block", "<i4"), ("reserved", "<i4")]
-REDUCE_DESC = [("part", "<u8"), ("out", "<u8"), ("rows", "<i4"), ("c", "<i4"), ("accumulate", "<i4"), ("first_block", "<i4")]
-PACK_DESC = [("w", "<u8"), ("kio", "<u8"), ("koi", "<u8"), ("c_out", "<i4"), ("c_in", "<i4"), ("ktaps", "<i4"),
-             ("first_block", "<i4")]
-
-
 @pytest.mark.parametrize("n,c,l,group,dtype", [(120, 64, 14, 20, torch.float32), (5120, 512, 7, 20, torch.bfloat16),
                                                (5120, 64, 56, 20, torch.bfloat16), (60, 96, 28, 20, torch.bfloat16),
                                                (40, 128, 28, 20, torch.bfloat16), (30, 64, 56, 30, torch.bfloat16)])
@@ -436,7 +421,7 @@ def test_batched_running_update_reduce_rows_and_pack():
     st = torch.cuda.current_stream().cuda_stream
     g = torch.Generator().manual_seed(22)
     # ---- running statistics of several BatchNorm layers in one launch == torch's sequential update ----
-    layers, rows_tab, first = [], [], 0
+    layers, rows_tab = [], []
     for (n, c, l, group) in [(100, 64, 14, 20), (100, 96, 7, 20), (60, 512, 7, 20)]:
         x = torch.randn(n, c, l, generator=g).to(DEV)
         bn = torch.nn.BatchNorm1d(c).to(DEV).train()
@@ -447,36 +432,32 @@ def test_batched_running_update_reduce_rows_and_pack():
         nbt = torch.zeros((), dtype=torch.long, device=DEV)
         layers.append((bn, rm, rv, nbt, n // group, mean, rstd))
         rows_tab.append((mean.data_ptr(), rstd.data_ptr(), rm.data_ptr(), rv.data_ptr(), nbt.data_ptr(), n // group,
-                         group * l, c, 0.1, first, 0))
-        first += (c + 63) // 64
-    tab = _desc_table(RUNNING_DESC, rows_tab)
-    _lib.call("dards_bn_running_update_batched", tab.data_ptr(), len(rows_tab), first, 1e-5, st)
+                         group * l, c, 0.1))
+    tab, total = _lib.desc_table(_lib.RunningDesc, rows_tab, DEV)
+    _lib.call("dards_bn_running_update_batched", tab.data_ptr(), len(rows_tab), total, 1e-5, st)
     for bn, rm, rv, nbt, ng, _, _ in layers:
         assert rel_err(rm, bn.running_mean) < 2e-5 and rel_err(rv, bn.running_var) < 2e-5 and int(nbt) == ng
     # ---- batched row reduction ----
     parts = [torch.randn(r, c, generator=g).to(DEV) for r, c in [(256, 64), (256, 448), (7, 12), (300, 512)]]
     outs = [torch.full((p.shape[1],), 3.0, device=DEV) for p in parts]
-    rows_tab, first = [], 0
-    for i, (p, o) in enumerate(zip(parts, outs)):
-        rows_tab.append((p.data_ptr(), o.data_ptr(), p.shape[0], p.shape[1], 1 if i == 2 else 0, first))
-        first += (p.shape[1] + 63) // 64
-    tab = _desc_table(REDUCE_DESC, rows_tab)
-    _lib.call("dards_reduce_rows_batched", tab.data_ptr(), len(parts), first, st)
+    rows_tab = [(p.data_ptr(), o.data_ptr(), p.shape[0], p.shape[1], 1 if i == 2 else 0)
+                for i, (p, o) in enumerate(zip(parts, outs))]
+    tab, total = _lib.desc_table(_lib.ReduceDesc, rows_tab, DEV)
+    _lib.call("dards_reduce_rows_batched", tab.data_ptr(), len(parts), total, st)
     for i, (p, o) in enumerate(zip(parts, outs)):
         assert rel_err(o, p.sum(0) + (3.0 if i == 2 else 0.0)) < 1e-5
     # ---- batched weight packing == per-tensor packing ----
     shapes = [(64, 64, 3), (128, 64, 1), (512, 256, 3), (32, 128, 3), (40, 24, 5)]
     ws = [torch.randn(s, generator=g).to(DEV) for s in shapes]
-    rows_tab, outs, first = [], [], 0
+    rows_tab, outs = [], []
     for wt in ws:
         co, ci, k = wt.shape
         kio = torch.zeros((k, ci, co), dtype=torch.bfloat16, device=DEV)
         koi = torch.zeros((k, co, ci), dtype=torch.bfloat16, device=DEV)
         outs.append((kio, koi))
-        rows_tab.append((wt.data_ptr(), kio.data_ptr(), koi.data_ptr(), co, ci, k, first))
-        first += ((co + 31) // 32) * ((ci + 31) // 32)
-    tab = _desc_table(PACK_DESC, rows_tab)
-    _lib.call("dards_pack_conv_weights_batched", tab.data_ptr(), len(ws), first, _lib.BF16, st)
+        rows_tab.append((wt.data_ptr(), kio.data_ptr(), koi.data_ptr(), co, ci, k))
+    tab, total = _lib.desc_table(_lib.PackDesc, rows_tab, DEV)
+    _lib.call("dards_pack_conv_weights_batched", tab.data_ptr(), len(ws), total, _lib.BF16, st)
     for wt, (kio, koi) in zip(ws, outs):
         r_kio, r_koi = K().pack_conv_weight(wt, torch.bfloat16)
         assert torch.equal(kio, r_kio) and torch.equal(koi, r_koi)
