@@ -12,7 +12,8 @@
 //  * streaming (generic fallback for tiles that do not fit): re-reads the tile from L1/L2 for every sweep.
 //
 // Statistics: the cached kernels use ONE sweep of sums shifted by a sample of the data (the group's first row), which loses
-// no digits in E[d^2] - E[d]^2; the streaming fallback uses two sweeps (mean, then centred sum of squares).
+// no digits in E[d^2] - E[d]^2 beyond a factor 1 + (sample - mean)^2 / var; the streaming fallback uses two sweeps (mean of
+// the differences from the group's first row, then the centred sum of squares).
 // Cross-group reductions (running statistics, dgamma/dbeta) are separate BATCHED kernels: one launch handles a
 // whole table of BatchNorm layers (an in-kernel "last CTA reduces" variant was measured 12-19 us slower per launch:
 // the gpu-scope fence of every CTA invalidates L1 and waits for its stores).
@@ -385,13 +386,16 @@ __global__ void __launch_bounds__(THREADS)
           if (dgamma_part) dgamma_part[(size_t)g * c + c0 + j] = acc[V + j];
         }
       }
-      // dx = sc*(g - m1 - xhat*m2) = sc*g + kb*x + kc  (FROZEN: dx = sc*g)
+      // dx = sc*(g - m1 - xhat*m2) = sc*g + kb*x + kc  (FROZEN: dx = sc*g).  fp32 keeps x - mean apart: with the mean
+      // folded into kc, kb*x and kc cancel when |mean| >> std (~50x torch's error at |mean|/std = 1e3); a bf16 x already
+      // carries 2^-9 |x| of rounding and keeps the fold
+      constexpr bool XC = sizeof(T) == 4;
       float kb[V], kc[V];
 #pragma unroll
       for (int j = 0; j < V; ++j) {
         const float m1 = acc[j] * inv_n, m2 = acc[V + j] * inv_n;
         kb[j] = FROZEN ? 0.f : -sc[j] * m2 * rstd[j];
-        kc[j] = FROZEN ? 0.f : -sc[j] * m1 - kb[j] * mean[j];
+        kc[j] = FROZEN ? 0.f : (XC ? -sc[j] * m1 : -sc[j] * m1 - kb[j] * mean[j]);
       }
       // ---- sweep 2 (shared -> global): dx; refill the cache with the next tile ----
       T* dxp = dx + row0 * dx_stride + c0;
@@ -413,7 +417,8 @@ __global__ void __launch_bounds__(THREADS)
         Vec<T>::unpack(rg, gv);
         Vec<T>::unpack(rx, xv);
 #pragma unroll
-        for (int j = 0; j < V; ++j) o[j] = FROZEN ? sc[j] * gv[j] : fmaf(sc[j], gv[j], fmaf(kb[j], xv[j], kc[j]));
+        for (int j = 0; j < V; ++j)
+          o[j] = FROZEN ? sc[j] * gv[j] : fmaf(sc[j], gv[j], fmaf(kb[j], XC ? xv[j] - mean[j] : xv[j], kc[j]));
         if (accumulate_dx) {
           float e[V];
           Vec<T>::unpack(ro, e);
@@ -473,20 +478,24 @@ __global__ void __launch_bounds__(BN_THREADS)
   const float inv_n = 1.f / (float)rows;
   const T* xp = x + row_base * x_stride + c0;
 
-  float s[V];
+  // the mean as the group's first row plus the mean of the differences: a constant channel gets its value exactly, however
+  // 1/rows rounds (with var = 0 and rstd = 1/sqrt(eps), a mean one ulp off moves the output by ~300 ulps of x)
+  float s[V], x0[V];
 #pragma unroll
-  for (int j = 0; j < V; ++j) s[j] = 0.f;
-  if (active)
+  for (int j = 0; j < V; ++j) s[j] = x0[j] = 0.f;
+  if (active) {
+    Vec<T>::unpack(ld16(xp), x0);
     for (int r = rl; r < rows; r += BN_LANES) {
       float v[V];
       Vec<T>::unpack(ld16(xp + (size_t)r * x_stride), v);
 #pragma unroll
-      for (int j = 0; j < V; ++j) s[j] += v[j];
+      for (int j = 0; j < V; ++j) s[j] += v[j] - x0[j];
     }
+  }
   lane_reduce<V>(s, red, bcast, rl, cq);
   float mean[V];
 #pragma unroll
-  for (int j = 0; j < V; ++j) mean[j] = s[j] * inv_n;
+  for (int j = 0; j < V; ++j) mean[j] = fmaf(s[j], inv_n, x0[j]);
 
   float q[V];
 #pragma unroll
@@ -606,12 +615,13 @@ __global__ void __launch_bounds__(BN_THREADS)
       if (dgamma_part) dgamma_part[(size_t)g * c + c0 + j] = s2[j];
     }
   }
+  constexpr bool XC = sizeof(T) == 4;  // fp32: kb*(x - mean) - sc*m1, as in the cached kernel
   float kb[V], kc[V];
 #pragma unroll
   for (int j = 0; j < V; ++j) {
     const float m1 = s1[j] * inv_n, m2 = s2[j] * inv_n;
     kb[j] = FROZEN ? 0.f : -sc[j] * m2 * rstd[j];
-    kc[j] = FROZEN ? 0.f : -sc[j] * m1 - kb[j] * mean[j];
+    kc[j] = FROZEN ? 0.f : (XC ? -sc[j] * m1 : -sc[j] * m1 - kb[j] * mean[j]);
   }
   T* dxp = dx + row_base * dx_stride + c0;
   T* drp = dres ? dres + row_base * dres_stride + c0 : nullptr;
@@ -619,7 +629,8 @@ __global__ void __launch_bounds__(BN_THREADS)
     float gv[V], xv[V], o[V];
     load_row(r, gv, xv);
 #pragma unroll
-    for (int j = 0; j < V; ++j) o[j] = FROZEN ? sc[j] * gv[j] : fmaf(sc[j], gv[j], fmaf(kb[j], xv[j], kc[j]));
+    for (int j = 0; j < V; ++j)
+      o[j] = FROZEN ? sc[j] * gv[j] : fmaf(sc[j], gv[j], fmaf(kb[j], XC ? xv[j] - mean[j] : xv[j], kc[j]));
     if (drp) st16(drp + (size_t)r * dres_stride, Vec<T>::pack(gv));
     if (accumulate_dx) {
       float e[V];

@@ -385,7 +385,14 @@ __global__ void __launch_bounds__(EPI == CB_FUSED ? CB_THREADS_FUSED : CB_THREAD
         tmem_ld16(t_row + (uint32_t)(half << 4), va);
         auto chunk = [&](int ch, const uint32_t (&v)[16]) {
           const uint32_t* cr = crow + (ch << 4);
-          if (first && ch == half) shift = __uint_as_float(v[0]);  // any sample of the channel's data will do
+          if (EPI != CB_PLAIN && first && ch == half) {
+            // any sample of the channel's data will do, but only a real column is one: the chunk's first column can be a
+            // halo column (L = 16: column 16 of the second half), and a junk column may hold anything, NaN included
+            shift = 0.f;
+#pragma unroll
+            for (int j = 15; j >= 0; --j)
+              if (cr[j] != 0xFFFFFFFFu) shift = __uint_as_float(v[j]);
+          }
           if (EPI != CB_PLAIN) {
             const uint4* cr4 = reinterpret_cast<const uint4*>(cr);
 #pragma unroll

@@ -20,6 +20,8 @@
 //             Chan-merges the records of its group (fixed order) and runs sweep 2 on its chunk;
 //   backward: PARTIAL pass -- every chunk CTA writes its input moments and its per-channel S1, S2, G_t sums; a small combine
 //             kernel adds the chunks of a group in order and applies the analytic BatchNorm / weight-gradient formula.
+//             The moments and G_t are sums of x - s, with s the mean of the group's first breath when the input has a DC
+//             offset (read by every chunk CTA, so their partial sums still add): with raw sums the formula cancels digits.
 // The caller provides the workspace for the chunk records (stem_workspace_bytes).
 #include "common.cuh"
 
@@ -216,6 +218,52 @@ __device__ __forceinline__ int stem_r_index(int a, int b) {  // a <= b
   return a * STEM_K - a * (a - 1) / 2 + (b - a);
 }
 
+// s, the shift of the backward's input moments (xb: the group's first breath): that breath's mean when it exceeds the
+// breath's spread (mean^2 > var), else 0.  Below that ratio the raw sums lose less than a digit, and s = 0 leaves the
+// arithmetic exactly that of the unshifted sums (x - 0 = x, mean - 0 * sum w = mean), so centred data such as z-scored
+// flow computes what it always computed.  Every CTA that needs s (the chunk CTAs of a group and the combine kernel) runs
+// this same sequence -- seven warp sums of 32 samples, added in order, products rounded on their own -- so they agree bit
+// for bit.  All threads of the block call it; red: 16 floats of shared memory no other code touches until the next barrier.
+__device__ __forceinline__ float stem_group_shift(const float* __restrict__ xb, float* red) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int vw = warp; vw < STEM_L / 32; vw += blockDim.x >> 5) {
+    const float v = xb[vw * 32 + lane];
+    const float s1 = warp_sum(v), s2 = warp_sum(__fmul_rn(v, v));
+    if (lane == 0) {
+      red[vw] = s1;
+      red[8 + vw] = s2;
+    }
+  }
+  __syncthreads();
+  float s1 = 0.f, s2 = 0.f;
+  for (int vw = 0; vw < STEM_L / 32; ++vw) {
+    s1 += red[vw];
+    s2 += red[8 + vw];
+  }
+  const float m = __fmul_rn(s1, 1.f / (float)STEM_L);
+  const float var = __fsub_rn(__fmul_rn(s2, 1.f / (float)STEM_L), __fmul_rn(m, m));
+  return __fmul_rn(m, m) > var ? m : 0.f;
+}
+
+// H_t / rstd = sum_a w_a R'[a][t] - mean_s X'_t, with xr = X' (7) then R' (28), sums of x - s, and mean_s = mean - s sum_a w_a
+// the mean of the convolution of x - s
+__device__ __forceinline__ float stem_h_over_rstd(const float (&w)[STEM_K], const float* xr, int t, float mean_s) {
+  float wr_r = 0.f;
+#pragma unroll
+  for (int a = 0; a < STEM_K; ++a) {
+    const int lo = a < t ? a : t, hi = a < t ? t : a;
+    wr_r = fmaf(w[a], xr[STEM_K + stem_r_index(lo, hi)], wr_r);
+  }
+  return wr_r - mean_s * xr[t];
+}
+
+__device__ __forceinline__ float stem_shifted_mean(const float (&w)[STEM_K], float mean, float shift) {
+  float wsum = 0.f;
+#pragma unroll
+  for (int a = 0; a < STEM_K; ++a) wsum += w[a];
+  return fmaf(-shift, wsum, mean);
+}
+
 // STAGE: the CTA's slice of dout (group x 56 rows x 16 channels) is brought into shared memory with cp.async while the
 // input moments are computed, and sweep B reads it from there.  With the gradient loaded from global memory inside the
 // sweep the kernel spent most of its time waiting on those loads (ncu: long-scoreboard stalls 5.9 per issue, issue
@@ -256,11 +304,13 @@ __global__ void __launch_bounds__(STEM_THREADS)
       stem_cp_async16(ds + row * STEM_CS + part * EPC, src + (size_t)row * dout_stride + part * EPC);
     }
   }
+  // the shift s of the moments, from the group's first breath in global memory (red's tail is free until section B)
+  const float shift = FROZEN ? 0.f : stem_group_shift(x + (size_t)g * group_all * STEM_L, red + STEM_THREADS * 8);
   stem_load_group(x + breath0 * STEM_L, xs, group);
   __syncthreads();
   const int n_conv = group * STEM_LC;
 
-  // ---- A. channel-independent input moments: X_t = sum xin_t, R[a][b] = sum xin_a * xin_b --------------
+  // ---- A. channel-independent input moments about s: X'_t = sum (xin_t - s), R'[a][b] = sum (xin_a - s)(xin_b - s) --
   if (!FROZEN) {
     float acc[STEM_K + STEM_NR];
 #pragma unroll
@@ -269,7 +319,7 @@ __global__ void __launch_bounds__(STEM_THREADS)
       const float* xb = xs + (i / STEM_LC) * STEM_BS + STEM_PAD + 2 * (i % STEM_LC) - 3;
       float xin[STEM_K];
 #pragma unroll
-      for (int t = 0; t < STEM_K; ++t) xin[t] = xb[t];
+      for (int t = 0; t < STEM_K; ++t) xin[t] = xb[t] - shift;
       int k = STEM_K;
 #pragma unroll
       for (int a = 0; a < STEM_K; ++a) {
@@ -299,9 +349,9 @@ __global__ void __launch_bounds__(STEM_THREADS)
     __syncthreads();
   }
 
-  // ---- B. per channel: S1 = sum g, S2 = sum g*xhat, G_t = sum g * xin_t ----------------------------------
+  // ---- B. per channel: S1 = sum g, S2 = sum g*xhat, G'_t = sum g * (xin_t - s) (FROZEN: G_t = sum g * xin_t) -------
   // run = 14 pool outputs; the 11-element input window x[4lp-5 .. 4lp+5] of the three conv positions feeding
-  // pool output lp (2lp-1, 2lp, 2lp+1) stays in registers and slides by 4 per pool output.
+  // pool output lp (2lp-1, 2lp, 2lp+1) stays in registers and slides by 4 per pool output; xd is the same window less s.
   float wr[STEM_K];
 #pragma unroll
   for (int t = 0; t < STEM_K; ++t) wr[t] = w[ch * STEM_K + t];
@@ -322,9 +372,12 @@ __global__ void __launch_bounds__(STEM_THREADS)
     const float* xb = xs + b * STEM_BS + STEM_PAD + 4 * lp0 - 5;  // xw[i] = xb[i + 4j]
     const T* dp_ptr = STAGE ? ds + (b * STEM_LP + lp0) * STEM_CS + c
                             : dout + ((breath0 + b) * STEM_LP + lp0) * dout_stride + ch;
-    float xw[11];
+    float xw[11], xd[11];
 #pragma unroll
-    for (int i = 0; i < 7; ++i) xw[i] = xb[i];
+    for (int i = 0; i < 7; ++i) {
+      xw[i] = xb[i];
+      xd[i] = FROZEN ? xw[i] : xw[i] - shift;
+    }
     float yl = stem_dot7(wr, xw[0], xw[1], xw[2], xw[3], xw[4], xw[5], xw[6]);
     bool okl = lp0 != 0;  // conv position -1 does not exist
 #pragma unroll
@@ -333,6 +386,8 @@ __global__ void __launch_bounds__(STEM_THREADS)
       const float2 n0 = *reinterpret_cast<const float2*>(xb + 7 + 4 * j);
       const float2 n1 = *reinterpret_cast<const float2*>(xb + 9 + 4 * j);
       xw[7] = n0.x; xw[8] = n0.y; xw[9] = n1.x; xw[10] = n1.y;
+#pragma unroll
+      for (int i = 7; i < 11; ++i) xd[i] = FROZEN ? xw[i] : xw[i] - shift;
       const float ym = stem_dot7(wr, xw[2], xw[3], xw[4], xw[5], xw[6], xw[7], xw[8]);
       const float yr = stem_dot7(wr, xw[4], xw[5], xw[6], xw[7], xw[8], xw[9], xw[10]);
       const float zl = okl ? fmaxf(fmaf(yl, sc, sh), 0.f) : 0.f;
@@ -360,13 +415,16 @@ __global__ void __launch_bounds__(STEM_THREADS)
       s2 = fmaf(gr, (yr - mean) * rstd, s2);
 #pragma unroll
       for (int t = 0; t < STEM_K; ++t) {
-        gt[t] = fmaf(gl, xw[t], gt[t]);
-        gt[t] = fmaf(gmid, xw[t + 2], gt[t]);
-        gt[t] = fmaf(gr, xw[t + 4], gt[t]);
+        gt[t] = fmaf(gl, xd[t], gt[t]);
+        gt[t] = fmaf(gmid, xd[t + 2], gt[t]);
+        gt[t] = fmaf(gr, xd[t + 4], gt[t]);
       }
       // slide by 4 inputs = 2 conv positions
 #pragma unroll
-      for (int i = 0; i < 7; ++i) xw[i] = xw[i + 4];
+      for (int i = 0; i < 7; ++i) {
+        xw[i] = xw[i + 4];
+        xd[i] = xd[i + 4];
+      }
       yl = yr;
       okl = true;
     }
@@ -407,33 +465,32 @@ __global__ void __launch_bounds__(STEM_THREADS)
       return;
     }
     // ---- C. BN backward folded into the weight gradient ------------------------------------------------
-    // dy = gamma*rstd*(g - S1/n - xhat*S2/n);  dW_t = sum dy*xin_t
-    //    = gamma*rstd*(G_t - S1/n * X_t - S2/n * H_t),  H_t = sum xhat*xin_t = rstd*(sum_a w_a R[a][t] - mean*X_t)
+    // dy = gamma*rstd*(g - S1/n - xhat*S2/n);  dW_t = sum dy*xin_t = sum dy*(xin_t - s), because sum dy = 0
+    //    = gamma*rstd*(G'_t - S1/n * X'_t - S2/n * H_t),  H_t = sum xhat*(xin_t - s) = rstd*(sum_a w_a R'[a][t] - mean_s*X'_t)
+    // (y - mean = sum_a w_a (xin_a - s) - mean_s, mean_s = mean - s * sum_a w_a)
     const float inv_n = 1.f / (float)n_conv;
+    const float mean_s = stem_shifted_mean(wr, mean, shift);
     dbeta_part[(size_t)g * c0 + ch] = s1;
     dgamma_part[(size_t)g * c0 + ch] = s2;
 #pragma unroll
     for (int t = 0; t < STEM_K; ++t) {
-      float wr_r = 0.f;
-#pragma unroll
-      for (int a = 0; a < STEM_K; ++a) {
-        int lo = a < t ? a : t, hi = a < t ? t : a;
-        wr_r = fmaf(wr[a], xr[STEM_K + stem_r_index(lo, hi)], wr_r);
-      }
-      float h = rstd * (wr_r - mean * xr[t]);
+      const float h = rstd * stem_h_over_rstd(wr, xr, t, mean_s);
       dw_part[((size_t)g * c0 + ch) * STEM_K + t] = sc * (gt[t] - s1 * inv_n * xr[t] - s2 * inv_n * h);
     }
   }
 }
 
-// chunked backward, second pass: thread = channel of one group; adds the chunk partials in order and applies section C
+// chunked backward, second pass: thread = channel of one group; adds the chunk partials (sums about the group's shift s) in
+// order and applies section C
 __global__ void __launch_bounds__(128)
-    stem_bwd_combine_kernel(const float* __restrict__ w, const float* __restrict__ gamma, const float* __restrict__ save_mean,
-                            const float* __restrict__ save_rstd, const float* __restrict__ mom_part,
-                            const float* __restrict__ ch_part, float* __restrict__ dw_part, float* __restrict__ dgamma_part,
-                            float* __restrict__ dbeta_part, int group, int n_chunks, int c0) {
+    stem_bwd_combine_kernel(const float* __restrict__ x, const float* __restrict__ w, const float* __restrict__ gamma,
+                            const float* __restrict__ save_mean, const float* __restrict__ save_rstd,
+                            const float* __restrict__ mom_part, const float* __restrict__ ch_part, float* __restrict__ dw_part,
+                            float* __restrict__ dgamma_part, float* __restrict__ dbeta_part, int group, int n_chunks, int c0) {
   __shared__ float xr[STEM_K + STEM_NR];
+  __shared__ float shift_red[16];
   const int g = blockIdx.x;
+  const float shift = stem_group_shift(x + (size_t)g * group * STEM_L, shift_red);  // the partial CTAs' s
   if (threadIdx.x < STEM_K + STEM_NR) {
     float s = 0.f;
     for (int k = 0; k < n_chunks; ++k) s += mom_part[(size_t)(g * n_chunks + k) * (STEM_K + STEM_NR) + threadIdx.x];
@@ -458,17 +515,12 @@ __global__ void __launch_bounds__(128)
   const float mean = save_mean[(size_t)g * c0 + ch], rstd = save_rstd[(size_t)g * c0 + ch];
   const float sc = rstd * gamma[ch];
   const float inv_n = 1.f / (float)(group * STEM_LC);
+  const float mean_s = stem_shifted_mean(wr, mean, shift);
   dbeta_part[(size_t)g * c0 + ch] = s1;
   dgamma_part[(size_t)g * c0 + ch] = s2;
 #pragma unroll
   for (int t = 0; t < STEM_K; ++t) {
-    float wr_r = 0.f;
-#pragma unroll
-    for (int a = 0; a < STEM_K; ++a) {
-      int lo = a < t ? a : t, hi = a < t ? t : a;
-      wr_r = fmaf(wr[a], xr[STEM_K + stem_r_index(lo, hi)], wr_r);
-    }
-    float h = rstd * (wr_r - mean * xr[t]);
+    const float h = rstd * stem_h_over_rstd(wr, xr, t, mean_s);
     dw_part[((size_t)g * c0 + ch) * STEM_K + t] = sc * (gt[t] - s1 * inv_n * xr[t] - s2 * inv_n * h);
   }
 }
@@ -624,7 +676,7 @@ int launch_stem_bwd(const void* dout, const float* x, const float* w, const floa
   DARDS_CHECK_LAUNCH("stem_bwd");
   if (nc > 1) {
     dim3 cgrid(n_groups, ceil_div(c0, 128));
-    stem_bwd_combine_kernel<<<cgrid, 128, 0, st>>>(w, gamma, save_mean, save_rstd, mom_part, ch_part, dw_part, dgamma_part,
+    stem_bwd_combine_kernel<<<cgrid, 128, 0, st>>>(x, w, gamma, save_mean, save_rstd, mom_part, ch_part, dw_part, dgamma_part,
                                                    dbeta_part, group, nc, c0);
     DARDS_CHECK_LAUNCH("stem_bwd (chunk combine)");
   }
