@@ -113,6 +113,12 @@ _SIGNATURES = {
     "dards_bn_frozen_bwd": [P, P, P, P, P, P, P, P, I, P, P, P, I, I, I, I, I, I, I, I, I, I, P],
     "dards_stem_frozen_chunks": [I],
     "dards_stem_frozen_bwd": [P, P, P, P, P, P, P, P, P, P, I, I, I, I, I, P],
+    "dards_stem_alt_workspace_bytes": [I, I, I, I],
+    "dards_stem_alt_fwd": [P, P, P, P, P, P, P, I, I, I, I, F, P, LL, I, P],
+    "dards_stem_alt_eval_fwd": [P, P, P, P, P, I, I, I, I, P],
+    "dards_stem_alt_bwd": [P, P, P, P, P, P, P, P, P, I, I, I, I, P, LL, I, P],
+    "dards_pool3s2_fwd": [P, P, I, I, I, I, I, I, I, P],
+    "dards_pool3s2_bwd": [P, P, P, I, I, I, I, I, I, I, I, P],
     "dards_avgpool2_fwd": [P, P, I, I, I, I, I, I, P],
     "dards_avgpool2_bwd": [P, P, I, I, I, I, I, I, P],
     "dards_avgpool_full_fwd": [P, P, I, I, I, I, I, P],
@@ -129,7 +135,7 @@ _SIGNATURES = {
     "dards_set_sm_limit": [I],
 }
 _RESTYPES = {"dards_last_error": ctypes.c_char_p, "dards_launch_count": c_longlong, "dards_conv1d_wgrad_workspace_bytes": c_longlong,
-             "dards_stem_workspace_bytes": c_longlong}
+             "dards_stem_workspace_bytes": c_longlong, "dards_stem_alt_workspace_bytes": c_longlong}
 
 EXPORTED_SYMBOLS = tuple(sorted(_SIGNATURES))
 

@@ -76,7 +76,7 @@ def run_plan(net, backbone, linear, x, group, mode, dropout_key=()):
     bn = engine.bn_mode(backbone)
     plan = engine.get_plan(net, backbone, linear, n, group, module_precision(net), mode,
                            dropout=dropout_key if training else (), update_running=training, bn=bn)
-    # Only the parameters the backward writes are inputs of the autograd node.  ResNet's conv1_alt / conv2 / bn2 never
-    # take part in forward() (resnet.py:141-163): in the reference they are not in the graph, their hooks never fire and
+    # Only the parameters the backward writes are inputs of the autograd node.  ResNet's conv1_alt / conv2 / bn2 (conv1 with
+    # double_conv_first=True) never take part in forward() (resnet.py:141-163): in the reference they are not in the graph, their hooks never fire and
     # their .grad stays None -- a None handed to a `p.register_hook(lambda g: g.clamp(...))` hook would raise.
     return PlanFunction.apply(plan, x, *plan.autograd_params())

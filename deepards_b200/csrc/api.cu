@@ -82,6 +82,14 @@ int launch_stem_bwd(const void*, const float*, const float*, const float*, const
                     float*, float*, float*, int, int, int, int, int, void*, long long, int, cudaStream_t);
 long long stem_workspace_bytes(int n_groups, int group, int c0, int backward);
 int launch_avgpool2(int, const void*, void*, int, int, int, int, int, int, cudaStream_t);
+long long stem_alt_workspace_bytes(int n_groups, int group, int c0, int backward);
+int launch_stem_alt_fwd(const float*, const float*, const float*, const float*, void*, float*, float*, int, int, int, int,
+                        float, void*, long long, int, cudaStream_t);
+int launch_stem_alt_eval_fwd(const float*, const float*, const float*, const float*, void*, int, int, int, int,
+                             cudaStream_t);
+int launch_stem_alt_bwd(const void*, const float*, const float*, const float*, const float*, const float*, float*, float*,
+                        float*, int, int, int, int, void*, long long, int, cudaStream_t);
+int launch_pool3s2(int, const void*, const void*, void*, int, int, int, int, int, int, int, int, cudaStream_t);
 int launch_avgpool_full_fwd(const void*, float*, int, int, int, int, int, cudaStream_t);
 int launch_avgpool_full_bwd(const float*, void*, int, int, int, int, int, cudaStream_t);
 int launch_dropout(void*, int, int, int, float, unsigned long long, const unsigned long long*, int, int, cudaStream_t);
@@ -443,6 +451,55 @@ int dards_stem_bwd(const void* dout, const float* x, const float* w, const float
   DARDS_CHECK_ARG(pool == 0 || pool == 1, "stem_bwd: pool must be 0 (max) or 1 (avg)");
   return launch_stem_bwd(dout, x, w, gamma, beta, save_mean, save_rstd, dw_part, dgamma_part, dbeta_part, n_groups, group,
                          c0, dout_stride, pool, workspace, workspace_bytes, dtype, S(stream));
+}
+
+long long dards_stem_alt_workspace_bytes(int n_groups, int group, int c0, int backward) {
+  return stem_alt_workspace_bytes(n_groups, group, c0, backward ? 1 : 0);
+}
+
+int dards_stem_alt_fwd(const float* x, const float* w, const float* gamma, const float* beta, void* out, float* save_mean,
+                       float* save_rstd, int n_groups, int group, int c0, int out_stride, float eps, void* workspace,
+                       long long workspace_bytes, int dtype, void* stream) {
+  DARDS_CHECK_ARG(x && w && gamma && beta && out && save_mean && save_rstd, "stem_alt_fwd: null pointer");
+  DARDS_CHECK_ARG(n_groups >= 0, "stem_alt_fwd: negative number of groups");
+  DARDS_CHECK_ARG(out_stride >= c0, "stem_alt_fwd: row stride smaller than channel count");
+  return launch_stem_alt_fwd(x, w, gamma, beta, out, save_mean, save_rstd, n_groups, group, c0, out_stride, eps, workspace,
+                             workspace_bytes, dtype, S(stream));
+}
+
+int dards_stem_alt_eval_fwd(const float* x, const float* w, const float* scale, const float* shift, void* out,
+                            int n_breaths, int c0, int out_stride, int dtype, void* stream) {
+  DARDS_CHECK_ARG(x && w && scale && shift && out, "stem_alt_eval_fwd: null pointer");
+  DARDS_CHECK_ARG(n_breaths >= 0, "stem_alt_eval_fwd: negative number of breaths");
+  DARDS_CHECK_ARG(out_stride >= c0, "stem_alt_eval_fwd: row stride smaller than channel count");
+  return launch_stem_alt_eval_fwd(x, w, scale, shift, out, n_breaths, c0, out_stride, dtype, S(stream));
+}
+
+int dards_stem_alt_bwd(const void* dout, const float* x, const float* w, const float* gamma, const float* save_mean,
+                       const float* save_rstd, float* dw_part, float* dgamma_part, float* dbeta_part, int n_groups, int group,
+                       int c0, int dout_stride, void* workspace, long long workspace_bytes, int dtype, void* stream) {
+  DARDS_CHECK_ARG(dout && x && w && gamma && save_mean && save_rstd && dw_part && dgamma_part && dbeta_part,
+                  "stem_alt_bwd: null pointer");
+  DARDS_CHECK_ARG(n_groups >= 0, "stem_alt_bwd: negative number of groups");
+  DARDS_CHECK_ARG(dout_stride >= c0, "stem_alt_bwd: row stride smaller than channel count");
+  return launch_stem_alt_bwd(dout, x, w, gamma, save_mean, save_rstd, dw_part, dgamma_part, dbeta_part, n_groups, group, c0,
+                             dout_stride, workspace, workspace_bytes, dtype, S(stream));
+}
+
+int dards_pool3s2_fwd(const void* in, void* out, int n_breaths, int l_in, int c, int in_stride, int out_stride, int pool,
+                      int dtype, void* stream) {
+  DARDS_CHECK_ARG(in && out, "pool3s2_fwd: null pointer");
+  DARDS_CHECK_ARG(n_breaths >= 0, "pool3s2_fwd: negative number of breaths");
+  DARDS_CHECK_ARG(pool == 0 || pool == 1, "pool3s2_fwd: pool must be 0 (max) or 1 (avg)");
+  return launch_pool3s2(0, in, nullptr, out, n_breaths, l_in, c, in_stride, in_stride, out_stride, pool, dtype, S(stream));
+}
+
+int dards_pool3s2_bwd(const void* dout, const void* in, void* din, int n_breaths, int l_in, int c, int dout_stride,
+                      int in_stride, int din_stride, int pool, int dtype, void* stream) {
+  DARDS_CHECK_ARG(dout && din && (in || pool == 1), "pool3s2_bwd: null pointer");
+  DARDS_CHECK_ARG(n_breaths >= 0, "pool3s2_bwd: negative number of breaths");
+  DARDS_CHECK_ARG(pool == 0 || pool == 1, "pool3s2_bwd: pool must be 0 (max) or 1 (avg)");
+  return launch_pool3s2(1, dout, in, din, n_breaths, l_in, c, dout_stride, in_stride, din_stride, pool, dtype, S(stream));
 }
 
 int dards_avgpool2_fwd(const void* in, void* out, int n_breaths, int l_in, int c, int in_stride, int out_stride,

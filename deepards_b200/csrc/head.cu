@@ -325,6 +325,107 @@ int launch_avgpool2(int bwd, const void* src, void* dst, int n_breaths, int l_in
   return DARDS_OK;
 }
 
+// ---- Max/AvgPool1d(3, 2, padding 1): (N,L,C) -> (N,(L-1)/2+1,C), the first pool of the two-convolution ResNet stem ------
+// Output q covers inputs 2q-1, 2q, 2q+1; index -1 (and L when L is even) is padding: -inf for max, 0 counted in the
+// divisor for avg (count_include_pad).  The max backward recomputes the window's arg-max from the stored input and routes
+// the gradient to its FIRST maximum (ATen's rule); each input gathers from the one or two windows that contain it, so
+// there are no atomics and the result is deterministic.
+__device__ __forceinline__ float pool3_pick(float v, int idx, float& best, int& arg) {
+  if (v > best) {
+    best = v;
+    arg = idx;
+  }
+  return best;
+}
+
+template <typename T>
+__global__ void pool3s2_fwd_kernel(const T* __restrict__ in, T* __restrict__ out, long long rows_out, int l_in, int l_out,
+                                   int c4, int in_stride, int out_stride, int pool) {
+  const long long total = rows_out * c4;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int cq = (int)(i % c4);
+    const long long r = i / c4;  // n*l_out + q
+    const long long n = r / l_out;
+    const int q = (int)(r % l_out);
+    const T* src = in + (size_t)n * l_in * in_stride + cq * 4;
+    float v[3][4];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      const int p = 2 * q - 1 + k;
+      const bool ok = p >= 0 && p < l_in;
+      const float4 a = ok ? Elem<T>::ld4(src + (size_t)p * in_stride) : make_float4(0.f, 0.f, 0.f, 0.f);
+      const float pad = pool == 0 ? -INFINITY : 0.f;
+      v[k][0] = ok ? a.x : pad; v[k][1] = ok ? a.y : pad; v[k][2] = ok ? a.z : pad; v[k][3] = ok ? a.w : pad;
+    }
+    float o[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      o[j] = pool == 0 ? fmaxf(fmaxf(v[0][j], v[1][j]), v[2][j]) : (v[0][j] + v[1][j] + v[2][j]) * (1.f / 3.f);
+    Elem<T>::st4(out + (size_t)r * out_stride + cq * 4, make_float4(o[0], o[1], o[2], o[3]));
+  }
+}
+
+template <typename T>
+__global__ void pool3s2_bwd_kernel(const T* __restrict__ dout, const T* __restrict__ in, T* __restrict__ din,
+                                   long long rows_in, int l_in, int l_out, int c4, int dout_stride, int in_stride,
+                                   int din_stride, int pool) {
+  const long long total = rows_in * c4;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int cq = (int)(i % c4);
+    const long long r = i / c4;  // n*l_in + p
+    const long long n = r / l_in;
+    const int p = (int)(r % l_in);
+    float acc[4] = {0.f, 0.f, 0.f, 0.f};
+    // windows q with 2q-1 <= p <= 2q+1, in increasing q
+    for (int q = p / 2; q <= (p + 1) / 2; ++q) {
+      if (q >= l_out || 2 * q - 1 > p) continue;
+      const float4 d = Elem<T>::ld4(dout + ((size_t)n * l_out + q) * dout_stride + cq * 4);
+      const float dv[4] = {d.x, d.y, d.z, d.w};
+      if (pool != 0) {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[j] += dv[j] * (1.f / 3.f);
+        continue;
+      }
+      float best[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
+      int arg[4] = {-1, -1, -1, -1};
+      for (int k = 0; k < 3; ++k) {
+        const int pp = 2 * q - 1 + k;
+        if (pp < 0 || pp >= l_in) continue;
+        const float4 a = Elem<T>::ld4(in + ((size_t)n * l_in + pp) * in_stride + cq * 4);
+        pool3_pick(a.x, pp, best[0], arg[0]);
+        pool3_pick(a.y, pp, best[1], arg[1]);
+        pool3_pick(a.z, pp, best[2], arg[2]);
+        pool3_pick(a.w, pp, best[3], arg[3]);
+      }
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+        if (arg[j] == p) acc[j] += dv[j];
+    }
+    Elem<T>::st4(din + (size_t)r * din_stride + cq * 4, make_float4(acc[0], acc[1], acc[2], acc[3]));
+  }
+}
+
+int launch_pool3s2(int bwd, const void* dout_or_in, const void* in, void* dst, int n_breaths, int l_in, int c,
+                   int src_stride, int in_stride, int dst_stride, int pool, int dtype, cudaStream_t st) {
+  DARDS_CHECK_ARG(l_in >= 1 && c % 4 == 0 && src_stride % 4 == 0 && in_stride % 4 == 0 && dst_stride % 4 == 0,
+                  "pool3s2: channels/strides must be multiples of 4");
+  const int l_out = (l_in - 1) / 2 + 1;
+  const long long rows = (long long)n_breaths * (bwd ? l_in : l_out);
+  if (rows == 0) return DARDS_OK;
+  const int blocks = grid_for(rows * (c / 4), 256);
+  DARDS_DISPATCH_DTYPE(dtype, {
+    if (!bwd)
+      pool3s2_fwd_kernel<T><<<blocks, 256, 0, st>>>(static_cast<const T*>(dout_or_in), static_cast<T*>(dst), rows, l_in,
+                                                    l_out, c / 4, src_stride, dst_stride, pool);
+    else
+      pool3s2_bwd_kernel<T><<<blocks, 256, 0, st>>>(static_cast<const T*>(dout_or_in), static_cast<const T*>(in),
+                                                    static_cast<T*>(dst), rows, l_in, l_out, c / 4, src_stride, in_stride,
+                                                    dst_stride, pool);
+  })
+  DARDS_CHECK_LAUNCH("pool3s2");
+  return DARDS_OK;
+}
+
 int launch_avgpool_full_fwd(const void* in, float* feat, int n_breaths, int l, int c, int in_stride, int dtype,
                             cudaStream_t st) {
   DARDS_CHECK_ARG(c % 4 == 0 && in_stride % 4 == 0, "avgpool: channels/stride must be multiples of 4");

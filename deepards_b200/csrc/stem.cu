@@ -23,6 +23,8 @@
 //             The moments and G_t are sums of x - s, with s the mean of the group's first breath when the input has a DC
 //             offset (read by every chunk CTA, so their partial sums still add): with raw sums the formula cancels digits.
 // The caller provides the workspace for the chunk records (stem_workspace_bytes).
+//
+// The second half of the file is stage 1 of the two-convolution stem (double_conv_first), see stem_alt_fwd_kernel.
 #include "common.cuh"
 
 namespace dards {
@@ -706,6 +708,444 @@ int launch_stem_frozen_bwd(const void* dout, const float* x, const float* w, con
   })
   if (rc) return rc;
   DARDS_CHECK_LAUNCH("stem_frozen_bwd");
+  return DARDS_OK;
+}
+
+
+// ==== stage 1 of the two-convolution stem (ResNet double_conv_first=True, resnet.py:145-147) ===========================
+// a0 = bn1(conv1_alt(x)): Conv1d(1->C0, k3, s1, p1) + grouped BatchNorm, no ReLU, no pool; x (N,224) fp32 -> a0 (N,224,C0)
+// channels-last in the plan dtype.  a0 is materialised: the following Conv1d(C0->C0, k7, s2, p3) runs on the generic
+// convolution kernels, and it zero-pads a0 (the BatchNorm output), so the two convolutions do not fold into one.
+// Same CTA layout, chunking and Chan merge as the stem above (group x 16 channels per CTA, x staged in shared memory);
+// every sweep walks runs of 32 positions with the 3-tap window in registers.
+constexpr int S1_K = 3;
+constexpr int S1_RUN = 32;                      // positions per run: 7 runs per breath
+constexpr int S1_RUNS = STEM_L / S1_RUN;
+constexpr int S1_NR = S1_K * (S1_K + 1) / 2;    // distinct entries of the 3x3 autocorrelation matrix: 6
+constexpr int S1_NM = S1_K + S1_NR;             // input moments: X_t (3) then R (6)
+constexpr int S1_NC = 2 + S1_K;                 // per-channel backward sums: S1, S2, G_t (3)
+
+__device__ __forceinline__ int s1_r_index(int a, int b) { return a * S1_K - a * (a - 1) / 2 + (b - a); }  // a <= b
+
+// MODE: STEM_FUSED / STEM_STATS / STEM_APPLY / STEM_EVAL, as stem_fwd_kernel
+template <typename T, int MODE>
+__global__ void __launch_bounds__(STEM_THREADS)
+    stem_alt_fwd_kernel(const float* __restrict__ x, const float* __restrict__ w, const float* __restrict__ gamma,
+                        const float* __restrict__ beta, T* __restrict__ out, float* __restrict__ save_mean,
+                        float* __restrict__ save_rstd, float* __restrict__ part, int group, int chunk, int n_chunks, int c0,
+                        int out_stride, float eps) {
+  extern __shared__ __align__(16) float xs[];
+  __shared__ float red[STEM_THREADS];
+  __shared__ float xt[S1_K];
+  const int g = blockIdx.x / n_chunks, k = blockIdx.x % n_chunks;
+  const int b0 = k * chunk;
+  const int nb = min(chunk, group - b0);
+  const size_t breath0 = (size_t)g * group + b0;
+  const int c = threadIdx.x % STEM_CS, rl = threadIdx.x / STEM_CS;
+  const int ch = blockIdx.y * STEM_CS + c;
+  stem_load_group(x + breath0 * STEM_L, xs, nb);
+  __syncthreads();
+  const float w0 = w[ch * S1_K], w1 = w[ch * S1_K + 1], w2 = w[ch * S1_K + 2];
+  const int n_runs = nb * S1_RUNS;
+  float sc, sh;
+  if (MODE == STEM_EVAL) {
+    sc = gamma[ch];
+    sh = beta[ch];
+  } else {
+    float mean, var;
+    if (MODE != STEM_APPLY) {
+      const float inv_n = 1.f / (float)(nb * STEM_L);
+      // X_t = sum over positions of x[l + t - 1] (channel independent)
+      float a0 = 0.f, a1 = 0.f, a2 = 0.f;
+      for (int i = threadIdx.x; i < nb * STEM_L; i += STEM_THREADS) {
+        const float* xb = xs + (i / STEM_L) * STEM_BS + STEM_PAD + (i % STEM_L) - 1;
+        a0 += xb[0];
+        a1 += xb[1];
+        a2 += xb[2];
+      }
+      a0 = warp_sum(a0);
+      a1 = warp_sum(a1);
+      a2 = warp_sum(a2);
+      const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+      if (lane == 0) {
+        red[warp * S1_K] = a0;
+        red[warp * S1_K + 1] = a1;
+        red[warp * S1_K + 2] = a2;
+      }
+      __syncthreads();
+      if (threadIdx.x < S1_K) {
+        float s = 0.f;
+        for (int wv = 0; wv < STEM_THREADS / 32; ++wv) s += red[wv * S1_K + threadIdx.x];
+        xt[threadIdx.x] = s;
+      }
+      __syncthreads();
+      mean = fmaf(w0, xt[0], fmaf(w1, xt[1], w2 * xt[2])) * inv_n;
+      // centred sum of squares
+      float q = 0.f;
+      for (int run = rl; run < n_runs; run += STEM_LANES) {
+        const float* xb = xs + (run / S1_RUNS) * STEM_BS + STEM_PAD + (run % S1_RUNS) * S1_RUN - 1;
+        float x0 = xb[0], x1 = xb[1];
+#pragma unroll 8
+        for (int j = 0; j < S1_RUN; ++j) {
+          const float x2 = xb[j + 2];
+          const float d = fmaf(w0, x0, fmaf(w1, x1, w2 * x2)) - mean;
+          q = fmaf(d, d, q);
+          x0 = x1;
+          x1 = x2;
+        }
+      }
+      const float m2 = stem_lane_sum(q, red, c, rl);
+      if (MODE == STEM_STATS) {
+        if (rl == 0) {
+          float* r = part + (size_t)blockIdx.x * 3 * c0 + ch;
+          r[0] = (float)(nb * STEM_L);
+          r[c0] = mean;
+          r[2 * c0] = m2;
+        }
+        return;
+      }
+      var = m2 * inv_n + eps;
+    } else {
+      float n = 0.f, m2 = 0.f;
+      mean = 0.f;
+      for (int kk = 0; kk < n_chunks; ++kk) {
+        const float* r = part + (size_t)(g * n_chunks + kk) * 3 * c0 + ch;
+        const float ne = r[0], me = r[c0], qe = r[2 * c0];
+        const float nn = n + ne, d = me - mean;
+        mean += d * (ne / nn);
+        m2 += qe + d * d * (n * ne / nn);
+        n = nn;
+      }
+      var = m2 / n + eps;
+    }
+    float rstd = rsqrtf(var);
+    rstd = rstd * (1.5f - 0.5f * var * rstd * rstd);
+    if (rl == 0 && k == 0) {
+      save_mean[(size_t)g * c0 + ch] = mean;
+      save_rstd[(size_t)g * c0 + ch] = rstd;
+    }
+    sc = rstd * gamma[ch];
+    sh = beta[ch] - mean * sc;
+  }
+  for (int run = rl; run < n_runs; run += STEM_LANES) {
+    const int b = run / S1_RUNS, l0 = (run % S1_RUNS) * S1_RUN;
+    const float* xb = xs + b * STEM_BS + STEM_PAD + l0 - 1;
+    T* op = out + ((breath0 + b) * STEM_L + l0) * out_stride + ch;
+    float x0 = xb[0], x1 = xb[1];
+#pragma unroll 8
+    for (int j = 0; j < S1_RUN; ++j) {
+      const float x2 = xb[j + 2];
+      Elem<T>::st(op + (size_t)j * out_stride, fmaf(fmaf(w0, x0, fmaf(w1, x1, w2 * x2)), sc, sh));
+      x0 = x1;
+      x1 = x2;
+    }
+  }
+}
+
+// H_t / rstd = sum_a w_a R'[a][t] - mean_s X'_t (as stem_h_over_rstd, 3 taps)
+__device__ __forceinline__ float s1_h_over_rstd(const float (&w)[S1_K], const float* xr, int t, float mean_s) {
+  float wr_r = 0.f;
+#pragma unroll
+  for (int a = 0; a < S1_K; ++a) {
+    const int lo = a < t ? a : t, hi = a < t ? t : a;
+    wr_r = fmaf(w[a], xr[S1_K + s1_r_index(lo, hi)], wr_r);
+  }
+  return wr_r - mean_s * xr[t];
+}
+
+// BatchNorm backward (no ReLU) folded into the weight gradient, from the group totals: see stem_bwd_kernel section C
+__device__ __forceinline__ void s1_finish(const float (&w)[S1_K], const float* xr, float s1, float s2, const float (&gt)[S1_K],
+                                          float mean, float rstd, float gm, float shift, float inv_n, float* dw,
+                                          float* dgamma, float* dbeta) {
+  const float sc = rstd * gm;
+  const float mean_s = fmaf(-shift, w[0] + w[1] + w[2], mean);
+  *dbeta = s1;
+  *dgamma = s2;
+#pragma unroll
+  for (int t = 0; t < S1_K; ++t) {
+    const float h = rstd * s1_h_over_rstd(w, xr, t, mean_s);
+    dw[t] = sc * (gt[t] - s1 * inv_n * xr[t] - s2 * inv_n * h);
+  }
+}
+
+// dout (N,224,C0) = d a0 -> per-group partials of dW (C0 x 3), dgamma, dbeta.  The input moments and G_t are sums of
+// x - s, s the group shift of stem_group_shift (the same rule and arithmetic as the stem backward).
+// PARTIAL: one CTA = one chunk of a group; moments and per-channel sums go to the workspace (stem_alt_bwd_combine_kernel).
+template <typename T, bool PARTIAL>
+__global__ void __launch_bounds__(STEM_THREADS)
+    stem_alt_bwd_kernel(const T* __restrict__ dout, const float* __restrict__ x, const float* __restrict__ w,
+                        const float* __restrict__ gamma, const float* __restrict__ save_mean,
+                        const float* __restrict__ save_rstd, float* __restrict__ dw_part, float* __restrict__ dgamma_part,
+                        float* __restrict__ dbeta_part, float* __restrict__ mom_part, float* __restrict__ ch_part,
+                        int group_all, int chunk, int n_chunks, int c0, int dout_stride) {
+  extern __shared__ __align__(16) float xs[];
+  __shared__ float red[STEM_THREADS * S1_NC];
+  __shared__ float xr[S1_NM];
+  const int g = blockIdx.x / n_chunks, kc = blockIdx.x % n_chunks;
+  const int b0 = kc * chunk;
+  const int group = min(chunk, group_all - b0);
+  const size_t breath0 = (size_t)g * group_all + b0;
+  const int tid = threadIdx.x;
+  const int c = tid % STEM_CS, rl = tid / STEM_CS;
+  const int ch = blockIdx.y * STEM_CS + c;
+  const float shift = stem_group_shift(x + (size_t)g * group_all * STEM_L, red + STEM_THREADS * S1_NC - 16);
+  stem_load_group(x + breath0 * STEM_L, xs, group);
+  __syncthreads();
+  const int n_pos = group * STEM_L;
+
+  // ---- A. input moments about s: X'_t = sum (xin_t - s), R'[a][b] = sum (xin_a - s)(xin_b - s) ----------------
+  {
+    float acc[S1_NM];
+#pragma unroll
+    for (int i = 0; i < S1_NM; ++i) acc[i] = 0.f;
+    for (int i = tid; i < n_pos; i += STEM_THREADS) {
+      const float* xb = xs + (i / STEM_L) * STEM_BS + STEM_PAD + (i % STEM_L) - 1;
+      float xin[S1_K];
+#pragma unroll
+      for (int t = 0; t < S1_K; ++t) xin[t] = xb[t] - shift;
+      int k = S1_K;
+#pragma unroll
+      for (int a = 0; a < S1_K; ++a) {
+        acc[a] += xin[a];
+#pragma unroll
+        for (int b = a; b < S1_K; ++b) {
+          acc[k] = fmaf(xin[a], xin[b], acc[k]);
+          ++k;
+        }
+      }
+    }
+#pragma unroll
+    for (int i = 0; i < S1_NM; ++i) acc[i] = warp_sum(acc[i]);
+    const int warp = tid >> 5, lane = tid & 31;
+    __syncthreads();  // the shift's scratch in red is read
+    if (lane == 0) {
+#pragma unroll
+      for (int i = 0; i < S1_NM; ++i) red[warp * S1_NM + i] = acc[i];
+    }
+    __syncthreads();
+    if (tid < S1_NM) {
+      float s = 0.f;
+      for (int wv = 0; wv < STEM_THREADS / 32; ++wv) s += red[wv * S1_NM + tid];
+      xr[tid] = s;
+      if (PARTIAL && blockIdx.y == 0) mom_part[(size_t)blockIdx.x * S1_NM + tid] = s;
+    }
+    __syncthreads();
+  }
+
+  // ---- B. per channel: S1 = sum g, S2 = sum g*xhat, G'_t = sum g * (xin_t - s) --------------------------------
+  float wr[S1_K];
+#pragma unroll
+  for (int t = 0; t < S1_K; ++t) wr[t] = w[ch * S1_K + t];
+  const float mean = save_mean[(size_t)g * c0 + ch], rstd = save_rstd[(size_t)g * c0 + ch];
+  float s1 = 0.f, s2 = 0.f, gt[S1_K] = {0.f, 0.f, 0.f};
+  const int n_runs = group * S1_RUNS;
+  for (int run = rl; run < n_runs; run += STEM_LANES) {
+    const int b = run / S1_RUNS, l0 = (run % S1_RUNS) * S1_RUN;
+    const float* xb = xs + b * STEM_BS + STEM_PAD + l0 - 1;
+    const T* dp = dout + ((breath0 + b) * STEM_L + l0) * dout_stride + ch;
+    float x0 = xb[0], x1 = xb[1];
+#pragma unroll 8
+    for (int j = 0; j < S1_RUN; ++j) {
+      const float x2 = xb[j + 2];
+      const float gv = Elem<T>::ld(dp + (size_t)j * dout_stride);
+      const float y = fmaf(wr[0], x0, fmaf(wr[1], x1, wr[2] * x2));
+      s1 += gv;
+      s2 = fmaf(gv, (y - mean) * rstd, s2);
+      gt[0] = fmaf(gv, x0 - shift, gt[0]);
+      gt[1] = fmaf(gv, x1 - shift, gt[1]);
+      gt[2] = fmaf(gv, x2 - shift, gt[2]);
+      x0 = x1;
+      x1 = x2;
+    }
+  }
+  __syncthreads();
+  red[tid * S1_NC + 0] = s1;
+  red[tid * S1_NC + 1] = s2;
+#pragma unroll
+  for (int t = 0; t < S1_K; ++t) red[tid * S1_NC + 2 + t] = gt[t];
+  __syncthreads();
+  if (rl != 0) return;
+  s1 = s2 = 0.f;
+#pragma unroll
+  for (int t = 0; t < S1_K; ++t) gt[t] = 0.f;
+  for (int r = 0; r < STEM_LANES; ++r) {
+    const int o = (r * STEM_CS + c) * S1_NC;
+    s1 += red[o + 0];
+    s2 += red[o + 1];
+#pragma unroll
+    for (int t = 0; t < S1_K; ++t) gt[t] += red[o + 2 + t];
+  }
+  if (PARTIAL) {
+    float* o = ch_part + (size_t)blockIdx.x * S1_NC * c0 + ch;
+    o[0] = s1;
+    o[c0] = s2;
+#pragma unroll
+    for (int t = 0; t < S1_K; ++t) o[(size_t)(2 + t) * c0] = gt[t];
+    return;
+  }
+  const size_t o = (size_t)g * c0 + ch;
+  s1_finish(wr, xr, s1, s2, gt, mean, rstd, gamma[ch], shift, 1.f / (float)n_pos, dw_part + o * S1_K, dgamma_part + o,
+            dbeta_part + o);
+}
+
+// chunked backward, second pass: thread = channel of one group; adds the chunk partials in order, then s1_finish
+__global__ void __launch_bounds__(128)
+    stem_alt_bwd_combine_kernel(const float* __restrict__ x, const float* __restrict__ w, const float* __restrict__ gamma,
+                                const float* __restrict__ save_mean, const float* __restrict__ save_rstd,
+                                const float* __restrict__ mom_part, const float* __restrict__ ch_part,
+                                float* __restrict__ dw_part, float* __restrict__ dgamma_part, float* __restrict__ dbeta_part,
+                                int group, int n_chunks, int c0) {
+  __shared__ float xr[S1_NM];
+  __shared__ float shift_red[16];
+  const int g = blockIdx.x;
+  const float shift = stem_group_shift(x + (size_t)g * group * STEM_L, shift_red);
+  if (threadIdx.x < S1_NM) {
+    float s = 0.f;
+    for (int k = 0; k < n_chunks; ++k) s += mom_part[(size_t)(g * n_chunks + k) * S1_NM + threadIdx.x];
+    xr[threadIdx.x] = s;
+  }
+  __syncthreads();
+  const int ch = blockIdx.y * 128 + threadIdx.x;
+  if (ch >= c0) return;
+  float s1 = 0.f, s2 = 0.f, gt[S1_K] = {0.f, 0.f, 0.f};
+  for (int k = 0; k < n_chunks; ++k) {
+    const float* o = ch_part + (size_t)(g * n_chunks + k) * S1_NC * c0 + ch;
+    s1 += o[0];
+    s2 += o[c0];
+#pragma unroll
+    for (int t = 0; t < S1_K; ++t) gt[t] += o[(size_t)(2 + t) * c0];
+  }
+  float wr[S1_K];
+#pragma unroll
+  for (int t = 0; t < S1_K; ++t) wr[t] = w[ch * S1_K + t];
+  const size_t o = (size_t)g * c0 + ch;
+  s1_finish(wr, xr, s1, s2, gt, save_mean[o], save_rstd[o], gamma[ch], shift, 1.f / (float)(group * STEM_L),
+            dw_part + o * S1_K, dgamma_part + o, dbeta_part + o);
+}
+
+long long stem_alt_workspace_bytes(int n_groups, int group, int c0, int backward) {
+  const int nc = stem_n_chunks(group);
+  if (nc == 1 || n_groups <= 0 || c0 <= 0) return 0;
+  const long long recs = (long long)n_groups * nc;
+  return (backward ? recs * ((long long)S1_NC * c0 + S1_NM) : recs * 3LL * c0) * (long long)sizeof(float);
+}
+
+int launch_stem_alt_fwd(const float* x, const float* w, const float* gamma, const float* beta, void* out, float* save_mean,
+                        float* save_rstd, int n_groups, int group, int c0, int out_stride, float eps, void* workspace,
+                        long long workspace_bytes, int dtype, cudaStream_t st) {
+  DARDS_CHECK_ARG(stem_c0_ok(c0), "stem_alt: initial planes must be a multiple of %d (got %d)", STEM_CS, c0);
+  DARDS_CHECK_ARG(group > 0, "stem_alt: BatchNorm group must be at least 1 breath (got %d)", group);
+  if (n_groups == 0) return DARDS_OK;
+  DARDS_CHECK_ARG(c0 / STEM_CS <= 65535, "stem_alt: grid too large");
+  const int nc = stem_n_chunks(group);
+  if (nc == 1) {
+    const size_t smem = (size_t)group * STEM_BS * sizeof(float);
+    dim3 grid(n_groups, c0 / STEM_CS);
+    static size_t granted[2] = {44 * 1024, 44 * 1024};
+    DARDS_DISPATCH_DTYPE(dtype, {
+      int rc = stem_smem_optin(stem_alt_fwd_kernel<T, STEM_FUSED>, smem, &granted[dtype == DARDS_BF16 ? 1 : 0]);
+      if (rc) return rc;
+      stem_alt_fwd_kernel<T, STEM_FUSED><<<grid, STEM_THREADS, smem, st>>>(x, w, gamma, beta, static_cast<T*>(out), save_mean,
+                                                                          save_rstd, nullptr, group, group, 1, c0,
+                                                                          out_stride, eps);
+    })
+    DARDS_CHECK_LAUNCH("stem_alt_fwd");
+    return DARDS_OK;
+  }
+  const long long need = stem_alt_workspace_bytes(n_groups, group, c0, 0);
+  DARDS_CHECK_ARG(workspace != nullptr && workspace_bytes >= need,
+                  "stem_alt_fwd: a BatchNorm group of %d breaths runs in chunks and needs %lld bytes of workspace (got %lld)",
+                  group, need, workspace_bytes);
+  DARDS_CHECK_ARG((long long)n_groups * nc <= 0x7fffffffLL, "stem_alt: grid too large");
+  float* part = static_cast<float*>(workspace);
+  const size_t smem = (size_t)STEM_CHUNK * STEM_BS * sizeof(float);
+  dim3 grid((unsigned)(n_groups * nc), c0 / STEM_CS);
+  static size_t granted[4] = {44 * 1024, 44 * 1024, 44 * 1024, 44 * 1024};
+  DARDS_DISPATCH_DTYPE(dtype, {
+    const int slot = dtype == DARDS_BF16 ? 1 : 0;
+    int rc = stem_smem_optin(stem_alt_fwd_kernel<T, STEM_STATS>, smem, &granted[slot]);
+    if (rc) return rc;
+    rc = stem_smem_optin(stem_alt_fwd_kernel<T, STEM_APPLY>, smem, &granted[2 + slot]);
+    if (rc) return rc;
+    stem_alt_fwd_kernel<T, STEM_STATS><<<grid, STEM_THREADS, smem, st>>>(x, w, gamma, beta, static_cast<T*>(out), save_mean,
+                                                                        save_rstd, part, group, STEM_CHUNK, nc, c0,
+                                                                        out_stride, eps);
+    DARDS_CHECK_LAUNCH("stem_alt_fwd (chunk statistics)");
+    stem_alt_fwd_kernel<T, STEM_APPLY><<<grid, STEM_THREADS, smem, st>>>(x, w, gamma, beta, static_cast<T*>(out), save_mean,
+                                                                        save_rstd, part, group, STEM_CHUNK, nc, c0,
+                                                                        out_stride, eps);
+  })
+  DARDS_CHECK_LAUNCH("stem_alt_fwd (chunk apply)");
+  return DARDS_OK;
+}
+
+int launch_stem_alt_eval_fwd(const float* x, const float* w, const float* scale, const float* shift, void* out,
+                             int n_breaths, int c0, int out_stride, int dtype, cudaStream_t st) {
+  DARDS_CHECK_ARG(stem_c0_ok(c0), "stem_alt: initial planes must be a multiple of %d (got %d)", STEM_CS, c0);
+  if (n_breaths == 0) return DARDS_OK;
+  DARDS_CHECK_ARG(c0 / STEM_CS <= 65535, "stem_alt: grid too large");
+  const int nc = ceil_div(n_breaths, STEM_CHUNK);
+  const size_t smem = (size_t)STEM_CHUNK * STEM_BS * sizeof(float);
+  dim3 grid((unsigned)nc, c0 / STEM_CS);
+  static size_t granted[2] = {44 * 1024, 44 * 1024};
+  DARDS_DISPATCH_DTYPE(dtype, {
+    int rc = stem_smem_optin(stem_alt_fwd_kernel<T, STEM_EVAL>, smem, &granted[dtype == DARDS_BF16 ? 1 : 0]);
+    if (rc) return rc;
+    stem_alt_fwd_kernel<T, STEM_EVAL><<<grid, STEM_THREADS, smem, st>>>(x, w, scale, shift, static_cast<T*>(out), nullptr,
+                                                                       nullptr, nullptr, n_breaths, STEM_CHUNK, nc, c0,
+                                                                       out_stride, 0.f);
+  })
+  DARDS_CHECK_LAUNCH("stem_alt_eval_fwd");
+  return DARDS_OK;
+}
+
+int launch_stem_alt_bwd(const void* dout, const float* x, const float* w, const float* gamma, const float* save_mean,
+                        const float* save_rstd, float* dw_part, float* dgamma_part, float* dbeta_part, int n_groups, int group,
+                        int c0, int dout_stride, void* workspace, long long workspace_bytes, int dtype, cudaStream_t st) {
+  DARDS_CHECK_ARG(stem_c0_ok(c0), "stem_alt: initial planes must be a multiple of %d (got %d)", STEM_CS, c0);
+  DARDS_CHECK_ARG(group > 0, "stem_alt: BatchNorm group must be at least 1 breath (got %d)", group);
+  if (n_groups == 0) return DARDS_OK;
+  DARDS_CHECK_ARG(c0 / STEM_CS <= 65535, "stem_alt: grid too large");
+  const int nc = stem_n_chunks(group);
+  const int chunk = nc == 1 ? group : STEM_CHUNK;
+  float* mom_part = nullptr;
+  float* ch_part = nullptr;
+  if (nc > 1) {
+    const long long need = stem_alt_workspace_bytes(n_groups, group, c0, 1);
+    DARDS_CHECK_ARG(workspace != nullptr && workspace_bytes >= need,
+                    "stem_alt_bwd: a BatchNorm group of %d breaths runs in chunks and needs %lld bytes of workspace (got %lld)",
+                    group, need, workspace_bytes);
+    DARDS_CHECK_ARG((long long)n_groups * nc <= 0x7fffffffLL, "stem_alt: grid too large");
+    ch_part = static_cast<float*>(workspace);
+    mom_part = ch_part + (size_t)n_groups * nc * S1_NC * c0;
+  }
+  const size_t smem = (size_t)chunk * STEM_BS * sizeof(float);
+  dim3 grid((unsigned)(n_groups * nc), c0 / STEM_CS);
+  static size_t granted[4] = {40 * 1024, 40 * 1024, 40 * 1024, 40 * 1024};  // 6 KB of static smem on top
+  DARDS_DISPATCH_DTYPE(dtype, {
+    const int slot = (dtype == DARDS_BF16 ? 1 : 0) + (nc > 1 ? 2 : 0);
+    const T* d = static_cast<const T*>(dout);
+    if (nc > 1) {
+      int rc = stem_smem_optin(stem_alt_bwd_kernel<T, true>, smem, &granted[slot]);
+      if (rc) return rc;
+      stem_alt_bwd_kernel<T, true><<<grid, STEM_THREADS, smem, st>>>(d, x, w, gamma, save_mean, save_rstd, dw_part,
+                                                                     dgamma_part, dbeta_part, mom_part, ch_part, group,
+                                                                     chunk, nc, c0, dout_stride);
+    } else {
+      int rc = stem_smem_optin(stem_alt_bwd_kernel<T, false>, smem, &granted[slot]);
+      if (rc) return rc;
+      stem_alt_bwd_kernel<T, false><<<grid, STEM_THREADS, smem, st>>>(d, x, w, gamma, save_mean, save_rstd, dw_part,
+                                                                      dgamma_part, dbeta_part, nullptr, nullptr, group,
+                                                                      chunk, 1, c0, dout_stride);
+    }
+  })
+  DARDS_CHECK_LAUNCH("stem_alt_bwd");
+  if (nc > 1) {
+    dim3 cgrid(n_groups, ceil_div(c0, 128));
+    stem_alt_bwd_combine_kernel<<<cgrid, 128, 0, st>>>(x, w, gamma, save_mean, save_rstd, mom_part, ch_part, dw_part,
+                                                       dgamma_part, dbeta_part, group, nc, c0);
+    DARDS_CHECK_LAUNCH("stem_alt_bwd (chunk combine)");
+  }
   return DARDS_OK;
 }
 

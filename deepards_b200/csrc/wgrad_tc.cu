@@ -21,7 +21,7 @@
 // the dout tile once instead of three times.
 //
 // Tile: 128 output channels (TMEM lanes) x up to 128 input channels (columns) x up to 3 taps (3 accumulators =
-// 384 TMEM columns).  Split-K over groups of breaths; every CTA writes its fp32 partial tile and a second kernel
+// 384 TMEM columns), or x 64 input channels x 7 taps (the stride-2 k7 convolution, tc_wgrad7_kernel).  Split-K over groups of breaths; every CTA writes its fp32 partial tile and a second kernel
 // reduces the partials in a fixed order (deterministic) into the parameter's (Cout, Cin, K) layout.
 #include <cstring>
 
@@ -69,10 +69,15 @@ struct WgTcParams {
 // the two 64-channel chunks of the input tile (the B operand's N = 128 columns are split between the two CTAs), which cuts
 // the operand stream from 66 to 49 KB per stage -- the single-CTA kernel needs 42 B/clk/SM, exactly the L2 -> SM limit.
 // Barriers as in tc_conv_pair_kernel: full[] in the leader, empty[] / done in both (multicast commits).
-template <bool PAIR>
-__global__ void __launch_bounds__(WG_TC_THREADS, 1)
-    tc_wgrad_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
-                    const __grid_constant__ CUtensorMap tm_d, float* __restrict__ partial, const WgTcParams p) {
+//
+// NT: the tap count the MMA issuer is compiled for.  WG_MAX_TAPS (tc_wgrad_kernel): 1 or 3 taps as p.n_taps says.
+// 7 (tc_wgrad7_kernel): the k7 / stride 2 / pad 3 convolution of the two-convolution ResNet stem, c_in <= 64, single CTA.
+// Its seven 64-column accumulators take 448 of the 512 TMEM columns, and its tap map is fixed: in[2q + t - 3] is, for odd
+// t, plane 0 row q + (t - 3)/2 and, for even t, plane 1 row q + (t - 4)/2; both planes are staged from row -2, so tap t
+// reads tile (t odd ? 0 : 1) shifted by (t + 1)/2 rows.
+template <bool PAIR, int NT>
+__device__ __forceinline__ void tc_wgrad_body(const CUtensorMap& tm_a, const CUtensorMap& tm_b, const CUtensorMap& tm_d,
+                                              float* __restrict__ partial, const WgTcParams& p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
@@ -167,6 +172,47 @@ __global__ void __launch_bounds__(WG_TC_THREADS, 1)
         }
       }
     }
+  } else if (warp == 1 && NT == 7) {
+    const bool issuer = elect_one();
+    // D=f32, A=B=bf16, both MN-major, N = 64, M = 128
+    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(64 >> 3) << 17) |
+                           ((uint32_t)(128 >> 4) << 24);
+    const uint64_t a_tmpl = make_sw128_desc(0, WG_CHUNK_A >> 4, 1024 >> 4, 1, 0);
+    const uint64_t b_tmpl = make_sw128_desc(0, WG_CHUNK_B >> 4, 1024 >> 4, 1, 0);
+    const uint32_t a_hi = (uint32_t)(a_tmpl >> 32), b_hi = (uint32_t)(b_tmpl >> 32);
+    const int k_steps = p.r_pad / 16;
+    const uint32_t stage16 = (uint32_t)p.stage_bytes >> 4;
+    const uint32_t s16_0 = (smem_base & 0x3FFFFu) >> 4;
+    uint32_t s16 = s16_0, fb = full_bar(0), eb = empty_bar(0);
+    int stage = 0;
+    uint32_t phase = 0;
+    for (int it = 0; it < n_iters; ++it) {
+      mbar_wait_tight(fb, phase);
+      tc_fence_after();
+      if (issuer) {
+        uint32_t a_lo = (uint32_t)a_tmpl + s16;
+        uint32_t b[NT];
+#pragma unroll
+        for (int t = 0; t < NT; ++t)
+          b[t] = (uint32_t)b_tmpl + s16 + ((uint32_t)(p.a_bytes + ((t & 1) ? 0 : p.b_bytes) + ((t + 1) >> 1) * 128) >> 4);
+        uint32_t acc = it != 0 ? 1u : 0u;
+        for (int kk = 0; kk < k_steps; ++kk) {
+#pragma unroll
+          for (int t = 0; t < NT; ++t) {
+            umma_bf16_lo2(tmem_base + (uint32_t)(t * 64), a_lo, a_hi, b[t], b_hi, idesc, acc);
+            b[t] += 128;
+          }
+          a_lo += 128;
+          acc = 1u;
+        }
+        umma_commit(eb);
+      }
+      s16 += stage16; fb += 8; eb += 8;
+      if (++stage == p.stages) {
+        stage = 0; phase ^= 1u; s16 = s16_0; fb = full_bar(0); eb = empty_bar(0);
+      }
+    }
+    if (issuer) umma_commit(done_bar);
   } else if (warp == 1) {
     // MMA issuer: whole warp, one elected lane issues; all descriptor arithmetic on the 32-bit low words
     if (!PAIR || lead) {
@@ -342,6 +388,19 @@ __global__ void __launch_bounds__(WG_TC_THREADS, 1)
   }
 }
 
+template <bool PAIR>
+__global__ void __launch_bounds__(WG_TC_THREADS, 1)
+    tc_wgrad_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
+                    const __grid_constant__ CUtensorMap tm_d, float* __restrict__ partial, const WgTcParams p) {
+  tc_wgrad_body<PAIR, WG_MAX_TAPS>(tm_a, tm_b, tm_d, partial, p);
+}
+
+__global__ void __launch_bounds__(WG_TC_THREADS, 1)
+    tc_wgrad7_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
+                     const __grid_constant__ CUtensorMap tm_d, float* __restrict__ partial, const WgTcParams p) {
+  tc_wgrad_body<false, 7>(tm_a, tm_b, tm_d, partial, p);
+}
+
 // dw[co][ci][t] (+)= sum_s partial[s][t][co][ci].  256 threads = (256 / LANES) float4 columns x LANES split lanes; every
 // lane sums its splits in order and the lane sums are combined in a fixed order -> deterministic.  LANES follows the
 // split count so that every thread has ~8-16 independent 16-byte loads in flight: with 9 splits (C = 512) one lane per
@@ -393,14 +452,22 @@ static WgPlan wg_plan(int n_breaths, int l_in, int l_out, int c_in, int c_out, i
   WgPlan w{};
   w.ok = false;
   WgTcParams& p = w.p;
-  if (!((ktaps == 3 && pad == 1) || (ktaps == 1 && pad == 0))) return w;
+  const bool k7 = ktaps == 7 && pad == 3 && stride == 2;  // tc_wgrad7_kernel
+  if (!((ktaps == 3 && pad == 1) || (ktaps == 1 && pad == 0) || k7)) return w;
   if (stride != 1 && stride != 2) return w;
   if (c_in % 16 || c_out % 8 || l_in != l_out * stride) return w;
+  if (k7 && (c_in > 64 || g_dbg_base_offset_mode == 0)) return w;  // 7 x 64 TMEM columns; base offset 0 only
   const int halo = ktaps == 3 ? 1 : 0;
   p.p_rows = l_out + halo;     // dout rows [0, L] (row L = zero fill), input rows [-1, L-1] (row -1 = zero fill)
   p.a_start = 0;
   p.n_taps = ktaps;
-  if (stride == 1) {
+  if (k7) {
+    // dout rows [0, L+2] (3 zero rows), both parity planes staged from row -2 (two zero rows); the tap map is in the kernel
+    p.p_rows = l_out + 3;
+    p.n_btiles = 2;
+    p.b_plane[0] = 0; p.b_start[0] = -2;
+    p.b_plane[1] = 1; p.b_start[1] = -2;
+  } else if (stride == 1) {
     p.n_btiles = 1;
     p.b_plane[0] = 0;
     p.b_start[0] = -halo;  // staged row i = in[i - 1]; tap t of dout row j pairs with staged row j + t
@@ -451,7 +518,7 @@ static WgPlan wg_plan(int n_breaths, int l_in, int l_out, int c_in, int c_out, i
   // memory address bits, so a descriptor whose start is advanced by whole 128-byte rows needs base_offset = 0;
   // base_offset = (start >> 7) & 7 gives wrong results for the shifted taps.
   p.base_offset_mode = g_dbg_base_offset_mode >= 0 ? g_dbg_base_offset_mode : 1;
-  p.tap_cols = p.fuse_taps ? 64 : 128;
+  p.tap_cols = p.fuse_taps || k7 ? 64 : 128;
   p.l2_hint = g_dbg_l2_hint != 0 ? 1 : 0;
   w.ok = true;
   return w;
@@ -478,8 +545,10 @@ int tc_conv_wgrad_accum(const void* in, const void* dout, float* dw_t, int n_bre
 }
 
 long long tc_wgrad_workspace_bytes(int n_breaths, int l_out, int c_in, int c_out, int ktaps) {
-  // the split count does not depend on stride/pad beyond validity; use the stride-1 plan shape
-  WgPlan w = wg_plan(n_breaths, l_out, l_out, c_in, c_out, ktaps, 1, ktaps == 3 ? 1 : 0);
+  // the split count depends on the rows staged per breath: the stride-1 plan shape gives them for k = 1 and 3; k = 7 has
+  // one plan only (stride 2, pad 3)
+  WgPlan w = ktaps == 7 ? wg_plan(n_breaths, 2 * l_out, l_out, c_in, c_out, 7, 2, 3)
+                        : wg_plan(n_breaths, l_out, l_out, c_in, c_out, ktaps, 1, ktaps == 3 ? 1 : 0);
   if (!w.ok) return 0;
   return (long long)w.splits * ktaps * c_in * c_out * (long long)sizeof(float);
 }
@@ -513,6 +582,21 @@ static int wg_launch(WgPlan& w, const void* in, const void* dout, float* partial
     if (rc) return rc;
   }
   const int smem = p.stages * p.stage_bytes + 1024 + 256;
+  dim3 grid(p.n_ci_tiles * p.n_co_tiles, w.splits);
+  if (p.n_taps == 7) {
+    static int attr_smem7 = 0;
+    if (smem > attr_smem7) {
+      cudaError_t e = cudaFuncSetAttribute(tc_wgrad7_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+      if (e != cudaSuccess) {
+        set_error("tcgen05 wgrad (7 taps): cannot opt in to %d bytes of shared memory: %s", smem, cudaGetErrorString(e));
+        return DARDS_ERR_CUDA;
+      }
+      attr_smem7 = smem;
+    }
+    tc_wgrad7_kernel<<<grid, WG_TC_THREADS, smem, st>>>(tm_a, tm_b, tm_d, partial, p);
+    DARDS_CHECK_LAUNCH("tc_wgrad7");
+    return DARDS_OK;
+  }
   static int attr_smem[2] = {0, 0};
   if (smem > attr_smem[p.pair]) {
     cudaError_t e = p.pair ? cudaFuncSetAttribute(tc_wgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)
@@ -523,7 +607,6 @@ static int wg_launch(WgPlan& w, const void* in, const void* dout, float* partial
     }
     attr_smem[p.pair] = smem;
   }
-  dim3 grid(p.n_ci_tiles * p.n_co_tiles, w.splits);
   if (p.pair) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;                 // grid.x is even (c_out % 256 == 0): clusters of 2 along x share blockIdx.y

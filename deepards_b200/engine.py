@@ -77,9 +77,12 @@ class nvtx_range(object):
 
 
 def resnet_bn_layers(backbone):
-    """(name, module) of the BatchNorm layers a ResNet's forward uses (resnet.py:141-163): the stem's bn1 and every block's
-    bn1 / bn2 / downsample BatchNorm.  The stem's bn2 (built by the constructor, never called) is not one of them."""
+    """(name, module) of the BatchNorm layers a ResNet's forward uses (resnet.py:141-163): the stem's bn1, its bn2 with
+    double_conv_first=True (the default stem builds bn2 and never calls it), and every block's bn1 / bn2 / downsample
+    BatchNorm."""
     out = [("bn1", backbone.bn1)]
+    if backbone.double_conv_first:
+        out.append(("bn2", backbone.bn2))
     for li, layer in enumerate((backbone.layer1, backbone.layer2, backbone.layer3, backbone.layer4), 1):
         for bi, blk in enumerate(layer):
             pre = "layer%d.%d." % (li, bi)
@@ -309,7 +312,9 @@ class Plan(object):
         if direction == "wgrad":
             if "wgrad" in _conv_impl_override():
                 return False
-            return ((c.k == 3 and c.pad == 1) or (c.k == 1 and c.pad == 0)) and c.cin % 16 == 0 and c.cout % 8 == 0
+            # k7 / stride 2 / pad 3 (the two-convolution stem's conv2): seven 64-column TMEM accumulators, c_in <= 64
+            k7 = c.k == 7 and c.pad == 3 and c.stride == 2 and c.cin <= 64
+            return ((c.k == 3 and c.pad == 1) or (c.k == 1 and c.pad == 0) or k7) and c.cin % 16 == 0 and c.cout % 8 == 0
         return c.cin % 8 == 0 and c.cout % 8 == 0
 
     def conv_fwd(self, c, src, src_stride, dst, dst_stride, l_in, dst_ptr_off=0, src_last_use=False):
@@ -636,8 +641,9 @@ class Plan(object):
         """The checks every ResNet plan shares, run before anything is recorded (the stem's shape is checked by _stem).
         Returns (stem pool type, c0, [(block, site prefix 'layer{li}.{bi}', l_in, l_out, cin, cout)])."""
         m = self.backbone
-        if m.double_conv_first:
-            raise NotImplementedError("resnet double_conv_first=True is not implemented on the B200 backend")
+        if m.double_conv_first and self.bn == "frozen":
+            raise NotImplementedError("resnet double_conv_first=True with frozen BatchNorm (train() with the BatchNorm "
+                                      "layers in eval()) is not implemented on the B200 backend")
         if self.mode == "features":
             raise NotImplementedError("'features' mode exists for DenseNet only (gradcam.py:45 needs .features)")
         blocks, L = [], 56
@@ -661,7 +667,10 @@ class Plan(object):
             # scale / shift / rstd of every layer from the running buffers, computed at the start of every forward
             self._coef = self._eval_coeffs(with_rstd=True)
         a = self.new((N, 56, c0))
-        stem_st = self._stem(m.conv1, m.bn1, pool, a.data_ptr(), c0)
+        if m.double_conv_first:
+            stem_st = self._double_stem_fwd(pool, c0, a.data_ptr())
+        else:
+            stem_st = self._stem(m.conv1, m.bn1, pool, a.data_ptr(), c0)
         recs = []
         for blk, site, L, lo, cin, cout in blocks:
             r = {"a_in": a}
@@ -746,7 +755,94 @@ class Plan(object):
                                 addend_stride=cout)
             d_out = d_in
             self.mark(blk.conv1.weight)
-        self._stem_bwd(m.conv1, m.bn1, pool, stem_st, d_out.data_ptr(), c0)
+        if m.double_conv_first:
+            self._double_stem_bwd(pool, c0, stem_st, d_out.data_ptr())
+        else:
+            self._stem_bwd(m.conv1, m.bn1, pool, stem_st, d_out.data_ptr(), c0)
+
+    # ------------------------------------------------------------------------------------------------------
+    # two-convolution stem (double_conv_first=True, resnet.py:145-150):
+    #   a0 = bn1(conv1_alt(x))  (N,224,C0)   stage 1, stem.cu (no ReLU)
+    #   r2 = relu(bn2(conv2(a0)))  (N,112,C0)   the generic convolution (k7, s2, p3) + BatchNorm, site "relu0"
+    #   a  = first_pool(r2)  (N,56,C0)   dards_pool3s2
+    # conv2 zero-pads a0, the BatchNorm output, so the two convolutions are not one 9-tap convolution of x.
+    # ------------------------------------------------------------------------------------------------------
+    def _double_stem_fwd(self, pool, c0, a_ptr):
+        m, N = self.backbone, self.N
+        self._check_double_stem(c0)
+        c2 = self.conv(m.conv2)
+        a0 = self.new((N, SEQ_LEN, c0))
+        y2 = self.new((N, 112, c0))
+        r2 = self.new((N, 112, c0))
+        mean1, rstd1 = self.stats(c0)
+        ws, ws_bytes = self._stem_alt_ws(c0, 0)
+        self.fwd.add("dards_stem_alt_fwd", self.x_buf.data_ptr(), m.conv1_alt.weight.data_ptr(), m.bn1.weight.data_ptr(),
+                     m.bn1.bias.data_ptr(), a0.data_ptr(), mean1.data_ptr(), rstd1.data_ptr(), self.G, self.group, c0, c0,
+                     BN_EPS, ws, ws_bytes, self.dt)
+        self._note_running(m.bn1, mean1, rstd1, self.group * SEQ_LEN, c0)
+        if self.cb_mode(c2, SEQ_LEN):
+            st2, _ = self.conv_bn_fwd(c2, m.bn2, a0.data_ptr(), c0, SEQ_LEN, y2, r2, True)
+        else:
+            self.conv_fwd(c2, a0.data_ptr(), c0, y2.data_ptr(), c0, SEQ_LEN)
+            st2 = self.gbn_fwd(m.bn2, y2.data_ptr(), c0, r2.data_ptr(), c0, self.group * 112, c0, True)
+        self.fwd.add("dards_pool3s2_fwd", r2.data_ptr(), a_ptr, N, 112, c0, c0, c0, pool, self.dt)
+        self.sites["relu0"] = r2
+        return dict(c2=c2, a0=a0, y2=y2, r2=r2, st1=(mean1, rstd1), st2=st2)
+
+    def _double_stem_bwd(self, pool, c0, r, d_a):
+        """d_a: gradient of the pooled stem output (N,56,C0)."""
+        m, N = self.backbone, self.N
+        dr2 = self.scratch("gB", (N, 112, c0))
+        self.bwd.add("dards_pool3s2_bwd", d_a, r["r2"].data_ptr(), dr2.data_ptr(), N, 112, c0, c0, c0, c0, pool, self.dt)
+        dy2 = self.scratch("gC", (N, 112, c0))
+        self.gbn_bwd(m.bn2, r["st2"], dr2.data_ptr(), c0, r["y2"].data_ptr(), c0, dy2.data_ptr(), c0, self.group * 112, c0, 2,
+                     mask=r["r2"].data_ptr(), mask_stride=c0)
+        self.conv_wgrad(r["c2"], r["a0"].data_ptr(), c0, dy2.data_ptr(), c0, SEQ_LEN)
+        da0 = self.scratch("gD", (N, SEQ_LEN, c0))
+        self.conv_dgrad(r["c2"], dy2.data_ptr(), c0, da0.data_ptr(), c0, SEQ_LEN)
+        mean1, rstd1 = r["st1"]
+        dwp = self.new((self.G, c0 * 3), torch.float32)
+        dgp = self.new((self.G, c0), torch.float32)
+        dbp = self.new((self.G, c0), torch.float32)
+        ws, ws_bytes = self._stem_alt_ws(c0, 1)
+        self.bwd.add("dards_stem_alt_bwd", da0.data_ptr(), self.x_buf.data_ptr(), m.conv1_alt.weight.data_ptr(),
+                     m.bn1.weight.data_ptr(), mean1.data_ptr(), rstd1.data_ptr(), dwp.data_ptr(), dgp.data_ptr(),
+                     dbp.data_ptr(), self.G, self.group, c0, c0, ws, ws_bytes, self.dt)
+        self._pending_red.append((dwp, self.G, c0 * 3, self.gptr(m.conv1_alt.weight)))
+        self._pending_red.append((dgp, self.G, c0, self.gptr(m.bn1.weight)))
+        self._pending_red.append((dbp, self.G, c0, self.gptr(m.bn1.bias)))
+        self._flush_reductions()
+
+    def _double_stem_eval(self, pool, c0, a_ptr):
+        """Eval plans: stage 1 with bn1's running-statistics affine map, then conv2 with bn2 + ReLU in its epilogue, then
+        the pool.  a0 and r2 get buffers of their own (a0 is four times the largest block activation)."""
+        m, N = self.backbone, self.N
+        self._check_double_stem(c0)
+        co = self._coef[id(m.bn1)]
+        a0 = self.new((N, SEQ_LEN, c0))
+        r2 = self.new((N, 112, c0))
+        self.act_bytes += (a0.numel() + r2.numel()) * a0.element_size()
+        self.eval_reads.add(id(m.conv1_alt.weight))
+        self.fwd.add("dards_stem_alt_eval_fwd", self.x_buf.data_ptr(), m.conv1_alt.weight.data_ptr(), co.scale, co.shift,
+                     a0.data_ptr(), N, c0, c0, self.dt)
+        self.conv_affine_fwd(self.conv(m.conv2), m.bn2, a0.data_ptr(), c0, SEQ_LEN, r2.data_ptr(), True, src_last_use=True)
+        self.fwd.add("dards_pool3s2_fwd", r2.data_ptr(), a_ptr, N, 112, c0, c0, c0, pool, self.dt)
+
+    def _check_double_stem(self, c0):
+        m = self.backbone
+        shapes = ((m.conv1_alt, 1, 3, 1, 1), (m.conv2, c0, 7, 2, 3))
+        for conv, cin, k, s, p in shapes:
+            if (conv.in_channels, conv.out_channels, conv.kernel_size[0], conv.stride[0], conv.padding[0]) != (cin, c0, k, s, p):
+                raise NotImplementedError("double_conv_first stem must be Conv1d(1, C0, 3, 1, 1) then Conv1d(C0, C0, 7, 2, 3)")
+        if c0 % 16:
+            raise NotImplementedError("double_conv_first stem: initial planes must be a multiple of 16 (got %d)" % c0)
+
+    def _stem_alt_ws(self, c0, backward):
+        nbytes = _lib.fn("dards_stem_alt_workspace_bytes")(self.G, self.group, c0, backward)
+        if not nbytes:
+            return None, 0
+        t = self.new(((nbytes + 3) // 4,), torch.float32)
+        return t.data_ptr(), t.numel() * 4
 
     # ------------------------------------------------------------------------------------------------------
     # ResNet in eval(): BatchNorm with the running statistics, a fixed per-channel affine map per layer
@@ -814,7 +910,10 @@ class Plan(object):
             return next(t for t in pool_bufs if all(t is not b for b in busy))
 
         a = pool_bufs[0]
-        self._stem(m.conv1, m.bn1, pool, a.data_ptr(), c0)
+        if m.double_conv_first:
+            self._double_stem_eval(pool, c0, a.data_ptr())
+        else:
+            self._stem(m.conv1, m.bn1, pool, a.data_ptr(), c0)
         for blk, _, L, lo, cin, cout in blocks:
             c1, c2 = self.conv(blk.conv1), self.conv(blk.conv2)
             a1 = free(a)

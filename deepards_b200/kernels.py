@@ -313,6 +313,66 @@ def stem_bwd(dout, x, w, gamma, beta, mean, rstd, group, pool):
     return dwp.sum(0).view(c0, 1, 7), dgp.sum(0), dbp.sum(0)
 
 
+def _stem_alt_workspace(n_groups, group, c0, backward, device):
+    nbytes = _lib.fn("dards_stem_alt_workspace_bytes")(n_groups, group, c0, backward)
+    return torch.empty(((nbytes + 3) // 4,), dtype=torch.float32, device=device) if nbytes else None
+
+
+def stem_alt_fwd(x, w, gamma, beta, group, dtype, eps=1e-5):
+    """Stage 1 of the two-convolution stem: x (N, 224) fp32, w (C0, 1, 3) -> a0 = bn1(conv1_alt(x)) (N, 224, C0) in `dtype`,
+    plus per-group mean / rstd."""
+    n, c0 = x.shape[0], w.shape[0]
+    g = n // group
+    out = torch.empty((n, 224, c0), dtype=dtype, device=x.device)
+    mean = torch.empty((g, c0), dtype=torch.float32, device=x.device)
+    rstd = torch.empty((g, c0), dtype=torch.float32, device=x.device)
+    ws = _stem_alt_workspace(g, group, c0, 0, x.device)
+    _lib.call("dards_stem_alt_fwd", x.data_ptr(), w.data_ptr(), gamma.data_ptr(), beta.data_ptr(), out.data_ptr(),
+              mean.data_ptr(), rstd.data_ptr(), g, group, c0, c0, eps, ws.data_ptr() if ws is not None else None,
+              ws.numel() * 4 if ws is not None else 0, _DT[dtype], _st(x))
+    return out, mean, rstd
+
+
+def stem_alt_eval_fwd(x, w, scale, shift, dtype):
+    n, c0 = x.shape[0], w.shape[0]
+    out = torch.empty((n, 224, c0), dtype=dtype, device=x.device)
+    _lib.call("dards_stem_alt_eval_fwd", x.data_ptr(), w.data_ptr(), scale.data_ptr(), shift.data_ptr(), out.data_ptr(), n,
+              c0, c0, _DT[dtype], _st(x))
+    return out
+
+
+def stem_alt_bwd(dout, x, w, gamma, mean, rstd, group):
+    """dout (N, 224, C0) -> dW (C0, 1, 3), dgamma, dbeta (summed over the groups)."""
+    n, c0 = x.shape[0], w.shape[0]
+    g = n // group
+    dev = x.device
+    dwp = torch.empty((g, c0 * 3), dtype=torch.float32, device=dev)
+    dgp = torch.empty((g, c0), dtype=torch.float32, device=dev)
+    dbp = torch.empty((g, c0), dtype=torch.float32, device=dev)
+    ws = _stem_alt_workspace(g, group, c0, 1, dev)
+    _lib.call("dards_stem_alt_bwd", dout.data_ptr(), x.data_ptr(), w.data_ptr(), gamma.data_ptr(), mean.data_ptr(),
+              rstd.data_ptr(), dwp.data_ptr(), dgp.data_ptr(), dbp.data_ptr(), g, group, c0, _rowstride(dout),
+              ws.data_ptr() if ws is not None else None, ws.numel() * 4 if ws is not None else 0, _dt(dout), _st(x))
+    return dwp.sum(0).view(c0, 1, 3), dgp.sum(0), dbp.sum(0)
+
+
+def pool3s2(x, pool):
+    """Max (pool 0) / Avg (pool 1) Pool1d(3, 2, 1): (N, L, C) -> (N, (L - 1) // 2 + 1, C)."""
+    n, l, c = x.shape
+    out = torch.empty((n, (l - 1) // 2 + 1, c), dtype=x.dtype, device=x.device)
+    _lib.call("dards_pool3s2_fwd", x.data_ptr(), out.data_ptr(), n, l, c, _rowstride(x), _rowstride(out), pool, _dt(x),
+              _st(x))
+    return out
+
+
+def pool3s2_bwd(dout, x, pool):
+    n, l, c = x.shape
+    din = torch.empty_like(x)
+    _lib.call("dards_pool3s2_bwd", dout.data_ptr(), x.data_ptr(), din.data_ptr(), n, l, c, _rowstride(dout), _rowstride(x),
+              _rowstride(din), pool, _dt(x), _st(x))
+    return din
+
+
 def avgpool2(x, backward=False):
     n, l, c = x.shape
     if not backward:

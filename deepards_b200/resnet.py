@@ -2,8 +2,12 @@
 
 Same factory names and keyword arguments (`resnet18(pretrained=False, initial_planes=64, first_pool_type='max',
 double_conv_first=False)`, resnet.py:83,166-174), same attributes (`n_out_filters`, `network_name`,
-`inplanes`, `expansion`) and the same `state_dict` keys -- including the stem's never-used `conv1_alt`,
-`conv2`, `bn2` (resnet.py:90-96) -- so checkpoints move between the two implementations unchanged.
+`inplanes`, `expansion`) and the same `state_dict` keys -- including the stem's `conv1_alt`,
+`conv2`, `bn2` (resnet.py:90-96), unused by the default stem -- so checkpoints move between the two implementations unchanged.
+
+`double_conv_first=True` selects the two-convolution stem (resnet.py:145-150): conv1_alt -> bn1 -> conv2 -> bn2 -> ReLU ->
+first pool, with `conv1` unused (its `.grad` stays None).  It runs in train() and eval(); train() with the BatchNorm layers
+in eval() (frozen BatchNorm) raises NotImplementedError for it.
 
 The `nn.Conv1d` / `nn.BatchNorm1d` children are parameter CONTAINERS only: `forward` does not call them, it
 runs the recorded kernel plan (engine.Plan) through autograd.  BatchNorm statistics are taken over the whole

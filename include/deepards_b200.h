@@ -286,7 +286,35 @@ int dards_stem_bwd(const void* dout, const float* x, const float* w, const float
                    float* dbeta_part, int n_groups, int group, int c0, int dout_stride, int pool, void* workspace,
                    long long workspace_bytes, int dtype, void* stream);
 
+/* ---- stage 1 of the two-convolution stem: Conv1d(1->C0,k3,s1,p1) + BN (ResNet double_conv_first) ------------- */
+/* resnet.py:145-147: x (N,224) fp32 -> a0 = bn1(conv1_alt(x)) (N,224,C0) in `dtype`, no ReLU, no pool; the batch statistics
+ * of every group go to save_mean / save_rstd [n_groups][C0].  The following Conv1d(C0,C0,k7,s2,p3) runs on
+ * dards_conv1d_fwd and zero-pads a0, and the first pool is dards_pool3s2_fwd.  Groups of more than 226 breaths run in
+ * chunks and need `workspace` of dards_stem_alt_workspace_bytes(...) bytes (0 otherwise; the pointer may then be NULL).
+ * C0 must be a multiple of 16. */
+long long dards_stem_alt_workspace_bytes(int n_groups, int group, int c0, int backward);
+int dards_stem_alt_fwd(const float* x, const float* w, const float* gamma, const float* beta, void* out,
+                       float* save_mean, float* save_rstd, int n_groups, int group, int c0, int out_stride, float eps,
+                       void* workspace, long long workspace_bytes, int dtype, void* stream);
+/* Eval mode: a0 = conv1_alt(x)*scale[c] + shift[c] (dards_bn_eval_coeffs_batched), every breath on its own, any n_breaths. */
+int dards_stem_alt_eval_fwd(const float* x, const float* w, const float* scale, const float* shift, void* out,
+                            int n_breaths, int c0, int out_stride, int dtype, void* stream);
+/* d a0 (N,224,C0) + x -> per-group partials dw_part [n_groups][C0][3], dgamma_part / dbeta_part [n_groups][C0] of
+ * conv1_alt and bn1, summed with dards_reduce_rows[_batched].  No gradient w.r.t. x. */
+int dards_stem_alt_bwd(const void* dout, const float* x, const float* w, const float* gamma, const float* save_mean,
+                       const float* save_rstd, float* dw_part, float* dgamma_part, float* dbeta_part, int n_groups,
+                       int group, int c0, int dout_stride, void* workspace, long long workspace_bytes, int dtype,
+                       void* stream);
+
 /* ---- pooling, dropout --------------------------------------------------------------- */
+/* nn.MaxPool1d / AvgPool1d(3, 2, padding 1) (resnet.py:101-104, 151-153): (N,L,C) -> (N,(L-1)/2+1,C).  pool: 0 max
+ * (-inf padding), 1 avg (padding counted, divisor 3).  The backward takes the forward's input `in` (max: the gradient goes
+ * to the first maximum of each window, recomputed from `in`; avg: `in` is not read and may be NULL) and writes every
+ * element of din (N,L,C).  C and the strides must be multiples of 4. */
+int dards_pool3s2_fwd(const void* in, void* out, int n_breaths, int l_in, int c, int in_stride, int out_stride, int pool,
+                      int dtype, void* stream);
+int dards_pool3s2_bwd(const void* dout, const void* in, void* din, int n_breaths, int l_in, int c, int dout_stride,
+                      int in_stride, int din_stride, int pool, int dtype, void* stream);
 /* nn.AvgPool1d(2,2) (densenet.py:77): (N,L,C) -> (N,L/2,C) and its backward. */
 int dards_avgpool2_fwd(const void* in, void* out, int n_breaths, int l_in, int c, int in_stride, int out_stride,
                        int dtype, void* stream);
