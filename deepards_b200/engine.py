@@ -11,7 +11,7 @@ parameter gradients are fp32.  Gradients land in one flat fp32 buffer (`Plan.gra
 `named_parameters()`), which is what the data-parallel all-reduce and the fused optimizer operate on.
 
 Reference semantics implemented here (file:line in /root/reference/deepards):
-  models/resnet.py:24-40, 141-163   BasicBlock / ResNet forward
+  models/resnet.py:24-40, 43-78, 141-163   BasicBlock / Bottleneck / ResNet forward
   models/densenet.py:18-43, 68-80, 179-193   dense layer / transition / DenseNet forward
   models/torch_cnn_linear_network.py:57-67, 104-113   per-breath and per-sequence linear heads
 """
@@ -78,8 +78,8 @@ class nvtx_range(object):
 
 def resnet_bn_layers(backbone):
     """(name, module) of the BatchNorm layers a ResNet's forward uses (resnet.py:141-163): the stem's bn1, its bn2 with
-    double_conv_first=True (the default stem builds bn2 and never calls it), and every block's bn1 / bn2 / downsample
-    BatchNorm."""
+    double_conv_first=True (the default stem builds bn2 and never calls it), and every block's bn1 / bn2 / bn3 (Bottleneck) /
+    downsample BatchNorm."""
     out = [("bn1", backbone.bn1)]
     if backbone.double_conv_first:
         out.append(("bn2", backbone.bn2))
@@ -87,6 +87,8 @@ def resnet_bn_layers(backbone):
         for bi, blk in enumerate(layer):
             pre = "layer%d.%d." % (li, bi)
             out += [(pre + "bn1", blk.bn1), (pre + "bn2", blk.bn2)]
+            if isinstance(getattr(blk, "bn3", None), torch.nn.BatchNorm1d):
+                out.append((pre + "bn3", blk.bn3))
             if blk.downsample is not None:
                 out.append((pre + "downsample.1", blk.downsample[1]))
     return out
@@ -635,11 +637,22 @@ class Plan(object):
         self.bwd.add("dards_avgpool_full_bwd", self.dfeat.data_ptr(), dact, self.N, l, f, dact_stride, self.dt)
 
     # ------------------------------------------------------------------------------------------------------
-    # ResNet (BasicBlock)
+    # ResNet (BasicBlock and Bottleneck)
     # ------------------------------------------------------------------------------------------------------
+    @staticmethod
+    def _block_stages(blk):
+        """The main branch of a block as (conv, bn) in order: conv1 / conv2 for BasicBlock (resnet.py:24-40), conv1 (1x1) /
+        conv2 (k3, the block's stride) / conv3 (1x1, x4) for Bottleneck (resnet.py:43-78).  Every stage but the last is
+        followed by a ReLU; the last one's BatchNorm is added to the identity or downsample branch before the ReLU."""
+        stages = [(blk.conv1, blk.bn1), (blk.conv2, blk.bn2)]
+        if getattr(blk, "conv3", None) is not None:
+            stages.append((blk.conv3, blk.bn3))
+        return stages
+
     def _resnet_blocks(self):
         """The checks every ResNet plan shares, run before anything is recorded (the stem's shape is checked by _stem).
-        Returns (stem pool type, c0, [(block, site prefix 'layer{li}.{bi}', l_in, l_out, cin, cout)])."""
+        Returns (stem pool type, c0, [(block, site prefix 'layer{li}.{bi}', l_in, l_out, cin, cout)]), cin / cout being the
+        block's input and output channels."""
         m = self.backbone
         if m.double_conv_first and self.bn == "frozen":
             raise NotImplementedError("resnet double_conv_first=True with frozen BatchNorm (train() with the BatchNorm "
@@ -649,10 +662,13 @@ class Plan(object):
         blocks, L = [], 56
         for li, layer in enumerate((m.layer1, m.layer2, m.layer3, m.layer4), 1):
             for bi, blk in enumerate(layer):
-                cin, cout, stride = blk.conv1.in_channels, blk.conv1.out_channels, blk.conv1.stride[0]
-                if blk.downsample is None and (cin != cout or stride != 1):
-                    raise RuntimeError("BasicBlock without downsample must keep the shape")
-                lo = (L + 2 - 3) // stride + 1
+                stages = self._block_stages(blk)
+                cin, cout = stages[0][0].in_channels, stages[-1][0].out_channels
+                lo = L
+                for conv, _ in stages:
+                    lo = (lo + 2 * conv.padding[0] - conv.kernel_size[0]) // conv.stride[0] + 1
+                if blk.downsample is None and (cin != cout or lo != L):
+                    raise RuntimeError("%s without downsample must keep the shape" % type(blk).__name__)
                 blocks.append((blk, "layer%d.%d" % (li, bi), L, lo, cin, cout))
                 L = lo
         if L != 7:
@@ -674,48 +690,59 @@ class Plan(object):
         recs = []
         for blk, site, L, lo, cin, cout in blocks:
             r = {"a_in": a}
-            c1, c2 = self.conv(blk.conv1), self.conv(blk.conv2)
-            y1 = self.new((N, lo, cout))
-            a1 = self.new((N, lo, cout))
-            if self.cb_mode(c1, L):
-                st1, _ = self.conv_bn_fwd(c1, blk.bn1, a.data_ptr(), cin, L, y1, a1, True)
-            else:
-                self.conv_fwd(c1, a.data_ptr(), cin, y1.data_ptr(), cout, L)
-                st1 = self.gbn_fwd(blk.bn1, y1.data_ptr(), cout, a1.data_ptr(), cout, self.group * lo, cout, True)
-            y2 = self.new((N, lo, cout))
+            # the main branch: every stage but the last -> conv + BatchNorm + ReLU (sites relu1, relu2)
+            convs = [self.conv(conv) for conv, _ in self._block_stages(blk)]
+            bns = [bn for _, bn in self._block_stages(blk)]
+            h, lh, ch = a, L, cin
+            stages = []
+            for i, (c, bn) in enumerate(zip(convs[:-1], bns[:-1])):
+                lc = (lh + 2 * c.pad - c.k) // c.stride + 1
+                y = self.new((N, lc, c.cout))
+                act = self.new((N, lc, c.cout))
+                if self.cb_mode(c, lh):
+                    st, _ = self.conv_bn_fwd(c, bn, h.data_ptr(), ch, lh, y, act, True, src_last_use=i > 0)
+                else:
+                    self.conv_fwd(c, h.data_ptr(), ch, y.data_ptr(), c.cout, lh, src_last_use=i > 0)
+                    st = self.gbn_fwd(bn, y.data_ptr(), c.cout, act.data_ptr(), c.cout, self.group * lc, c.cout, True)
+                stages.append(dict(c=c, bn=bn, src=h, cin=ch, l_in=lh, y=y, act=act, st=st))
+                self.sites[site + ".relu%d" % (i + 1)] = act
+                h, lh, ch = act, lc, c.cout
+            # the last stage: out = relu(bn(conv(h)) + identity or downsample branch)
+            cl, bnl = convs[-1], bns[-1]
+            yl = self.new((N, lo, cout))
             out = self.new((N, lo, cout))
-            m2 = self.cb_mode(c2, lo, blk.downsample is not None)
+            ml = self.cb_mode(cl, lh, blk.downsample is not None)
             if blk.downsample is not None:
                 cd = self.conv(blk.downsample[0])
                 yd = self.new((N, lo, cout))
-                if m2 and self.cb_mode(cd, L, True) == m2:
-                    st2, std = self.conv_bn_fwd(c2, blk.bn2, a1.data_ptr(), cout, lo, y2, out, True, src_last_use=True,
+                if ml and self.cb_mode(cd, L, True) == ml:
+                    stl, std = self.conv_bn_fwd(cl, bnl, h.data_ptr(), ch, lh, yl, out, True, src_last_use=True,
                                                 ds=(cd, blk.downsample[1], a.data_ptr(), cin, L, yd), merged_branch=True)
                 elif self.bn == "frozen":
-                    # out = relu(bn2(y2) + bn_d(y_d)): one pass over both branches
-                    self.conv_fwd(c2, a1.data_ptr(), cout, y2.data_ptr(), cout, lo, src_last_use=True)
+                    # out = relu(bn(y) + bn_d(y_d)): one pass over both branches
+                    self.conv_fwd(cl, h.data_ptr(), ch, yl.data_ptr(), cout, lh, src_last_use=True)
                     self.conv_fwd(cd, a.data_ptr(), cin, yd.data_ptr(), cout, L)
-                    st2 = self.bn_affine_apply(blk.bn2, y2.data_ptr(), cout, out.data_ptr(), cout, N * lo, cout, True,
+                    stl = self.bn_affine_apply(bnl, yl.data_ptr(), cout, out.data_ptr(), cout, N * lo, cout, True,
                                                second=(blk.downsample[1], yd.data_ptr(), cout))
                     std = self._coef[id(blk.downsample[1])]
                 else:
-                    self.conv_fwd(c2, a1.data_ptr(), cout, y2.data_ptr(), cout, lo, src_last_use=True)
+                    self.conv_fwd(cl, h.data_ptr(), ch, yl.data_ptr(), cout, lh, src_last_use=True)
                     self.conv_fwd(cd, a.data_ptr(), cin, yd.data_ptr(), cout, L)
                     res = self.scratch("ds_res", (N, lo, cout))
                     std = self.gbn_fwd(blk.downsample[1], yd.data_ptr(), cout, res.data_ptr(), cout, self.group * lo,
                                        cout, False)
-                    st2 = self.gbn_fwd(blk.bn2, y2.data_ptr(), cout, out.data_ptr(), cout, self.group * lo, cout, True,
+                    stl = self.gbn_fwd(bnl, yl.data_ptr(), cout, out.data_ptr(), cout, self.group * lo, cout, True,
                                        res=res.data_ptr(), res_stride=cout)
                 r.update(cd=cd, yd=yd, std=std)
-            elif m2:
-                st2, _ = self.conv_bn_fwd(c2, blk.bn2, a1.data_ptr(), cout, lo, y2, out, True, res=a, src_last_use=True)
+            elif ml:
+                stl, _ = self.conv_bn_fwd(cl, bnl, h.data_ptr(), ch, lh, yl, out, True, res=a, src_last_use=True)
             else:
-                self.conv_fwd(c2, a1.data_ptr(), cout, y2.data_ptr(), cout, lo, src_last_use=True)
-                st2 = self.gbn_fwd(blk.bn2, y2.data_ptr(), cout, out.data_ptr(), cout, self.group * lo, cout, True,
+                self.conv_fwd(cl, h.data_ptr(), ch, yl.data_ptr(), cout, lh, src_last_use=True)
+                stl = self.gbn_fwd(bnl, yl.data_ptr(), cout, out.data_ptr(), cout, self.group * lo, cout, True,
                                    res=a.data_ptr(), res_stride=cout)
-            r.update(c1=c1, c2=c2, y1=y1, a1=a1, st1=st1, y2=y2, st2=st2, out=out)
-            self.sites[site + ".relu1"] = a1
-            self.sites[site + ".relu2"] = out
+            stages.append(dict(c=cl, bn=bnl, src=h, cin=ch, l_in=lh, y=yl, act=out, st=stl))
+            r.update(stages=stages, out=out)
+            self.sites[site + ".relu%d" % len(stages)] = out
             recs.append(r)
             a = out
         L, f = blocks[-1][3], blocks[-1][5]
@@ -725,33 +752,41 @@ class Plan(object):
         d_out = self.scratch("gA", (N, L, f))
         self._head_bwd(d_out.data_ptr(), f, L, f)
         for (blk, _, l_in, lo, cin, cout), r in zip(reversed(blocks), reversed(recs)):
-            rows = self.group * lo
-            # out = relu(bn2(y2) + res):  g = d_out * (out > 0) written over d_out; dy2 = BN2 backward
-            dy2 = self.scratch("gB", (N, lo, cout))
-            self.gbn_bwd(blk.bn2, r["st2"], d_out.data_ptr(), cout, r["y2"].data_ptr(), cout, dy2.data_ptr(), cout, rows,
-                         cout, 2, mask=r["out"].data_ptr(), mask_stride=cout, dres=d_out.data_ptr(), dres_stride=cout)
-            # wgrad before dgrad: measured 1 % faster per step than the other order (the BatchNorm backward that follows
-            # finds dgrad's output still in L2)
-            self.conv_wgrad(r["c2"], r["a1"].data_ptr(), cout, dy2.data_ptr(), cout, lo)
-            da1 = self.scratch("gC", (N, lo, cout))
-            self.conv_dgrad(r["c2"], dy2.data_ptr(), cout, da1.data_ptr(), cout, lo)
-            # a1 = relu(bn1(y1)): dy1 in place over da1
-            self.gbn_bwd(blk.bn1, r["st1"], da1.data_ptr(), cout, r["y1"].data_ptr(), cout, da1.data_ptr(), cout, rows,
-                         cout, 1)
-            self.conv_wgrad(r["c1"], r["a_in"].data_ptr(), cin, da1.data_ptr(), cout, l_in)
+            stages = r["stages"]
+            last = stages[-1]
+            # out = relu(bn(y) + res):  g = d_out * (out > 0) written over d_out; dy = the last BatchNorm's backward
+            dy = self.scratch("gB", (N, lo, cout))
+            self.gbn_bwd(last["bn"], last["st"], d_out.data_ptr(), cout, last["y"].data_ptr(), cout, dy.data_ptr(), cout,
+                         self.group * lo, cout, 2, mask=r["out"].data_ptr(), mask_stride=cout, dres=d_out.data_ptr(),
+                         dres_stride=cout)
+            # back through the main branch to the first stage's output gradient
+            for k in range(len(stages) - 1, 0, -1):
+                s, prev = stages[k], stages[k - 1]
+                cp = prev["c"].cout
+                # wgrad before dgrad: measured 1 % faster per step than the other order (the BatchNorm backward that
+                # follows finds dgrad's output still in L2)
+                self.conv_wgrad(s["c"], s["src"].data_ptr(), s["cin"], dy.data_ptr(), s["c"].cout, s["l_in"])
+                da = self.scratch("gC" if k == len(stages) - 1 else "gD", (N, s["l_in"], cp))
+                self.conv_dgrad(s["c"], dy.data_ptr(), s["c"].cout, da.data_ptr(), cp, s["l_in"])
+                # prev's output = relu(bn(y)): its y gradient in place over da
+                self.gbn_bwd(prev["bn"], prev["st"], da.data_ptr(), cp, prev["y"].data_ptr(), cp, da.data_ptr(), cp,
+                             self.group * s["l_in"], cp, 1)
+                dy = da
+            c1, p1 = stages[0]["c"], stages[0]["c"].cout
+            self.conv_wgrad(c1, r["a_in"].data_ptr(), cin, dy.data_ptr(), p1, l_in)
             if blk.downsample is not None:
                 # residual branch: g -> BN(ds) backward in place -> conv1x1 backward
                 self.gbn_bwd(blk.downsample[1], r["std"], d_out.data_ptr(), cout, r["yd"].data_ptr(), cout,
-                             d_out.data_ptr(), cout, rows, cout, 0)
+                             d_out.data_ptr(), cout, self.group * lo, cout, 0)
                 self.conv_wgrad(r["cd"], r["a_in"].data_ptr(), cin, d_out.data_ptr(), cout, l_in)
                 d_in = self.scratch("gA", (N, l_in, cin))
-                # main branch first (writes every position), then the 1x1 stride-2 branch accumulates in place
-                self.conv_dgrad(r["c1"], da1.data_ptr(), cout, d_in.data_ptr(), cin, l_in)
+                # main branch first (writes every position), then the 1x1 downsample branch accumulates in place
+                self.conv_dgrad(c1, dy.data_ptr(), p1, d_in.data_ptr(), cin, l_in)
                 self.conv_dgrad(r["cd"], d_out.data_ptr(), cout, d_in.data_ptr(), cin, l_in, addend=d_in.data_ptr(),
                                 addend_stride=cin)
             else:
                 d_in = d_out  # g is the identity-branch gradient: accumulate conv1's dgrad onto it in place
-                self.conv_dgrad(r["c1"], da1.data_ptr(), cout, d_in.data_ptr(), cin, l_in, addend=d_out.data_ptr(),
+                self.conv_dgrad(c1, dy.data_ptr(), p1, d_in.data_ptr(), cin, l_in, addend=d_out.data_ptr(),
                                 addend_stride=cout)
             d_out = d_in
             self.mark(blk.conv1.weight)
@@ -897,7 +932,9 @@ class Plan(object):
         """Forward only: pack, coefficients, eval stem, then per block conv1 -> affine + ReLU and conv2 -> affine + residual +
         ReLU (the downsample branch -> affine into a scratch buffer first), avgpool, head.  No statistics, no running-statistics
         update, no gradient buffers.  Activations rotate through four buffers, each the size of the largest (N, L, C)
-        activation: block input (= identity residual), conv1 output, downsample output, block output."""
+        activation: block input (= identity residual), the main branch's inner activation, downsample output, block output.
+        A Bottleneck's two inner activations take turns in the same two buffers: conv2 reads a1 and writes a2, and nothing
+        reads a1 after that, so its buffer takes the downsample output."""
         m = self.backbone
         pool, c0, blocks = self._resnet_blocks()
         N = self.N
@@ -915,18 +952,23 @@ class Plan(object):
         else:
             self._stem(m.conv1, m.bn1, pool, a.data_ptr(), c0)
         for blk, _, L, lo, cin, cout in blocks:
-            c1, c2 = self.conv(blk.conv1), self.conv(blk.conv2)
-            a1 = free(a)
-            self.conv_affine_fwd(c1, blk.bn1, a.data_ptr(), cin, L, a1.data_ptr(), True)
+            stages = self._block_stages(blk)
+            convs = [self.conv(conv) for conv, _ in stages]
+            h, lh = a, L
+            for i, (c, (_, bn)) in enumerate(zip(convs[:-1], stages[:-1])):
+                # the main branch's inner stages: affine + ReLU; a Bottleneck's a1 is free again once a2 is written
+                nxt = free(a, h)
+                self.conv_affine_fwd(c, bn, h.data_ptr(), c.cin, lh, nxt.data_ptr(), True, src_last_use=i > 0)
+                h, lh = nxt, (lh + 2 * c.pad - c.k) // c.stride + 1
             if blk.downsample is not None:
                 cd = self.conv(blk.downsample[0])
-                res = free(a, a1)
+                res = free(a, h)
                 self.conv_affine_fwd(cd, blk.downsample[1], a.data_ptr(), cin, L, res.data_ptr(), False, src_last_use=True)
             else:
                 res = a
-            out = free(a, a1, res)
-            self.conv_affine_fwd(c2, blk.bn2, a1.data_ptr(), cout, lo, out.data_ptr(), True, res=res.data_ptr(),
-                                 src_last_use=True)
+            out = free(a, h, res)
+            self.conv_affine_fwd(convs[-1], stages[-1][1], h.data_ptr(), convs[-1].cin, lh, out.data_ptr(), True,
+                                 res=res.data_ptr(), src_last_use=True)
             a = out
         L, f = blocks[-1][3], blocks[-1][5]
         self._head_fwd(a.data_ptr(), f, L, f)

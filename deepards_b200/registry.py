@@ -7,13 +7,16 @@ head (:938-939, :963-964).  `install(module)` patches a loaded `train_ards_detec
 package with no other change (INTEGRATION.md shows the two-line edit a maintainer would make instead).
 """
 from .densenet import densenet18, densenet121
-from .resnet import resnet18, resnet34
+from .resnet import resnet18, resnet34, resnet50, resnet101, resnet152
 from .torch_cnn_linear_network import (CNNDoubleLinearNetwork, CNNLinearComprToRF, CNNLinearNetwork, CNNLinearToMean,
                                        CNNLSTMNetwork, CNNRegressor, CNNSingleBreathLinearNetwork, CNNTransformerNetwork)
 
 base_networks = {
     'resnet18': resnet18,
     'resnet34': resnet34,
+    'resnet50': resnet50,
+    'resnet101': resnet101,
+    'resnet152': resnet152,
     'densenet18': densenet18,
     'densenet121': densenet121,
 }

@@ -1,7 +1,8 @@
 """1-D ResNet backbones on the B200 backend -- drop-in for deepards/models/resnet.py.
 
-Same factory names and keyword arguments (`resnet18(pretrained=False, initial_planes=64, first_pool_type='max',
-double_conv_first=False)`, resnet.py:83,166-174), same attributes (`n_out_filters`, `network_name`,
+Same factory names (resnet18/34 with BasicBlock, resnet50/101/152 with Bottleneck, resnet.py:166-222) and keyword
+arguments (`resnet18(pretrained=False, initial_planes=64, first_pool_type='max', double_conv_first=False)`,
+resnet.py:83,166-174), same attributes (`n_out_filters`, `network_name`,
 `inplanes`, `expansion`) and the same `state_dict` keys -- including the stem's `conv1_alt`,
 `conv2`, `bn2` (resnet.py:90-96), unused by the default stem -- so checkpoints move between the two implementations unchanged.
 
@@ -52,11 +53,33 @@ class BasicBlock(_Picklable, nn.Module):
         raise RuntimeError("deepards_b200.BasicBlock holds parameters only; call the enclosing ResNet")
 
 
+class Bottleneck(_Picklable, nn.Module):
+    """conv1x1-bn-relu-conv3(stride)-bn-relu-conv1x1(x4)-bn (+ downsampled identity) -relu; parameter container
+    (resnet.py:43-78, the Bottleneck convolutions at :48-53, torchvision's layout): conv1 is 1x1 inplanes -> planes,
+    conv2 is k3 / stride / padding 1 planes -> planes, conv3 is 1x1 planes -> 4 * planes; no bias anywhere."""
+    expansion = 4
+
+    def __init__(self, inplanes, planes, stride=1, downsample=None):
+        super(Bottleneck, self).__init__()
+        self.conv1 = nn.Conv1d(inplanes, planes, kernel_size=1, bias=False)
+        self.bn1 = nn.BatchNorm1d(planes)
+        self.conv2 = _conv3(planes, planes, stride)
+        self.bn2 = nn.BatchNorm1d(planes)
+        self.conv3 = nn.Conv1d(planes, planes * self.expansion, kernel_size=1, bias=False)
+        self.bn3 = nn.BatchNorm1d(planes * self.expansion)
+        self.relu = nn.ReLU(inplace=True)
+        self.downsample = downsample
+        self.stride = stride
+
+    def forward(self, x):
+        raise RuntimeError("deepards_b200.Bottleneck holds parameters only; call the enclosing ResNet")
+
+
 class ResNet(_Picklable, nn.Module):
     def __init__(self, block, layers, initial_planes=64, first_pool_type='max', double_conv_first=False):
         super(ResNet, self).__init__()
-        if block is not BasicBlock:
-            raise NotImplementedError("only BasicBlock ResNets (resnet18/34) run on the B200 backend")
+        if block not in (BasicBlock, Bottleneck):
+            raise NotImplementedError("only BasicBlock and Bottleneck ResNets run on the B200 backend")
         if first_pool_type not in ('max', 'avg'):
             raise ValueError("first_pool_type must be 'max' or 'avg'")
         self.inplanes = initial_planes
@@ -84,7 +107,10 @@ class ResNet(_Picklable, nn.Module):
             elif isinstance(m, nn.BatchNorm1d):
                 m.weight.data.fill_(1)
                 m.bias.data.zero_()
-        self.n_out_filters = self.inplanes * block.expansion
+        # the features the backbone returns: the last stage's output channels, 8 * initial_planes * expansion.  The
+        # reference computes `self.inplanes * block.expansion` here, which is the same for BasicBlock (expansion 1) but
+        # 4x too large for Bottleneck, where self.inplanes already includes the expansion.
+        self.n_out_filters = self.inplanes
         self.network_name = 'resnet'
         self.precision = None  # None -> DEEPARDS_B200_PRECISION or 'bf16' (tcgen05 path); 'fp32' = the 1e-4 parity path
 
@@ -117,4 +143,25 @@ def resnet34(pretrained=False, **kwargs):
     """1-D ResNet-34 (resnet.py:178-186)."""
     model = ResNet(BasicBlock, [3, 4, 6, 3], **kwargs)
     model.network_name = 'resnet34'
+    return model
+
+
+def resnet50(pretrained=False, **kwargs):
+    """1-D ResNet-50 (resnet.py:188-198): Bottleneck, [3, 4, 6, 3]."""
+    model = ResNet(Bottleneck, [3, 4, 6, 3], **kwargs)
+    model.network_name = 'resnet50'
+    return model
+
+
+def resnet101(pretrained=False, **kwargs):
+    """1-D ResNet-101 (resnet.py:200-210): Bottleneck, [3, 4, 23, 3]."""
+    model = ResNet(Bottleneck, [3, 4, 23, 3], **kwargs)
+    model.network_name = 'resnet101'
+    return model
+
+
+def resnet152(pretrained=False, **kwargs):
+    """1-D ResNet-152 (resnet.py:212-222): Bottleneck, [3, 8, 36, 3]."""
+    model = ResNet(Bottleneck, [3, 8, 36, 3], **kwargs)
+    model.network_name = 'resnet152'
     return model
