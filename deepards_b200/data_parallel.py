@@ -13,6 +13,14 @@ notes is effectively unusable (:198-203).  Semantics kept from that path (SURVEY
   * parameters that never receive a gradient (ResNet's conv1_alt/conv2/bn2; frozen parameters) are left out of
     the update, exactly like torch.optim skipping `p.grad is None`.
 
+Every head of the package trains here.  CNNLinearNetwork and CNNSingleBreathLinearNetwork with the default
+BCEWithLogits loss run the fused plan (linear head and loss in the recorded kernels).  Every other head, and those two
+with a caller-supplied `criterion`, run the generic step: the backbone plan forward, the head's own torch arithmetic
+(`net._head`, the code its forward() runs) and the criterion under autograd, their gradients written into the flat
+gradient buffer, then the backbone plan backward and the same reduction and update.  CNNRegressor takes a flat batch of
+breaths (N, 1, 224); its BatchNorm group is the rank's whole flat batch, i.e. each rank normalises its own shard, as
+each nn.DataParallel replica normalises its own chunk.
+
 The gradient buffer is reduced in buckets, last layers first, on a communication stream that waits on events
 recorded inside the backward pass, so the reduction of layer4's 11.5 MB overlaps the backward of layers 1-3.
 """
@@ -118,11 +126,34 @@ class BucketedAllReduce(object):
         self.handles = []
 
 
+class _HeadCall(torch.nn.Module):
+    """forward(feat) = net._head(feat): lets torch.func.functional_call run the head on substitute parameters."""
+
+    def __init__(self, net):
+        super(_HeadCall, self).__init__()
+        self.net = net
+
+    def forward(self, feat):
+        return self.net._head(feat)
+
+
 class DataParallelTrainer(object):
+    """criterion: any callable (outputs, target) -> scalar tensor, given what the module's forward returns ((B, 2),
+    (B, S, 2), the LSTM's per-step outputs without its state, the regressor's (N, n_final_features)).  None means
+    nn.BCEWithLogitsLoss(), the reference's default; on CNNLinearNetwork / CNNSingleBreathLinearNetwork it keeps the
+    fused plan with the loss kernel."""
+
     def __init__(self, net, lr=1e-3, optimizer="sgd", momentum=0.9, weight_decay=1e-4, clip_val=0.01, group=None,
-                 bucket_mb=1.0, use_graph=False):
+                 bucket_mb=1.0, use_graph=False, criterion=None):
         if optimizer not in ("sgd", "adam"):
             raise ValueError("optimizer must be 'sgd' or 'adam'")
+        from .torch_cnn_linear_network import CNNLinearNetwork, CNNRegressor, CNNSingleBreathLinearNetwork, _HeadBase
+        if not isinstance(net, _HeadBase) or not hasattr(net, "_head"):
+            raise TypeError("DataParallelTrainer trains the heads of deepards_b200 (registry.network_heads), not %s"
+                            % type(net).__name__)
+        self.fused = criterion is None and isinstance(net, (CNNLinearNetwork, CNNSingleBreathLinearNetwork))
+        self.criterion = torch.nn.BCEWithLogitsLoss() if criterion is None else criterion
+        self.flat_batch = isinstance(net, CNNRegressor)     # (N, 1, 224) breaths, one BatchNorm group per rank
         self.use_graph = use_graph
         # world > 1: "segments" (default) replays one graph per backward segment with the NCCL calls issued from the host
         # in between.  "whole" (opt-in, experimental) captures the entire step INCLUDING the bucketed NCCL all-reduces
@@ -152,6 +183,10 @@ class DataParallelTrainer(object):
             if 0 < reserve < sms:
                 _lib.call("dards_set_sm_limit", sms - reserve)
         self.loss_buf = torch.zeros(1, dtype=torch.float32, device=self.device)
+        backbone = set(id(p) for p in net.breath_block.parameters())
+        self.head_named = [("net." + n, p) for n, p, _ in self.layout if id(p) not in backbone and p.requires_grad]
+        self.head_params = [p for _, p in self.head_named]
+        self._head_call = _HeadCall(net)
 
     # ---- flat parameter / optimizer-state buffers (same slot table as Plan.grad_flat) ----------------------
     def _flatten(self):
@@ -171,20 +206,15 @@ class DataParallelTrainer(object):
             dist.broadcast(self.param_flat, src=0, group=self.group)  # DataParallel broadcasts device-0 weights
 
     def plan_for(self, x):
+        if not self.fused:
+            return self._generic_plan(x)
         net = self.net
         bb = net.breath_block
         from .torch_cnn_linear_network import CNNSingleBreathLinearNetwork, _drop_key
         mode = "per_breath" if isinstance(net, CNNSingleBreathLinearNetwork) else "cnn_linear"
         n = x.numel() // engine.SEQ_LEN
         training = bb.training
-        # the same rule as the autograd path (autograd.run_plan, engine.bn_mode): batch statistics, or frozen running
-        # statistics when every BatchNorm layer of a ResNet in train() is in eval(); mixed states raise
-        bn = engine.bn_mode(bb)
-        if bn == "eval":
-            # a ResNet in eval() is inference only (its backward raises on the autograd path as well)
-            raise NotImplementedError("deepards_b200: DataParallelTrainer trains a ResNet in train() mode only (BatchNorm "
-                                      "layers all in train(), or all in eval() to fine-tune with frozen statistics); "
-                                      "this one is in eval()")
+        bn = self._bn_mode(bb)
         from .autograd import module_precision
         plan = engine.get_plan(net, bb, net.linear_final, n, x.shape[1], module_precision(net), mode,
                                dropout=_drop_key(bb) if training else (), update_running=training, bn=bn)
@@ -195,8 +225,92 @@ class DataParallelTrainer(object):
             plan._dp_buckets = make_buckets(self.total, [off for off, _ in plan.bwd_marks], self.bucket_elems)
         return plan
 
+    @staticmethod
+    def _bn_mode(bb):
+        # the same rule as the autograd path (autograd.run_plan, engine.bn_mode): batch statistics, or frozen running
+        # statistics when every BatchNorm layer of a ResNet in train() is in eval(); mixed states raise
+        bn = engine.bn_mode(bb)
+        if bn == "eval":
+            # a ResNet in eval() is inference only (its backward raises on the autograd path as well)
+            raise NotImplementedError("deepards_b200: DataParallelTrainer trains a ResNet in train() mode only (BatchNorm "
+                                      "layers all in train(), or all in eval() to fine-tune with frozen statistics); "
+                                      "this one is in eval()")
+        return bn
+
+    def _generic_plan(self, x):
+        """The backbone plan of the generic step.  Its owner is the head module, so its grad_flat has the slot table of
+        param_layout(net), the head's parameters included.  BatchNorm group: the sequence (x.shape[1]), or for
+        CNNRegressor the rank's whole flat batch."""
+        net = self.net
+        bb = net.breath_block
+        from .torch_cnn_linear_network import CNNDoubleLinearNetwork, CNNLinearNetwork, _drop_key
+        from .autograd import module_precision
+        if x.shape[-1] != engine.SEQ_LEN:
+            raise Exception('input breaths must have sequence length of 224')
+        n = x.numel() // engine.SEQ_LEN
+        group = n if self.flat_batch else x.shape[1]
+        want = {CNNLinearNetwork: group * bb.n_out_filters, CNNDoubleLinearNetwork: 2 * group}.get(type(net))
+        if want is not None and net.linear_final.in_features != want:
+            raise NotImplementedError("deepards_b200: metadata_features > 0 is not implemented (linear_final expects %d "
+                                      "features, the head provides %d)" % (net.linear_final.in_features, want))
+        training = bb.training
+        bn = self._bn_mode(bb)
+        plan = engine.get_plan(net, bb, None, n, group, module_precision(net), "backbone",
+                               dropout=_drop_key(bb) if training else (), update_running=training, bn=bn)
+        if getattr(plan, "_dp_buckets", None) is None:
+            # the head's slots come last in named_parameters() order: they are in the first (suffix) bucket, which is
+            # complete before the backbone backward starts
+            plan._dp_buckets = make_buckets(self.total, [off for off, _ in plan.bwd_marks], self.bucket_elems)
+        # _dp_ranges: set by the first _head_step, which sees which head parameters get a gradient
+        return plan
+
+    def _static_target(self, plan, target):
+        """The generic step's target, copied into a per-plan device buffer (captured CUDA graphs read it there).  A
+        target of another shape or dtype gets a new buffer and drops the graphs that read the old one."""
+        t = plan.__dict__.get("_dp_target")
+        if t is None or t.shape != target.shape or t.dtype != target.dtype:
+            plan.__dict__.pop("_dp_graph", None)
+            plan.__dict__.pop("_dp_seg", None)
+            t = plan._dp_target = torch.empty(target.shape, dtype=target.dtype, device=self.device)
+        t.copy_(target, non_blocking=True)
+        return t
+
+    def _head_step(self, plan, target):
+        """Generic step, between the backbone forward and backward: the head's torch arithmetic on the pooled features,
+        the criterion, and their backward.  The feature gradient goes to plan.dfeat, each head parameter's gradient to
+        its slot of plan.grad_flat; the loss is back-propagated with the weight gs = world * B_local / global_batch, as
+        dards_bce_with_logits scales dlogits on the fused path."""
+        feat = plan.feat.detach()          # (N, F)
+        if not self.flat_batch:
+            feat = feat.view(plan.G, plan.group, -1)
+        feat.requires_grad_(True)
+        # fresh leaves over the parameters' storage every step: a head that keeps part of its last autograd graph alive
+        # (the transformer's attention map) would otherwise hand a parameter's AccumulateGrad node, created on the stream
+        # of an eager step, to the CUDA-graph capture of a later one, and the capture fails
+        leaves = dict((n, p.detach().requires_grad_(True)) for n, p in self.head_named)
+        params = list(leaves.values())
+        with torch.enable_grad():
+            out = torch.func.functional_call(self._head_call, leaves, (feat,), strict=False, tie_weights=False)
+            if isinstance(out, tuple):      # CNNLSTMNetwork: (per-step outputs, (hx, cx))
+                out = out[0]
+            loss = self.criterion(out, target)
+            if loss.numel() != 1:
+                raise ValueError("criterion must return a scalar loss, got shape %s" % (tuple(loss.shape),))
+            gs = plan.__dict__.get("_dp_grad_scale", 1.0)
+            grads = torch.autograd.grad(loss, [feat] + params, grad_outputs=torch.full_like(loss, gs), allow_unused=True)
+        self.loss_buf.copy_(loss.detach().reshape(1))
+        plan.dfeat.copy_(grads[0].reshape(plan.dfeat.shape))
+        for (_, p), g in zip(self.head_named, grads[1:]):
+            if g is not None:
+                plan.grad_view(p).copy_(g)
+        if plan.__dict__.get("_dp_ranges") is None:
+            live = set(i for i in plan.grad_written if any(id(p) == i and p.requires_grad for _, p, _ in self.layout))
+            live.update(id(p) for (_, p), g in zip(self.head_named, grads[1:]) if g is not None)
+            plan._dp_ranges = live_ranges(self.layout, live)
+
     def train_step(self, x, target, global_batch=None):
-        """x: this rank's (B_local, 20, 1, 224) on the device, target (B_local, 2).  Returns the device tensor
+        """x: this rank's (B_local, 20, 1, 224) on the device (CNNRegressor: (N_local, 1, 224) breaths), target what the
+        criterion takes ((B_local, 2) for the default loss of the sequence-level heads).  Returns the device tensor
         holding the local mean loss (no host synchronisation).
         global_batch: total number of sequences over all ranks.  The reference's DataParallel computes ONE mean loss over
         the gathered outputs (train_ards_detector.py:153-163); with equal shards that is the mean of the ranks' local means
@@ -236,14 +350,17 @@ class DataParallelTrainer(object):
             plan.load_input(x)
         else:
             plan.load_raw(x, *scaling)
-        t_static = plan.__dict__.get("_dp_target")
-        if t_static is None:
-            t_static = plan._dp_target = torch.empty((plan.logits.numel(),), dtype=torch.float32, device=self.device)
-        t_static.copy_(target.reshape(-1), non_blocking=True)
+        if self.fused:
+            t_static = plan.__dict__.get("_dp_target")
+            if t_static is None:
+                t_static = plan._dp_target = torch.empty((plan.logits.numel(),), dtype=torch.float32, device=self.device)
+            t_static.copy_(target.reshape(-1), non_blocking=True)
+        else:
+            t_static = self._static_target(plan, target)
         if self.use_graph and self.world == 1 and self.optimizer == "sgd":
             return self._graphed_step(plan, t_static)
         if self.use_graph and self.world > 1 and self.optimizer == "sgd":
-            if self.dp_graph == "whole":
+            if self.dp_graph == "whole" and self.fused:
                 try:
                     return self._graphed_step(plan, t_static)
                 except RuntimeError as e:       # NCCL under stream capture refused: replay per segment instead
@@ -259,8 +376,11 @@ class DataParallelTrainer(object):
     def _step_body(self, plan, t_static):
         st = plan._stream()
         plan.run_forward()
-        _lib.call("dards_bce_with_logits", plan.logits.data_ptr(), t_static.data_ptr(), self.loss_buf.data_ptr(),
-                  plan.dlogits.data_ptr(), plan.logits.numel(), plan.__dict__.get("_dp_grad_scale", 1.0), st)
+        if self.fused:
+            _lib.call("dards_bce_with_logits", plan.logits.data_ptr(), t_static.data_ptr(), self.loss_buf.data_ptr(),
+                      plan.dlogits.data_ptr(), plan.logits.numel(), plan.__dict__.get("_dp_grad_scale", 1.0), st)
+        else:
+            self._head_step(plan, t_static)
         if self.world > 1:
             self.step_count += 1
             self._backward_overlapped(plan)   # all-reduce + optimizer per bucket, on the communication stream
@@ -357,8 +477,11 @@ class DataParallelTrainer(object):
             if plan.dropout:
                 plan.seed_dev[0:1].add_(1)
             plan.fwd.run(st)
-            _lib.call("dards_bce_with_logits", plan.logits.data_ptr(), t_static.data_ptr(), self.loss_buf.data_ptr(),
-                      plan.dlogits.data_ptr(), plan.logits.numel(), plan.__dict__.get("_dp_grad_scale", 1.0), st)
+            if self.fused:
+                _lib.call("dards_bce_with_logits", plan.logits.data_ptr(), t_static.data_ptr(), self.loss_buf.data_ptr(),
+                          plan.dlogits.data_ptr(), plan.logits.numel(), plan.__dict__.get("_dp_grad_scale", 1.0), st)
+            else:
+                self._head_step(plan, t_static)
 
         out["fwd"] = capture(fwd)
         # backward segments: cut after every call index that carries a mark

@@ -61,6 +61,11 @@ class CNNLinearNetwork(_HeadBase):
         return _ag.run_plan(self, self.breath_block, self.linear_final, x, x.shape[1], "cnn_linear",
                             _drop_key(self.breath_block))
 
+    def _head(self, feat):
+        """(B, S, F) features -> (B, 2) logits in torch: what the plan's fused linear computes.  DataParallelTrainer uses
+        it with a caller-supplied criterion; forward() keeps the fused head."""
+        return self.linear_final(feat.reshape(feat.shape[0], -1))
+
 
 class CNNSingleBreathLinearNetwork(_HeadBase):
     """One prediction per breath: Linear(F, 2) on every breath's pooled features -> (B, breaths, 2)."""
@@ -76,9 +81,14 @@ class CNNSingleBreathLinearNetwork(_HeadBase):
         return _ag.run_plan(self, self.breath_block, self.linear_final, x, x.shape[1], "per_breath",
                             _drop_key(self.breath_block))
 
+    def _head(self, feat):
+        """(B, S, F) features -> (B, S, 2) logits in torch (see CNNLinearNetwork._head)."""
+        return self.linear_final(feat)
+
 
 # ---- sibling heads on the same backbone (SURVEY.md 8f-4): the backbone runs as one batched plan, the few-kB head
-# ---- arithmetic behind it stays in torch ------------------------------------------------------------------------
+# ---- arithmetic behind it stays in torch.  `_head(feat)` is that arithmetic: forward() and DataParallelTrainer both
+# ---- call it on the plan's pooled features ----------------------------------------------------------------------
 class CNNLinearToMean(_HeadBase):
     """Linear(F, 2) on the mean of the sequence's breath features (torch_cnn_linear_network.py:7-25)."""
 
@@ -89,7 +99,10 @@ class CNNLinearToMean(_HeadBase):
         self.linear_final = nn.Linear(self.breath_block.n_out_filters, 2)
 
     def forward(self, x, metadata=None):
-        return self.linear_final(torch.mean(self._sequence_features(x), dim=1))
+        return self._head(self._sequence_features(x))
+
+    def _head(self, feat):
+        return self.linear_final(torch.mean(feat, dim=1))
 
 
 class CNNLinearComprToRF(_HeadBase):
@@ -102,7 +115,10 @@ class CNNLinearComprToRF(_HeadBase):
         self.linear_final = nn.Linear(self.breath_block.n_out_filters, 2)
 
     def forward(self, x, metadata=None):
-        return self.linear_final(torch.median(self._sequence_features(x), dim=1)[0])
+        return self._head(self._sequence_features(x))
+
+    def _head(self, feat):
+        return self.linear_final(torch.median(feat, dim=1)[0])
 
 
 class CNNDoubleLinearNetwork(_HeadBase):
@@ -116,8 +132,10 @@ class CNNDoubleLinearNetwork(_HeadBase):
         self.linear_final = nn.Linear(2 * sequence_size + metadata_features, 2)
 
     def forward(self, x, metadata=None):
-        feat = self._sequence_features(x)
-        return self.linear_final(self.linear_intermediate(feat).reshape(x.shape[0], -1))
+        return self._head(self._sequence_features(x))
+
+    def _head(self, feat):
+        return self.linear_final(self.linear_intermediate(feat).reshape(feat.shape[0], -1))
 
 
 class CNNRegressor(_HeadBase):
@@ -134,7 +152,10 @@ class CNNRegressor(_HeadBase):
         # input should be in shape: (batches, chans, 224)
         if x.shape[-1] != 224:
             raise Exception('input breaths must have sequence length of 224')
-        return self.linear_final(self.breath_block(x).squeeze())
+        return self._head(self.breath_block(x))
+
+    def _head(self, feat):
+        return self.linear_final(feat.squeeze())
 
 
 class CNNLSTMNetwork(_HeadBase):
@@ -157,7 +178,9 @@ class CNNLSTMNetwork(_HeadBase):
     def forward(self, x, metadata=None, hx_cx=None):
         if metadata is not None and not torch.any(torch.isnan(metadata)):
             raise NotImplementedError("deepards_b200: breath metadata is not implemented on this backend")
-        feat = self._sequence_features(x)
+        return self._head(self._sequence_features(x), hx_cx)
+
+    def _head(self, feat, hx_cx=None):
         # the fp32 path promises the reference's fp32 numbers: keep cuDNN's LSTM GEMMs out of TF32 (its default)
         with torch.backends.cudnn.flags(allow_tf32=_ag.module_precision(self) == "bf16"):
             out, (hx, cx) = self.lstm(feat, hx_cx)
@@ -236,7 +259,9 @@ class CNNTransformerNetwork(_HeadBase):
     def forward(self, x, metadata=None):
         if metadata is not None and not torch.any(torch.isnan(metadata)):
             raise NotImplementedError("deepards_b200: breath metadata is not implemented on this backend")
-        feat = self._sequence_features(x)
+        return self._head(self._sequence_features(x))
+
+    def _head(self, feat):
         with _no_tf32(self):
             return self.linear_final(self.transformer(feat))
 
