@@ -117,6 +117,9 @@ _SIGNATURES = {
     "dards_stem_alt_fwd": [P, P, P, P, P, P, P, I, I, I, I, F, P, LL, I, P],
     "dards_stem_alt_eval_fwd": [P, P, P, P, P, I, I, I, I, P],
     "dards_stem_alt_bwd": [P, P, P, P, P, P, P, P, P, I, I, I, I, P, LL, I, P],
+    "dards_stem_dgrad": [P, P, P, P, P, P, P, P, P, P, I, I, I, I, I, I, P],
+    "dards_stem_frozen_dgrad": [P, P, P, P, P, P, I, I, I, I, I, P],
+    "dards_stem_alt_dgrad": [P, P, P, P, P, P, P, P, P, I, I, I, I, I, P],
     "dards_pool3s2_fwd": [P, P, I, I, I, I, I, I, I, P],
     "dards_pool3s2_bwd": [P, P, P, I, I, I, I, I, I, I, I, P],
     "dards_avgpool2_fwd": [P, P, I, I, I, I, I, I, P],

@@ -81,6 +81,12 @@ int launch_stem_fwd(const float*, const float*, const float*, const float*, void
 int launch_stem_bwd(const void*, const float*, const float*, const float*, const float*, const float*, const float*,
                     float*, float*, float*, int, int, int, int, int, void*, long long, int, cudaStream_t);
 long long stem_workspace_bytes(int n_groups, int group, int c0, int backward);
+int launch_stem_dgrad(const void*, const float*, const float*, const float*, const float*, const float*, const float*,
+                      const float*, const float*, float*, int, int, int, int, int, int, cudaStream_t);
+int launch_stem_frozen_dgrad(const void*, const float*, const float*, const float*, const float*, float*, int, int, int, int,
+                             int, cudaStream_t);
+int launch_stem_alt_dgrad(const void*, const float*, const float*, const float*, const float*, const float*, const float*,
+                          const float*, float*, int, int, int, int, int, cudaStream_t);
 int launch_avgpool2(int, const void*, void*, int, int, int, int, int, int, cudaStream_t);
 long long stem_alt_workspace_bytes(int n_groups, int group, int c0, int backward);
 int launch_stem_alt_fwd(const float*, const float*, const float*, const float*, void*, float*, float*, int, int, int, int,
@@ -451,6 +457,38 @@ int dards_stem_bwd(const void* dout, const float* x, const float* w, const float
   DARDS_CHECK_ARG(pool == 0 || pool == 1, "stem_bwd: pool must be 0 (max) or 1 (avg)");
   return launch_stem_bwd(dout, x, w, gamma, beta, save_mean, save_rstd, dw_part, dgamma_part, dbeta_part, n_groups, group,
                          c0, dout_stride, pool, workspace, workspace_bytes, dtype, S(stream));
+}
+
+int dards_stem_dgrad(const void* dout, const float* x, const float* w, const float* gamma, const float* beta,
+                     const float* save_mean, const float* save_rstd, const float* dgamma_part, const float* dbeta_part,
+                     float* dx, int n_groups, int group, int c0, int dout_stride, int pool, int dtype, void* stream) {
+  DARDS_CHECK_ARG(dout && x && w && gamma && beta && save_mean && save_rstd && dgamma_part && dbeta_part && dx,
+                  "stem_dgrad: null pointer");
+  DARDS_CHECK_ARG(n_groups >= 0, "stem_dgrad: negative number of groups");
+  DARDS_CHECK_ARG(pool == 0 || pool == 1, "stem_dgrad: pool must be 0 (max) or 1 (avg)");
+  DARDS_CHECK_ARG(dout_stride >= c0, "stem_dgrad: row stride smaller than channel count");
+  return launch_stem_dgrad(dout, x, w, gamma, beta, save_mean, save_rstd, dgamma_part, dbeta_part, dx, n_groups, group, c0,
+                           dout_stride, pool, dtype, S(stream));
+}
+
+int dards_stem_frozen_dgrad(const void* dout, const float* x, const float* w, const float* scale, const float* shift,
+                            float* dx, int n_breaths, int c0, int dout_stride, int pool, int dtype, void* stream) {
+  DARDS_CHECK_ARG(dout && x && w && scale && shift && dx, "stem_frozen_dgrad: null pointer");
+  DARDS_CHECK_ARG(n_breaths >= 0, "stem_frozen_dgrad: negative number of breaths");
+  DARDS_CHECK_ARG(pool == 0 || pool == 1, "stem_frozen_dgrad: pool must be 0 (max) or 1 (avg)");
+  DARDS_CHECK_ARG(dout_stride >= c0, "stem_frozen_dgrad: row stride smaller than channel count");
+  return launch_stem_frozen_dgrad(dout, x, w, scale, shift, dx, n_breaths, c0, dout_stride, pool, dtype, S(stream));
+}
+
+int dards_stem_alt_dgrad(const void* dout, const float* x, const float* w, const float* gamma, const float* save_mean,
+                         const float* save_rstd, const float* dgamma_part, const float* dbeta_part, float* dx, int n_groups,
+                         int group, int c0, int dout_stride, int dtype, void* stream) {
+  DARDS_CHECK_ARG(dout && x && w && gamma && save_mean && save_rstd && dgamma_part && dbeta_part && dx,
+                  "stem_alt_dgrad: null pointer");
+  DARDS_CHECK_ARG(n_groups >= 0, "stem_alt_dgrad: negative number of groups");
+  DARDS_CHECK_ARG(dout_stride >= c0, "stem_alt_dgrad: row stride smaller than channel count");
+  return launch_stem_alt_dgrad(dout, x, w, gamma, save_mean, save_rstd, dgamma_part, dbeta_part, dx, n_groups, group, c0,
+                               dout_stride, dtype, S(stream));
 }
 
 long long dards_stem_alt_workspace_bytes(int n_groups, int group, int c0, int backward) {

@@ -266,6 +266,66 @@ __device__ __forceinline__ float stem_shifted_mean(const float (&w)[STEM_K], flo
   return fmaf(-shift, wsum, mean);
 }
 
+// The backward's recompute sweep over one RUN of 14 pool outputs lp0 .. lp0+13 of one breath and one channel: the three
+// conv outputs of every pool window (conv positions 2lp-1, 2lp, 2lp+1), the ReLU, and the gradient each of them receives
+// from d(pool out) with the ReLU mask and the max-pool arg-max applied.  xb: the breath's padded shared-memory input from
+// position 4*lp0 - 5; dp_ptr: d(pool out) of lp0, dp_stride apart.  For pool output lp0 + j it calls
+//   visit(j, xd, yl, ym, yr, gl, gmid, gr)
+// with y* the conv outputs before BatchNorm, g* their gradients and xd the 11-element input window x[4lp-5 .. 4lp+5] less
+// `shift` (FROZEN: the window itself).  The weight gradient (stem_bwd_kernel) and the input gradient (stem_dgrad_kernel)
+// both run this code, so the two take the same decisions.
+template <typename T, bool FROZEN, typename Visit>
+__device__ __forceinline__ void stem_bwd_run(const float* xb, const T* dp_ptr, int dp_stride, const float (&wr)[STEM_K],
+                                             float sc, float sh, float shift, int lp0, int pool, Visit&& visit) {
+  float xw[11], xd[11];
+#pragma unroll
+  for (int i = 0; i < 7; ++i) {
+    xw[i] = xb[i];
+    xd[i] = FROZEN ? xw[i] : xw[i] - shift;
+  }
+  float yl = stem_dot7(wr, xw[0], xw[1], xw[2], xw[3], xw[4], xw[5], xw[6]);
+  bool okl = lp0 != 0;  // conv position -1 does not exist
+#pragma unroll
+  for (int j = 0; j < STEM_RUN / 2; ++j) {
+    const float dp = Elem<T>::ld(dp_ptr + (size_t)j * dp_stride);
+    const float2 n0 = *reinterpret_cast<const float2*>(xb + 7 + 4 * j);
+    const float2 n1 = *reinterpret_cast<const float2*>(xb + 9 + 4 * j);
+    xw[7] = n0.x; xw[8] = n0.y; xw[9] = n1.x; xw[10] = n1.y;
+#pragma unroll
+    for (int i = 7; i < 11; ++i) xd[i] = FROZEN ? xw[i] : xw[i] - shift;
+    const float ym = stem_dot7(wr, xw[2], xw[3], xw[4], xw[5], xw[6], xw[7], xw[8]);
+    const float yr = stem_dot7(wr, xw[4], xw[5], xw[6], xw[7], xw[8], xw[9], xw[10]);
+    const float zl = okl ? fmaxf(fmaf(yl, sc, sh), 0.f) : 0.f;
+    const float zm = fmaxf(fmaf(ym, sc, sh), 0.f);
+    const float zr = fmaxf(fmaf(yr, sc, sh), 0.f);
+    float gl, gmid, gr;
+    if (pool == 0) {
+      // first strict maximum wins (ATen max_pool semantics); a zero maximum carries no gradient (ReLU)
+      const bool wl = zl > 0.f;
+      const bool wm = zm > (wl ? zl : 0.f);
+      const float best = wm ? zm : (wl ? zl : 0.f);
+      const bool wrt = zr > best;
+      gl = (wl && !wm && !wrt) ? dp : 0.f;
+      gmid = (wm && !wrt) ? dp : 0.f;
+      gr = wrt ? dp : 0.f;
+    } else {
+      const float d3 = dp * (1.f / 3.f);
+      gl = zl > 0.f ? d3 : 0.f;
+      gmid = zm > 0.f ? d3 : 0.f;
+      gr = zr > 0.f ? d3 : 0.f;
+    }
+    visit(j, xd, yl, ym, yr, gl, gmid, gr);
+    // slide by 4 inputs = 2 conv positions
+#pragma unroll
+    for (int i = 0; i < 7; ++i) {
+      xw[i] = xw[i + 4];
+      xd[i] = xd[i + 4];
+    }
+    yl = yr;
+    okl = true;
+  }
+}
+
 // STAGE: the CTA's slice of dout (group x 56 rows x 16 channels) is brought into shared memory with cp.async while the
 // input moments are computed, and sweep B reads it from there.  With the gradient loaded from global memory inside the
 // sweep the kernel spent most of its time waiting on those loads (ncu: long-scoreboard stalls 5.9 per issue, issue
@@ -374,62 +434,19 @@ __global__ void __launch_bounds__(STEM_THREADS)
     const float* xb = xs + b * STEM_BS + STEM_PAD + 4 * lp0 - 5;  // xw[i] = xb[i + 4j]
     const T* dp_ptr = STAGE ? ds + (b * STEM_LP + lp0) * STEM_CS + c
                             : dout + ((breath0 + b) * STEM_LP + lp0) * dout_stride + ch;
-    float xw[11], xd[11];
+    stem_bwd_run<T, FROZEN>(xb, dp_ptr, dp_stride, wr, sc, sh, shift, lp0, pool,
+                            [&s1, &s2, &gt, mean, rstd](int, const float (&xd)[11], float yl, float ym, float yr, float gl, float gmid, float gr) {
+                              s1 += gl + gmid + gr;
+                              s2 = fmaf(gl, (yl - mean) * rstd, s2);
+                              s2 = fmaf(gmid, (ym - mean) * rstd, s2);
+                              s2 = fmaf(gr, (yr - mean) * rstd, s2);
 #pragma unroll
-    for (int i = 0; i < 7; ++i) {
-      xw[i] = xb[i];
-      xd[i] = FROZEN ? xw[i] : xw[i] - shift;
-    }
-    float yl = stem_dot7(wr, xw[0], xw[1], xw[2], xw[3], xw[4], xw[5], xw[6]);
-    bool okl = lp0 != 0;  // conv position -1 does not exist
-#pragma unroll
-    for (int j = 0; j < STEM_RUN / 2; ++j) {
-      const float dp = Elem<T>::ld(dp_ptr + (size_t)j * dp_stride);
-      const float2 n0 = *reinterpret_cast<const float2*>(xb + 7 + 4 * j);
-      const float2 n1 = *reinterpret_cast<const float2*>(xb + 9 + 4 * j);
-      xw[7] = n0.x; xw[8] = n0.y; xw[9] = n1.x; xw[10] = n1.y;
-#pragma unroll
-      for (int i = 7; i < 11; ++i) xd[i] = FROZEN ? xw[i] : xw[i] - shift;
-      const float ym = stem_dot7(wr, xw[2], xw[3], xw[4], xw[5], xw[6], xw[7], xw[8]);
-      const float yr = stem_dot7(wr, xw[4], xw[5], xw[6], xw[7], xw[8], xw[9], xw[10]);
-      const float zl = okl ? fmaxf(fmaf(yl, sc, sh), 0.f) : 0.f;
-      const float zm = fmaxf(fmaf(ym, sc, sh), 0.f);
-      const float zr = fmaxf(fmaf(yr, sc, sh), 0.f);
-      float gl, gmid, gr;
-      if (pool == 0) {
-        // first strict maximum wins (ATen max_pool semantics); a zero maximum carries no gradient (ReLU)
-        const bool wl = zl > 0.f;
-        const bool wm = zm > (wl ? zl : 0.f);
-        const float best = wm ? zm : (wl ? zl : 0.f);
-        const bool wrt = zr > best;
-        gl = (wl && !wm && !wrt) ? dp : 0.f;
-        gmid = (wm && !wrt) ? dp : 0.f;
-        gr = wrt ? dp : 0.f;
-      } else {
-        const float d3 = dp * (1.f / 3.f);
-        gl = zl > 0.f ? d3 : 0.f;
-        gmid = zm > 0.f ? d3 : 0.f;
-        gr = zr > 0.f ? d3 : 0.f;
-      }
-      s1 += gl + gmid + gr;
-      s2 = fmaf(gl, (yl - mean) * rstd, s2);
-      s2 = fmaf(gmid, (ym - mean) * rstd, s2);
-      s2 = fmaf(gr, (yr - mean) * rstd, s2);
-#pragma unroll
-      for (int t = 0; t < STEM_K; ++t) {
-        gt[t] = fmaf(gl, xd[t], gt[t]);
-        gt[t] = fmaf(gmid, xd[t + 2], gt[t]);
-        gt[t] = fmaf(gr, xd[t + 4], gt[t]);
-      }
-      // slide by 4 inputs = 2 conv positions
-#pragma unroll
-      for (int i = 0; i < 7; ++i) {
-        xw[i] = xw[i + 4];
-        xd[i] = xd[i + 4];
-      }
-      yl = yr;
-      okl = true;
-    }
+                              for (int t = 0; t < STEM_K; ++t) {
+                                gt[t] = fmaf(gl, xd[t], gt[t]);
+                                gt[t] = fmaf(gmid, xd[t + 2], gt[t]);
+                                gt[t] = fmaf(gr, xd[t + 4], gt[t]);
+                              }
+                            });
   }
   // reduce the 9 accumulators over the row lanes
   __syncthreads();
@@ -708,6 +725,172 @@ int launch_stem_frozen_bwd(const void* dout, const float* x, const float* w, con
   })
   if (rc) return rc;
   DARDS_CHECK_LAUNCH("stem_frozen_bwd");
+  return DARDS_OK;
+}
+
+// ==== input gradient of the stem: dx (N,224) fp32, run after the weight-gradient backward ==========================
+// dz = d(conv output) = sc * (g - S1/M - xhat * S2/M) with batch statistics (sc = gamma * rstd, M = group * 112, S1 / S2 the
+// group's dbeta / dgamma totals that stem_bwd wrote), sc * g with running statistics (FROZEN, sc = scale); g, the gradient
+// of the conv output through pool and ReLU, comes from stem_bwd_run, so the decisions are the weight gradient's.
+// dx[t] = sum_c sum_k w[c][k] * dz[c][q] over 2q - 3 + k = t.
+// One CTA = DG_CHUNK breaths x ALL channels, 16 channels (a slab) at a time:
+//   1. the sweep writes the slab's dz into shared memory, rows q = -1 .. 113 of every breath (rows -1, 112, 113 stay 0).
+//      A run owns conv positions 2lp0 .. 2lp0+27; the left tap of its first window (2lp0 - 1, the previous run's last
+//      position) is added after a barrier, from `carry`.
+//   2. thread = pair of outputs (2u, 2u+1) of one breath: 7 taps x 16 channels from dz rows u-1 .. u+2, accumulated in
+//      registers over the slabs in order.  No atomics: the sum over channels has a fixed order, dx is deterministic.
+constexpr int DG_CHUNK = 8;                      // breaths per CTA
+constexpr int DG_ROWS = STEM_LC + 3;             // dz rows per breath: q = -1 .. 113
+constexpr int DG_PAIRS = DG_CHUNK * STEM_LC / STEM_THREADS + 1;  // output pairs per thread (896 / 256 -> 4)
+
+template <typename T, bool FROZEN>
+__global__ void __launch_bounds__(STEM_THREADS)
+    stem_dgrad_kernel(const T* __restrict__ dout, const float* __restrict__ x, const float* __restrict__ w,
+                      const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ save_mean,
+                      const float* __restrict__ save_rstd, const float* __restrict__ dgamma_part,
+                      const float* __restrict__ dbeta_part, float* __restrict__ dx, int n_breaths, int group, int c0,
+                      int dout_stride, int pool) {
+  extern __shared__ __align__(16) float smem[];
+  float* dzs = smem;                                       // [DG_CHUNK][DG_ROWS][16]
+  float* xs = smem + DG_CHUNK * DG_ROWS * STEM_CS;         // [DG_CHUNK][STEM_BS]
+  __shared__ __align__(16) float ws[STEM_CS * 8];          // the slab's weights, [c][k] padded to 8
+  __shared__ float carry[DG_CHUNK * 4 * STEM_CS];          // [run][c]
+  const int tid = threadIdx.x;
+  const int c = tid % STEM_CS, rl = tid / STEM_CS;
+  const size_t breath0 = (size_t)blockIdx.x * DG_CHUNK;
+  const int nb = min(DG_CHUNK, n_breaths - (int)breath0);
+  stem_load_group(x + breath0 * STEM_L, xs, nb);
+  for (int i = tid; i < DG_CHUNK * DG_ROWS * STEM_CS; i += STEM_THREADS) dzs[i] = 0.f;
+  const int n_runs = nb * (STEM_LC / STEM_RUN);
+  const int n_pairs = nb * STEM_LC;
+  float acc_e[DG_PAIRS], acc_o[DG_PAIRS];
+#pragma unroll
+  for (int i = 0; i < DG_PAIRS; ++i) acc_e[i] = acc_o[i] = 0.f;
+  const float inv_m = 1.f / (float)(group * STEM_LC);
+
+  for (int slab = 0; slab < c0 / STEM_CS; ++slab) {
+    __syncthreads();  // xs / dzs zeroed, or the previous slab's step 2 is done with dzs and ws
+    const int ch = slab * STEM_CS + c;
+    if (tid < STEM_CS * STEM_K) ws[(tid / STEM_K) * 8 + tid % STEM_K] = w[(slab * STEM_CS) * STEM_K + tid];
+    float wr[STEM_K];
+#pragma unroll
+    for (int t = 0; t < STEM_K; ++t) wr[t] = w[ch * STEM_K + t];
+    // ---- 1. dz of this slab ----------------------------------------------------------------------------------
+    for (int run = rl; run < n_runs; run += STEM_LANES) {
+      const int b = run >> 2, lp0 = (run & 3) * (STEM_RUN / 2);
+      const int g = FROZEN ? 0 : (int)((breath0 + b) / group);
+      const float mean = FROZEN ? 0.f : save_mean[(size_t)g * c0 + ch], rstd = FROZEN ? 0.f : save_rstd[(size_t)g * c0 + ch];
+      const float gm = gamma[ch];
+      // the weight-gradient kernel's scale / shift, the same expressions
+      const float sc = FROZEN ? gm : rstd * gm, sh = FROZEN ? beta[ch] : beta[ch] - mean * sc;
+      const float a1 = FROZEN ? 0.f : dbeta_part[(size_t)g * c0 + ch] * inv_m;
+      const float a2 = FROZEN ? 0.f : dgamma_part[(size_t)g * c0 + ch] * inv_m;
+      const float* xb = xs + b * STEM_BS + STEM_PAD + 4 * lp0 - 5;
+      const T* dp_ptr = dout + ((breath0 + b) * STEM_LP + lp0) * dout_stride + ch;
+      float* dz = dzs + (b * DG_ROWS + 1) * STEM_CS + c;  // dz[q * 16]: row q
+      float pend = 0.f;
+      stem_bwd_run<T, FROZEN>(xb, dp_ptr, dout_stride, wr, sc, sh, 0.f, lp0, pool,
+                              [&](int j, const float (&)[11], float, float ym, float yr, float gl, float gmid, float gr) {
+                                const int q = 2 * (lp0 + j);
+                                if (j == 0) carry[run * STEM_CS + c] = sc * gl;
+                                else dz[(q - 1) * STEM_CS] = fmaf(sc, gl, pend);
+                                if (FROZEN) {
+                                  dz[q * STEM_CS] = sc * gmid;
+                                  pend = sc * gr;
+                                } else {
+                                  dz[q * STEM_CS] = sc * (gmid - a1 - (ym - mean) * rstd * a2);
+                                  pend = sc * (gr - a1 - (yr - mean) * rstd * a2);
+                                }
+                              });
+      dz[(2 * lp0 + STEM_RUN - 1) * STEM_CS] = pend;
+    }
+    __syncthreads();
+    for (int run = rl; run < n_runs; run += STEM_LANES) {
+      const int b = run >> 2, lp0 = (run & 3) * (STEM_RUN / 2);
+      if (lp0 != 0) dzs[(b * DG_ROWS + 2 * lp0) * STEM_CS + c] += carry[run * STEM_CS + c];  // row q = 2lp0 - 1
+    }
+    __syncthreads();
+    // ---- 2. dx += the slab's 16 channels ---------------------------------------------------------------------
+#pragma unroll
+    for (int i = 0; i < DG_PAIRS; ++i) {
+      const int p = tid + i * STEM_THREADS;
+      if (p < n_pairs) {
+        const int b = p / STEM_LC, u = p % STEM_LC;
+        const float4* r = reinterpret_cast<const float4*>(dzs + (b * DG_ROWS + u) * STEM_CS);  // row q = u - 1
+        float e = acc_e[i], o = acc_o[i];
+#pragma unroll
+        for (int c4 = 0; c4 < STEM_CS / 4; ++c4) {
+          const float4 r0 = r[c4], r1 = r[4 + c4], r2 = r[8 + c4], r3 = r[12 + c4];  // q = u-1, u, u+1, u+2
+          const float d0[4] = {r0.x, r0.y, r0.z, r0.w}, d1[4] = {r1.x, r1.y, r1.z, r1.w};
+          const float d2[4] = {r2.x, r2.y, r2.z, r2.w}, d3[4] = {r3.x, r3.y, r3.z, r3.w};
+#pragma unroll
+          for (int cc = 0; cc < 4; ++cc) {
+            const float4 wa = *reinterpret_cast<const float4*>(ws + (4 * c4 + cc) * 8);
+            const float4 wb = *reinterpret_cast<const float4*>(ws + (4 * c4 + cc) * 8 + 4);
+            e = fmaf(wa.y, d2[cc], e);  // t = 2u: k = 1, 3, 5 -> q = u+1, u, u-1
+            e = fmaf(wa.w, d1[cc], e);
+            e = fmaf(wb.y, d0[cc], e);
+            o = fmaf(wa.x, d3[cc], o);  // t = 2u+1: k = 0, 2, 4, 6 -> q = u+2, u+1, u, u-1
+            o = fmaf(wa.z, d2[cc], o);
+            o = fmaf(wb.x, d1[cc], o);
+            o = fmaf(wb.z, d0[cc], o);
+          }
+        }
+        acc_e[i] = e;
+        acc_o[i] = o;
+      }
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < DG_PAIRS; ++i) {
+    const int p = tid + i * STEM_THREADS;
+    if (p < n_pairs) {
+      const int b = p / STEM_LC, u = p % STEM_LC;
+      *reinterpret_cast<float2*>(dx + (breath0 + b) * STEM_L + 2 * u) = make_float2(acc_e[i], acc_o[i]);
+    }
+  }
+}
+
+template <bool FROZEN>
+static int stem_dgrad_launch(const void* dout, const float* x, const float* w, const float* gamma, const float* beta,
+                             const float* save_mean, const float* save_rstd, const float* dgamma_part,
+                             const float* dbeta_part, float* dx, int n_breaths, int group, int c0, int dout_stride, int pool,
+                             int dtype, cudaStream_t st) {
+  const size_t smem = (size_t)DG_CHUNK * (DG_ROWS * STEM_CS + STEM_BS) * sizeof(float);
+  dim3 grid((unsigned)ceil_div(n_breaths, DG_CHUNK));
+  static size_t granted[2] = {44 * 1024, 44 * 1024};
+  DARDS_DISPATCH_DTYPE(dtype, {
+    int rc = stem_smem_optin(stem_dgrad_kernel<T, FROZEN>, smem, &granted[dtype == DARDS_BF16 ? 1 : 0]);
+    if (rc) return rc;
+    stem_dgrad_kernel<T, FROZEN><<<grid, STEM_THREADS, smem, st>>>(static_cast<const T*>(dout), x, w, gamma, beta, save_mean,
+                                                                   save_rstd, dgamma_part, dbeta_part, dx, n_breaths, group,
+                                                                   c0, dout_stride, pool);
+  })
+  return DARDS_OK;
+}
+
+int launch_stem_dgrad(const void* dout, const float* x, const float* w, const float* gamma, const float* beta,
+                      const float* save_mean, const float* save_rstd, const float* dgamma_part, const float* dbeta_part,
+                      float* dx, int n_groups, int group, int c0, int dout_stride, int pool, int dtype, cudaStream_t st) {
+  DARDS_CHECK_ARG(stem_c0_ok(c0), "stem: initial planes must be a multiple of %d (got %d)", STEM_CS, c0);
+  DARDS_CHECK_ARG(group > 0, "stem: BatchNorm group must be at least 1 breath (got %d)", group);
+  if (n_groups == 0) return DARDS_OK;
+  DARDS_CHECK_ARG((long long)n_groups * group <= 0x7fffffffLL, "stem_dgrad: too many breaths");
+  int rc = stem_dgrad_launch<false>(dout, x, w, gamma, beta, save_mean, save_rstd, dgamma_part, dbeta_part, dx,
+                                    n_groups * group, group, c0, dout_stride, pool, dtype, st);
+  if (rc) return rc;
+  DARDS_CHECK_LAUNCH("stem_dgrad");
+  return DARDS_OK;
+}
+
+int launch_stem_frozen_dgrad(const void* dout, const float* x, const float* w, const float* scale, const float* shift,
+                             float* dx, int n_breaths, int c0, int dout_stride, int pool, int dtype, cudaStream_t st) {
+  DARDS_CHECK_ARG(stem_c0_ok(c0), "stem: initial planes must be a multiple of %d (got %d)", STEM_CS, c0);
+  if (n_breaths == 0) return DARDS_OK;
+  int rc = stem_dgrad_launch<true>(dout, x, w, scale, shift, nullptr, nullptr, nullptr, nullptr, dx, n_breaths, 1, c0,
+                                   dout_stride, pool, dtype, st);
+  if (rc) return rc;
+  DARDS_CHECK_LAUNCH("stem_frozen_dgrad");
   return DARDS_OK;
 }
 
@@ -1146,6 +1329,112 @@ int launch_stem_alt_bwd(const void* dout, const float* x, const float* w, const 
                                                        dgamma_part, dbeta_part, group, nc, c0);
     DARDS_CHECK_LAUNCH("stem_alt_bwd (chunk combine)");
   }
+  return DARDS_OK;
+}
+
+// Input gradient of stage 1, run after stem_alt_bwd: d a0 (N,224,C0) -> dx (N,224) fp32.
+// dz = sc * (g - S1/M - xhat * S2/M), sc = gamma * rstd, M = group * 224, S1 / S2 the group totals stem_alt_bwd wrote to
+// dbeta_part / dgamma_part; dx[t] = sum_c sum_k w[c][k] * dz[c][t + 1 - k].
+// One CTA = S1_DG_CHUNK breaths, one breath at a time: the breath's group coefficients are staged in shared memory, thread
+// (c, rl) computes dz at positions l = rl + 16i for channels c, c + 16, ... and sums u_k(l) = sum_c w[c][k] dz[c][l] over
+// them, the 16 channel lanes are added with a fixed butterfly (deterministic), then dx[t] = u_0(t+1) + u_1(t) + u_2(t-1).
+constexpr int S1_DG_CHUNK = 8;
+
+template <typename T>
+__global__ void __launch_bounds__(STEM_THREADS)
+    stem_alt_dgrad_kernel(const T* __restrict__ dout, const float* __restrict__ x, const float* __restrict__ w,
+                          const float* __restrict__ gamma, const float* __restrict__ save_mean,
+                          const float* __restrict__ save_rstd, const float* __restrict__ dgamma_part,
+                          const float* __restrict__ dbeta_part, float* __restrict__ dx, int n_breaths, int group, int c0,
+                          int dout_stride) {
+  extern __shared__ __align__(16) float coef[];  // [c0][8]: w0 w1 w2 sc a1 mean rstd a2
+  __shared__ float xs[STEM_L + 2];
+  __shared__ float us[STEM_L + 2][S1_K];         // u_k(l) at row l + 1; rows 0 and 225 stay 0
+  const int tid = threadIdx.x;
+  const int c = tid % STEM_CS, rl = tid / STEM_CS;
+  const float inv_m = 1.f / (float)(group * STEM_L);
+  if (tid < S1_K) {
+    us[0][tid] = 0.f;
+    us[STEM_L + 1][tid] = 0.f;
+  }
+  int staged = -1;
+  for (int bi = 0; bi < S1_DG_CHUNK; ++bi) {
+    const size_t breath = (size_t)blockIdx.x * S1_DG_CHUNK + bi;
+    if (breath >= (size_t)n_breaths) break;
+    const int g = (int)(breath / group);
+    __syncthreads();  // the previous breath is done with xs, us and coef
+    if (g != staged) {
+      for (int ch = tid; ch < c0; ch += STEM_THREADS) {
+        const size_t o = (size_t)g * c0 + ch;
+        const float rstd = save_rstd[o];
+        float* k = coef + ch * 8;
+        k[0] = w[ch * S1_K];
+        k[1] = w[ch * S1_K + 1];
+        k[2] = w[ch * S1_K + 2];
+        k[3] = rstd * gamma[ch];
+        k[4] = dbeta_part[o] * inv_m;
+        k[5] = save_mean[o];
+        k[6] = rstd;
+        k[7] = dgamma_part[o] * inv_m;
+      }
+      staged = g;
+    }
+    for (int i = tid; i < STEM_L + 2; i += STEM_THREADS) {
+      const int p = i - 1;
+      xs[i] = (p >= 0 && p < STEM_L) ? x[breath * STEM_L + p] : 0.f;
+    }
+    __syncthreads();
+    for (int l = rl; l < STEM_L; l += STEM_LANES) {  // 14 positions per lane, the same count in every lane
+      const float x0 = xs[l], x1 = xs[l + 1], x2 = xs[l + 2];
+      const T* dp = dout + (breath * STEM_L + l) * dout_stride;
+      float u0 = 0.f, u1 = 0.f, u2 = 0.f;
+      for (int ch = c; ch < c0; ch += STEM_CS) {
+        const float4 ka = *reinterpret_cast<const float4*>(coef + ch * 8);
+        const float4 kb = *reinterpret_cast<const float4*>(coef + ch * 8 + 4);
+        const float gv = Elem<T>::ld(dp + ch);
+        // y and xhat exactly as stem_alt_bwd_kernel computes them
+        const float y = fmaf(ka.x, x0, fmaf(ka.y, x1, ka.z * x2));
+        const float dz = ka.w * (gv - kb.x - (y - kb.y) * kb.z * kb.w);
+        u0 = fmaf(ka.x, dz, u0);
+        u1 = fmaf(ka.y, dz, u1);
+        u2 = fmaf(ka.z, dz, u2);
+      }
+#pragma unroll
+      for (int off = STEM_CS / 2; off > 0; off >>= 1) {
+        u0 += __shfl_xor_sync(0xffffffffu, u0, off);
+        u1 += __shfl_xor_sync(0xffffffffu, u1, off);
+        u2 += __shfl_xor_sync(0xffffffffu, u2, off);
+      }
+      if (c == 0) {
+        us[l + 1][0] = u0;
+        us[l + 1][1] = u1;
+        us[l + 1][2] = u2;
+      }
+    }
+    __syncthreads();
+    if (tid < STEM_L) dx[breath * STEM_L + tid] = us[tid + 2][0] + us[tid + 1][1] + us[tid][2];
+  }
+}
+
+int launch_stem_alt_dgrad(const void* dout, const float* x, const float* w, const float* gamma, const float* save_mean,
+                          const float* save_rstd, const float* dgamma_part, const float* dbeta_part, float* dx, int n_groups,
+                          int group, int c0, int dout_stride, int dtype, cudaStream_t st) {
+  DARDS_CHECK_ARG(stem_c0_ok(c0), "stem_alt: initial planes must be a multiple of %d (got %d)", STEM_CS, c0);
+  DARDS_CHECK_ARG(group > 0, "stem_alt: BatchNorm group must be at least 1 breath (got %d)", group);
+  if (n_groups == 0) return DARDS_OK;
+  DARDS_CHECK_ARG((long long)n_groups * group <= 0x7fffffffLL, "stem_alt_dgrad: too many breaths");
+  const int n = n_groups * group;
+  const size_t smem = (size_t)c0 * 8 * sizeof(float);
+  dim3 grid((unsigned)ceil_div(n, S1_DG_CHUNK));
+  static size_t granted[2] = {44 * 1024, 44 * 1024};
+  DARDS_DISPATCH_DTYPE(dtype, {
+    int rc = stem_smem_optin(stem_alt_dgrad_kernel<T>, smem, &granted[dtype == DARDS_BF16 ? 1 : 0]);
+    if (rc) return rc;
+    stem_alt_dgrad_kernel<T><<<grid, STEM_THREADS, smem, st>>>(static_cast<const T*>(dout), x, w, gamma, save_mean,
+                                                               save_rstd, dgamma_part, dbeta_part, dx, n, group, c0,
+                                                               dout_stride);
+  })
+  DARDS_CHECK_LAUNCH("stem_alt_dgrad");
   return DARDS_OK;
 }
 

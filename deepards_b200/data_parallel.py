@@ -126,6 +126,30 @@ class BucketedAllReduce(object):
         self.handles = []
 
 
+def head_backbone_plan(net, x, bn_rule, update_running, input_grad=False):
+    """The "backbone" plan that runs a head's backbone when the head's own arithmetic (`net._head`) stays in torch: the
+    trainer's generic step and saliency.input_gradients.  Its owner is the head module, so its grad_flat has the slot table
+    of param_layout(net), the head's parameters included.  BatchNorm group: the sequence (x.shape[1]), or for CNNRegressor
+    the whole flat batch.  bn_rule(backbone) -> the plan's bn ('train' / 'frozen'); dropout follows the backbone's
+    training flag."""
+    bb = net.breath_block
+    from .torch_cnn_linear_network import CNNDoubleLinearNetwork, CNNLinearNetwork, CNNRegressor, _drop_key
+    from .autograd import module_precision
+    if x.shape[-1] != engine.SEQ_LEN:
+        raise Exception('input breaths must have sequence length of 224')
+    n = x.numel() // engine.SEQ_LEN
+    group = n if isinstance(net, CNNRegressor) else x.shape[1]
+    want = {CNNLinearNetwork: group * bb.n_out_filters, CNNDoubleLinearNetwork: 2 * group}.get(type(net))
+    if want is not None and net.linear_final.in_features != want:
+        raise NotImplementedError("deepards_b200: metadata_features > 0 is not implemented (linear_final expects %d "
+                                  "features, the head provides %d)" % (net.linear_final.in_features, want))
+    training = bb.training
+    bn = bn_rule(bb)
+    return engine.get_plan(net, bb, None, n, group, module_precision(net), "backbone",
+                           dropout=_drop_key(bb) if training else (), update_running=update_running, bn=bn,
+                           input_grad=input_grad)
+
+
 class _HeadCall(torch.nn.Module):
     """forward(feat) = net._head(feat): lets torch.func.functional_call run the head on substitute parameters."""
 
@@ -238,25 +262,8 @@ class DataParallelTrainer(object):
         return bn
 
     def _generic_plan(self, x):
-        """The backbone plan of the generic step.  Its owner is the head module, so its grad_flat has the slot table of
-        param_layout(net), the head's parameters included.  BatchNorm group: the sequence (x.shape[1]), or for
-        CNNRegressor the rank's whole flat batch."""
-        net = self.net
-        bb = net.breath_block
-        from .torch_cnn_linear_network import CNNDoubleLinearNetwork, CNNLinearNetwork, _drop_key
-        from .autograd import module_precision
-        if x.shape[-1] != engine.SEQ_LEN:
-            raise Exception('input breaths must have sequence length of 224')
-        n = x.numel() // engine.SEQ_LEN
-        group = n if self.flat_batch else x.shape[1]
-        want = {CNNLinearNetwork: group * bb.n_out_filters, CNNDoubleLinearNetwork: 2 * group}.get(type(net))
-        if want is not None and net.linear_final.in_features != want:
-            raise NotImplementedError("deepards_b200: metadata_features > 0 is not implemented (linear_final expects %d "
-                                      "features, the head provides %d)" % (net.linear_final.in_features, want))
-        training = bb.training
-        bn = self._bn_mode(bb)
-        plan = engine.get_plan(net, bb, None, n, group, module_precision(net), "backbone",
-                               dropout=_drop_key(bb) if training else (), update_running=training, bn=bn)
+        """The backbone plan of the generic step (head_backbone_plan)."""
+        plan = head_backbone_plan(self.net, x, self._bn_mode, self.net.breath_block.training)
         if getattr(plan, "_dp_buckets", None) is None:
             # the head's slots come last in named_parameters() order: they are in the first (suffix) bucket, which is
             # complete before the backbone backward starts

@@ -160,16 +160,22 @@ class Plan(object):
     'per_breath' (-> logits (B,group,2)), 'features' (DenseNet only, -> norm5 output (N,F,7)).
     bn: 'train' (batch statistics; forward and backward), 'eval' (ResNet only: BatchNorm with the running statistics,
     applied in the convolution epilogues; a forward only, see _build_resnet_eval) or 'frozen' (ResNet only: BatchNorm with
-    the running statistics, forward and backward, no running-statistics update; see bn_mode and _build_resnet)."""
+    the running statistics, forward and backward, no running-statistics update; see bn_mode and _build_resnet).
+    input_grad (train and frozen plans): the backward also writes the gradient w.r.t. the input, `dx` (N, 224) fp32, with the
+    stem's dgrad kernel recorded right after the stem's weight-gradient backward (saliency.input_gradients)."""
 
-    def __init__(self, net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running, bn="train"):
+    def __init__(self, net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running, bn="train",
+                 input_grad=False):
         if precision not in _DTYPES:
             raise ValueError("precision must be 'fp32' or 'bf16', got %r" % (precision,))
         if n_breaths % group != 0:
             raise ValueError("number of breaths (%d) is not a multiple of the BatchNorm group (%d)" % (n_breaths, group))
         if bn not in ("train", "eval", "frozen"):
             raise ValueError("bn must be 'train', 'eval' or 'frozen', got %r" % (bn,))
+        if input_grad and bn == "eval":
+            raise ValueError("an eval plan has no backward: input_grad needs bn='train' or 'frozen'")
         self.bn = bn
+        self.input_grad = input_grad
         self.net, self.backbone, self.linear = net, backbone, linear
         self.N, self.group, self.G = n_breaths, group, n_breaths // group
         self.precision, self.mode = precision, mode
@@ -213,6 +219,7 @@ class Plan(object):
 
         # ---- I/O buffers ------------------------------------------------------------------------------------
         self.x_buf = self.new((n_breaths, SEQ_LEN), torch.float32)
+        self.dx = self.new((n_breaths, SEQ_LEN), torch.float32) if input_grad else None
         # [0] forward counter (fresh dropout masks per step), [1] global index of this rank's first sequence
         self.seed_dev = self.new((2,), torch.int64, zero=True)
         self._seq_offset = 0
@@ -588,6 +595,9 @@ class Plan(object):
             self.bwd.add("dards_stem_frozen_bwd", dout, self.x_buf.data_ptr(), conv.weight.data_ptr(), st.scale, st.shift,
                          st.mean, st.rstd, dwp.data_ptr(), dgp.data_ptr(), dbp.data_ptr(), self.N, c0, dout_stride, pool,
                          self.dt)
+            if self.input_grad:
+                self.bwd.add("dards_stem_frozen_dgrad", dout, self.x_buf.data_ptr(), conv.weight.data_ptr(), st.scale,
+                             st.shift, self.dx.data_ptr(), self.N, c0, dout_stride, pool, self.dt)
             self._pending_red.append((dwp, nc, c0 * 7, self.gptr(conv.weight)))
             self._pending_red.append((dgp, nc, c0, self.gptr(bn.weight)))
             self._pending_red.append((dbp, nc, c0, self.gptr(bn.bias)))
@@ -601,6 +611,10 @@ class Plan(object):
         self.bwd.add("dards_stem_bwd", dout, self.x_buf.data_ptr(), conv.weight.data_ptr(), bn.weight.data_ptr(),
                      bn.bias.data_ptr(), mean.data_ptr(), rstd.data_ptr(), dwp.data_ptr(), dgp.data_ptr(), dbp.data_ptr(),
                      self.G, self.group, c0, dout_stride, pool, ws, ws_bytes, self.dt)
+        if self.input_grad:  # reads the group totals dgp / dbp that the backward just wrote
+            self.bwd.add("dards_stem_dgrad", dout, self.x_buf.data_ptr(), conv.weight.data_ptr(), bn.weight.data_ptr(),
+                         bn.bias.data_ptr(), mean.data_ptr(), rstd.data_ptr(), dgp.data_ptr(), dbp.data_ptr(),
+                         self.dx.data_ptr(), self.G, self.group, c0, dout_stride, pool, self.dt)
         self._pending_red.append((dwp, self.G, c0 * 7, self.gptr(conv.weight)))
         self._pending_red.append((dgp, self.G, c0, self.gptr(bn.weight)))
         self._pending_red.append((dbp, self.G, c0, self.gptr(bn.bias)))
@@ -843,6 +857,10 @@ class Plan(object):
         self.bwd.add("dards_stem_alt_bwd", da0.data_ptr(), self.x_buf.data_ptr(), m.conv1_alt.weight.data_ptr(),
                      m.bn1.weight.data_ptr(), mean1.data_ptr(), rstd1.data_ptr(), dwp.data_ptr(), dgp.data_ptr(),
                      dbp.data_ptr(), self.G, self.group, c0, c0, ws, ws_bytes, self.dt)
+        if self.input_grad:
+            self.bwd.add("dards_stem_alt_dgrad", da0.data_ptr(), self.x_buf.data_ptr(), m.conv1_alt.weight.data_ptr(),
+                         m.bn1.weight.data_ptr(), mean1.data_ptr(), rstd1.data_ptr(), dgp.data_ptr(), dbp.data_ptr(),
+                         self.dx.data_ptr(), self.G, self.group, c0, c0, self.dt)
         self._pending_red.append((dwp, self.G, c0 * 3, self.gptr(m.conv1_alt.weight)))
         self._pending_red.append((dgp, self.G, c0, self.gptr(m.bn1.weight)))
         self._pending_red.append((dbp, self.G, c0, self.gptr(m.bn1.bias)))
@@ -1231,7 +1249,8 @@ class Plan(object):
         return out
 
 
-def get_plan(net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running, bn="train"):
+def get_plan(net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running, bn="train",
+             input_grad=False):
     """Plan cache on the owning module (invalidated when a parameter's storage moves)."""
     cache = net.__dict__.setdefault("_dards_plans", {})
     # multi-rank plans flush their pending partial-sum reductions at every all-reduce mark: a plan built before
@@ -1239,8 +1258,10 @@ def get_plan(net, backbone, linear, n_breaths, group, precision, mode, dropout, 
     key = (n_breaths, group, precision, mode, tuple(dropout), bool(update_running), _multi_rank())
     if bn != "train":
         key += (bn,)
+    if input_grad:
+        key += ("input_grad",)
     plan = cache.get(key)
     if plan is None or not plan.valid():
-        plan = Plan(net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running, bn)
+        plan = Plan(net, backbone, linear, n_breaths, group, precision, mode, dropout, update_running, bn, input_grad)
         cache[key] = plan
     return plan

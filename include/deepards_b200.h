@@ -285,6 +285,15 @@ int dards_stem_bwd(const void* dout, const float* x, const float* w, const float
                    const float* save_mean, const float* save_rstd, float* dw_part, float* dgamma_part,
                    float* dbeta_part, int n_groups, int group, int c0, int dout_stride, int pool, void* workspace,
                    long long workspace_bytes, int dtype, void* stream);
+/* Input gradient of the stem, run after dards_stem_bwd on the same dout: dx (N,224) fp32, N = n_groups * group.  The pool
+ * arg-max and the ReLU mask are recomputed exactly as dards_stem_bwd recomputes them; dgamma_part / dbeta_part are the
+ * group totals [n_groups][C0] that dards_stem_bwd wrote.  Deterministic (no atomics), no workspace. */
+int dards_stem_dgrad(const void* dout, const float* x, const float* w, const float* gamma, const float* beta,
+                     const float* save_mean, const float* save_rstd, const float* dgamma_part, const float* dbeta_part,
+                     float* dx, int n_groups, int group, int c0, int dout_stride, int pool, int dtype, void* stream);
+/* Input gradient of dards_stem_eval_fwd (running statistics): dx (N,224) fp32, with the forward's scale / shift. */
+int dards_stem_frozen_dgrad(const void* dout, const float* x, const float* w, const float* scale, const float* shift,
+                            float* dx, int n_breaths, int c0, int dout_stride, int pool, int dtype, void* stream);
 
 /* ---- stage 1 of the two-convolution stem: Conv1d(1->C0,k3,s1,p1) + BN (ResNet double_conv_first) ------------- */
 /* resnet.py:145-147: x (N,224) fp32 -> a0 = bn1(conv1_alt(x)) (N,224,C0) in `dtype`, no ReLU, no pool; the batch statistics
@@ -305,6 +314,11 @@ int dards_stem_alt_bwd(const void* dout, const float* x, const float* w, const f
                        const float* save_rstd, float* dw_part, float* dgamma_part, float* dbeta_part, int n_groups,
                        int group, int c0, int dout_stride, void* workspace, long long workspace_bytes, int dtype,
                        void* stream);
+/* Input gradient of stage 1, run after dards_stem_alt_bwd on the same d a0: dx (N,224) fp32, N = n_groups * group, from the
+ * group totals dgamma_part / dbeta_part [n_groups][C0] that dards_stem_alt_bwd wrote.  Deterministic, no workspace. */
+int dards_stem_alt_dgrad(const void* dout, const float* x, const float* w, const float* gamma, const float* save_mean,
+                         const float* save_rstd, const float* dgamma_part, const float* dbeta_part, float* dx, int n_groups,
+                         int group, int c0, int dout_stride, int dtype, void* stream);
 
 /* ---- pooling, dropout --------------------------------------------------------------- */
 /* nn.MaxPool1d / AvgPool1d(3, 2, padding 1) (resnet.py:101-104, 151-153): (N,L,C) -> (N,(L-1)/2+1,C).  pool: 0 max
